@@ -20,6 +20,8 @@ exposed exchange).  `c5` holds the same record for BASELINE.json configs[4] (uni
 
 Other workloads (`--workload c1|c3|c4|c5shard`) time the remaining configurations as the primary one (single GPU).
 `--also` names further methods timed after the primary one; their numbers land in "methods".
+`--dump-outputs DIR` (N = 1) writes y of the primary method's last timed step to DIR (see --help); the matrix and x
+come from fixed seeds, so two builds run with the same arguments can be compared output for output.
 
 One JSON line on stdout (rank 0).  `value` = whole-job GFLOP/s with everything resident in HBM; `e2e` = the same
 metric with HOST x / y (pinned), H2D + kernels + D2H inside the timed region (N = 1: one spmv() call of the C-ABI with
@@ -40,6 +42,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # no __pycache__ in the tree: it may be read-only
 
 METHODS = {"serial": 0, "parallel": 1, "balanced": 2, "balanced2": 3, "balanced_yid": 4, "sell": 5, "csr5": 6}
 REF_METHOD_NAMES = ["Method_Serial", "Method_Parallel", "Method_Balanced", "Method_Balanced2", "Method_BalancedYid",
@@ -224,11 +227,11 @@ def host_c2(small: bool, device_matrix=None):
     return M.CSR(rows, rows, rowptr, np.concatenate([p.col for p in parts]), np.concatenate([p.val for p in parts]), "c2")
 
 
-def cpu_time_reference(steps: int, warmup: int, small: bool, device_matrix=None, budget_s: float = 40.0):
+def cpu_time_reference(steps: int, warmup: int, small: bool, device_matrix=None):
     """Best OpenMP+AVX2 method of the reference on all host threads (protocol of src/samples/test_spmv.c:87-124: create
     with nthreads = team size, warm-up, timed spmv() calls).  The method is chosen from 10 calls each on a 2^21-row
     sample (creating CSR5 / SELL handles for half a billion non-zeros six times over would take minutes); the two
-    fastest are then created and timed on the FULL matrix and the better one is reported."""
+    fastest are then created and timed on the FULL matrix, `steps` calls each, and the better one is reported."""
     from oracle import oracle as O
     from spmv_b200 import matrices as M
     A = host_c2(small, device_matrix)
@@ -269,17 +272,13 @@ def cpu_time_reference(steps: int, warmup: int, small: bool, device_matrix=None,
             h = R.create(A.m, A.n, A.rowptr, A.col, A.val, T, method)
             for _ in range(max(warmup, 2)):
                 R.spmv(h, x, y)
-            t0 = time.perf_counter()
-            R.spmv(h, x, y)
-            dt = time.perf_counter() - t0
-            k = max(10, min(steps, int(budget_s / 2 / max(dt, 1e-4))))
             times = []
-            for _ in range(k):
+            for _ in range(steps):
                 t0 = time.perf_counter()
                 R.spmv(h, x, y)
                 times.append(time.perf_counter() - t0)
             h.destroy()
-            log(f"  cpu reference, full C2, {REF_METHOD_NAMES[method]}: {k} calls, avg {np.mean(times) * 1e3:.1f} ms, best {min(times) * 1e3:.1f} ms")
+            log(f"  cpu reference, full C2, {REF_METHOD_NAMES[method]}: {steps} calls, avg {np.mean(times) * 1e3:.1f} ms, best {min(times) * 1e3:.1f} ms")
             if best is None or np.mean(times) < np.mean(best[1]):
                 best = (method, times)
         method, times = best
@@ -290,7 +289,7 @@ def cpu_time_reference(steps: int, warmup: int, small: bool, device_matrix=None,
         __import__("ctypes").CDLL("libgomp.so.1").omp_set_num_threads(T)
         P.spmv_serial(A.rowptr, A.col, A.val, x, parallel=True)
         times = []
-        for _ in range(max(10, min(steps, 20))):
+        for _ in range(steps):
             t0 = time.perf_counter()
             P.spmv_serial(A.rowptr, A.col, A.val, x, parallel=True)
             times.append(time.perf_counter() - t0)
@@ -305,7 +304,7 @@ def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return  # rank 0 alone runs and prints; the others exit 0 without work
-    cb, steps, avg, A = cpu_time_reference(args.steps, args.warmup, args.small, budget_s=60.0)
+    cb, steps, avg, A = cpu_time_reference(args.steps, args.warmup, args.small)
     line = {"metric": "spmv_gflops_fp64_csr", "value": cb["value"], "unit": "GFLOP/s", "impl": "reference",
             "n_gpus": args.gpus, "steps": steps, "warmup": args.warmup, "ms_per_step": avg * 1e3,
             "higher_is_better": True, "scaling": "strong" if args.gpus > 1 else "weak", "vs_baseline": None, "dtype": "f64",
@@ -363,9 +362,24 @@ def max_over_ranks(torch, dist, values):
     return [float(v) for v in t.tolist()]
 
 
-def bench_matrix(name, args, torch, steps, warmup, methods, want_e2e):
+DUMP_ROWS = 1 << 21  # rows of y written by --dump-outputs: 2^21 x (8 B value + 8 B row index) = 32 MiB at most
+
+
+def y_sample(torch, y):
+    """Host copy of y at a fixed, seeded set of rows (all rows when y has at most DUMP_ROWS): (values, rows)."""
+    m = y.numel()
+    if m <= DUMP_ROWS:
+        rows = np.arange(m, dtype=np.int64)
+    else:
+        rows = np.sort(np.random.default_rng(0).choice(m, size=DUMP_ROWS, replace=False))
+    vals = y.index_select(0, torch.from_numpy(rows).to(y.device)).cpu().numpy()
+    return vals, rows.astype(np.float64)
+
+
+def bench_matrix(name, args, torch, steps, warmup, methods, want_e2e, outputs=None):
     """One single-GPU workload: every method in `methods` timed device-resident (L2 flushed between steps when the
-    matrix would fit L2), the first one also L2-warm and through host pointers.  Returns a record."""
+    matrix would fit L2), the first one also L2-warm and through host pointers.  Returns a record.  With `outputs`
+    (a dict), y of the first method's last timed step is sampled into outputs["y"] / outputs["y_rows"]."""
     from spmv_b200 import api
     A, n, vsize, desc, seed, _ = make_workload(name, args.small)
     tdt = torch.float64 if vsize == 8 else torch.float32
@@ -404,6 +418,8 @@ def bench_matrix(name, args, torch, steps, warmup, methods, want_e2e):
             ms = time_steps(fn, steps, 0, torch, None, flush)
             launches = api.launch_count() - l0
             clocks = sampler.result()
+            if outputs is not None:
+                outputs["y"], outputs["y_rows"] = y_sample(torch, y)
         else:
             ms = time_steps(fn, steps, warmup, torch, None, flush)
         per = ms / steps
@@ -595,6 +611,8 @@ def run_gpu_arm(args):
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if world != args.gpus:
         log(f"note: --gpus {args.gpus} but WORLD_SIZE={world}; using WORLD_SIZE")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes y of the single-GPU SpMV; it is not available with N > 1")
     torch.cuda.set_device(local)
     dist = None
     if world > 1:
@@ -617,7 +635,13 @@ def single_gpu(args, torch, api):
     default_method = {"c1": "parallel", "c2": "parallel", "c3": "csr5", "c4": "sell", "c5shard": "parallel"}[name]
     primary = args.method or default_method
     methods = [primary] + [mname for mname in args.also.split(",") if mname and mname != primary]
-    rec = bench_matrix(name, args, torch, args.steps, args.warmup, methods, want_e2e=True)
+    outputs = {} if args.dump_outputs else None
+    rec = bench_matrix(name, args, torch, args.steps, args.warmup, methods, want_e2e=True, outputs=outputs)
+    if outputs is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for key, arr in outputs.items():
+            np.save(os.path.join(args.dump_outputs, key + ".npy"), arr)
+        log(f"wrote {', '.join(k + '.npy' for k in outputs)} ({len(outputs['y'])} of {rec['m']} rows of y) to {args.dump_outputs}")
     r = rec["methods"][primary]
     per = r["ms_per_step"]
     peak, peak_src = measured_peak()
@@ -844,7 +868,14 @@ def main():
     ap.add_argument("--ce-lanes", type=int, default=1, help="streams (copy engines) a slice is spread over in the copy-engine exchange")
     ap.add_argument("--align-bands", type=int, default=1, help="N >= 3: as many column bands as ranks for the C2 shards")
     ap.add_argument("--small", action="store_true", help="64x smaller matrices (script debugging only; not a bench)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write y of the last timed step as DIR/y.npy (values) and DIR/y_rows.npy "
+                         "(their row indices): all rows up to 2^21, else a fixed seeded sample of 2^21 rows")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; it is not available with --impl reference")
     claim_stdout()
     args.warmup = max(args.warmup, 3)
     if args.workload != "c2":

@@ -12,7 +12,7 @@ import numpy as np
 import pytest
 
 from conftest import bits_equal
-from cases import all_cases, expected_band_segments
+from cases import GOLDEN_CASES, all_cases, expected_band_segments
 from spmv_b200 import api, matrices as M
 
 pytestmark = pytest.mark.gpu
@@ -69,6 +69,23 @@ def test_all_methods_match_reference_serial(libpath, port, serial_ref, name, dt)
         h.spmv(x, y2)
         assert bits_equal(y, y2), tag + ": not reproducible run to run"
         h.destroy()
+
+
+@pytest.mark.parametrize("name", list(GOLDEN_CASES))
+def test_all_methods_match_the_stored_reference_y(libpath, port, golden, name):
+    """Every method against y of the reference's own Method_Serial as stored in tests/golden (Method_Serial bit for
+    bit): the same bars as above with the reference's outputs, not the port's, on the other side."""
+    A = GOLDEN_CASES[name]()
+    for dt, tag in ((np.float64, "d"), (np.float32, "s")):
+        a = A.astype(dt)
+        x = M.make_x(a.n, 1234, dt)  # the x tests/golden/make_golden.py used
+        stored = golden[f"{name}/y_serial_{tag}"]
+        for method in METHODS:
+            h = api.Handle(a.m, a.n, a.rowptr, a.col, a.val, method, nthreads=8)
+            y = np.full(a.m, np.nan, dtype=dt)
+            h.spmv(x, y)
+            check_y(port, lambda *_: stored, a, x, y, method, f"{name}/{dt.__name__}/{api.METHOD_NAMES[method]}[{h.kernel}]")
+            h.destroy()
 
 
 @pytest.mark.parametrize("dt", [np.float64, np.float32], ids=["fp64", "fp32"])

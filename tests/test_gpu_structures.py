@@ -3,7 +3,7 @@ splitters (a9), SELL permutation (a13), CSR5 tile_ptr / tile_desc / offsets / tr
 import numpy as np
 import pytest
 
-from cases import all_cases
+from cases import GOLDEN_CASES, SELL_NT, all_cases
 from spmv_b200 import api, matrices as M
 
 pytestmark = pytest.mark.gpu
@@ -147,6 +147,28 @@ def test_sell_permutation_against_live_reference(libpath, ref):
     h = api.Handle(a.m, a.n, a.rowptr, a.col, a.val, api.Method_SellCSigma)
     assert np.array_equal(h.structure("sell_perm", np.int32), perm)
     h.destroy()
+
+
+def test_sell_permutation_matches_the_stored_reference(libpath, golden):
+    """The device-built SELL permutation against the reference's own, as stored in tests/golden: every stored window
+    (sigma = 4*floor(m/nthreads/4)) that is a whole number of 32-row slices."""
+    checked = []
+    try:
+        for name, make in GOLDEN_CASES.items():
+            a = make()
+            for nt in SELL_NT:
+                sigma, banner = (int(v) for v in golden[f"{name}/sell_nt{nt}_sigma"])
+                if sigma == 0 or sigma % 32 or sigma > 4096:
+                    continue
+                api.set_option("sell_sigma", sigma)
+                h = api.Handle(a.m, a.n, a.rowptr, a.col, a.val, api.Method_SellCSigma)
+                assert (h.info("sigma"), h.info("banner")) == (sigma, banner), (name, nt)
+                assert np.array_equal(h.structure("sell_perm", np.int32), golden[f"{name}/sell_nt{nt}_perm"]), (name, nt)
+                h.destroy()
+                checked.append((name, nt))
+    finally:
+        api.set_option("sell_sigma", 256)
+    assert checked == [("lap48", 1), ("lap48", 3), ("rmat10", 1), ("st27_9", 11)]
 
 
 @pytest.mark.parametrize("name", list(BIG))
