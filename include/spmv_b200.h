@@ -144,6 +144,9 @@ SPMV_B200_API int spmv_b200_permute_csr(int m, const int *RowPtr, const int *Col
 
 /* kernels launched by this process on the spmv() path since load (for benchmark accounting) */
 SPMV_B200_API unsigned long long spmv_b200_launch_count(void);
+/* device allocations the library currently holds for its own use, in all handles and calls of this process (for leak
+ * checks).  Generated matrices handed to the caller and spmv_b200_malloc blocks are the caller's and not counted. */
+SPMV_B200_API long long spmv_b200_live_allocations(void);
 
 /* ---- multi-GPU row partition -------------------------------------------------------------------
  * splitter[g] = right_boundary(RowPtr, min(g*ceil(nnz/parts), nnz), m+1) - 1, g = 0..parts: the
@@ -205,7 +208,8 @@ SPMV_B200_API int spmv_b200_memcpy(void *dst, const void *src, size_t bytes, int
 
 /* ---- on-device synthetic matrices (SURVEY.md 8d; bit-identical to spmv_b200/matrices.py) ----------
  * Each fills *out with DEVICE pointers owned by the caller (release with spmv_b200_csr_free).
- * `size` = sizeof(double) or sizeof(float).  Returns 0 or -1 (see spmv_b200_last_error). */
+ * `size` = sizeof(double) or sizeof(float).  Returns 0 or -1 (see spmv_b200_last_error); on failure *out holds
+ * nothing to free (arguments that are rejected leave it untouched). */
 typedef struct spmv_b200_csr {
     int m, n;
     long long nnz;

@@ -39,7 +39,7 @@ EXPORTED_FUNCTIONS = [
     "spmv_b200_set_y_peers", "spmv_b200_ipc_export", "spmv_b200_ipc_open", "spmv_b200_ipc_close",
     "spmv_b200_recommend_method", "spmv_b200_bands", "spmv_b200_band_columns", "spmv_b200_spmv_bands",
     "spmv_b200_spmv_finish", "spmv_b200_memcpy_async", "spmv_b200_stream_write32", "spmv_b200_stream_wait32_geq",
-    "spmv_b200_reorder", "spmv_b200_permute_csr", "spmv_b200_update_values"]
+    "spmv_b200_reorder", "spmv_b200_permute_csr", "spmv_b200_update_values", "spmv_b200_live_allocations"]
 EXPORTED_DATA = ["Methods_names", "Vectorized_names", "funcNames"]
 
 
@@ -96,6 +96,7 @@ def lib() -> C.CDLL:
     L.spmv_b200_structure.argtypes = [spmv_Handle_t, C.c_char_p, vp, C.c_size_t]
     L.spmv_b200_structure.restype = ll
     L.spmv_b200_launch_count.restype = C.c_ulonglong
+    L.spmv_b200_live_allocations.restype = ll
     L.spmv_b200_partition_rows.argtypes = [vp, i, i, vp]
     L.spmv_b200_recommend_method.argtypes = [i, vp]
     L.spmv_b200_malloc.argtypes = [C.c_size_t]
@@ -333,6 +334,11 @@ def get_option(key: str) -> int:
 
 def launch_count() -> int:
     return int(lib().spmv_b200_launch_count())
+
+
+def live_allocations() -> int:
+    """Device allocations the library holds for its own use (handles, layouts, temporaries of a running call)."""
+    return int(lib().spmv_b200_live_allocations())
 
 
 def partition_rows(rowptr: np.ndarray, parts: int) -> np.ndarray:

@@ -33,7 +33,69 @@ constexpr int kMaxPeers = 8;        // extra y destinations of the fused SpMV + 
 static inline int ceil_div(long long a, long long b) { return (int)((a + b - 1) / b); }
 
 // ------------------------------------------------------------------------------------------------
-// Device-resident state hanging off spmv_Handle::extraHandle.
+// Device arrays (host code).  Every device allocation the library makes for its own use is held by a DeviceArray or
+// a DeviceBytes: freed when the owner is destroyed, reset or assigned over, so a builder's temporaries are freed on
+// every return path and abandoning a layout is one assignment of an empty group.
+// ------------------------------------------------------------------------------------------------
+void count_allocation(int delta);  // spmv_b200_live_allocations
+
+template <typename U>
+class DeviceArray {
+  public:
+    DeviceArray() = default;
+    DeviceArray(DeviceArray &&o) noexcept : p_(o.p_) { o.p_ = nullptr; }
+    DeviceArray &operator=(DeviceArray &&o) noexcept
+    {
+        if (this != &o) {
+            reset();
+            p_ = o.p_;
+            o.p_ = nullptr;
+        }
+        return *this;
+    }
+    DeviceArray(const DeviceArray &) = delete;
+    DeviceArray &operator=(const DeviceArray &) = delete;
+    ~DeviceArray() { reset(); }
+
+    // `count` elements, at least one, in place of what the owner held; a failure latches the error (SB_CUDA)
+    bool alloc(size_t count)
+    {
+        reset();
+        void *p = nullptr;
+        if (!SB_CUDA(cudaMalloc(&p, (count ? count : 1) * sizeof(U)))) return false;
+        p_ = (U *)p;
+        count_allocation(1);
+        return true;
+    }
+    void reset()
+    {
+        if (!p_) return;
+        cudaFree(p_);
+        count_allocation(-1);
+        p_ = nullptr;
+    }
+    U *get() const { return p_; }
+    operator U *() const { return p_; }  // kernels and copies take the raw pointer; the owner keeps the allocation
+
+  private:
+    U *p_ = nullptr;
+};
+
+// float or double values: the element size is chosen at create (DeviceState::vsize)
+class DeviceBytes {
+  public:
+    bool alloc(size_t count, size_t elem_bytes) { return bytes_.alloc((count ? count : 1) * elem_bytes); }
+    void *get() const { return bytes_.get(); }
+    template <typename T>
+    T *as() const { return (T *)bytes_.get(); }
+
+  private:
+    DeviceArray<unsigned char> bytes_;
+};
+
+// ------------------------------------------------------------------------------------------------
+// Device-resident state hanging off spmv_Handle::extraHandle.  The device arrays are grouped by the builder that
+// fills them, each group with the sizes that describe its arrays.
 // ------------------------------------------------------------------------------------------------
 struct DeviceState {
     uint32_t magic = 0x5b200a11u;
@@ -56,10 +118,11 @@ struct DeviceState {
     int n_peers = 0;                // spmv_b200_set_y_peers
     void *peers[kMaxPeers] = {};
 
-    // CSR on the device (owned upload, or the caller's device arrays adopted in place)
+    // CSR on the device: the caller's device arrays adopted in place, or our upload (32 bytes of slack behind every
+    // array).  rowptr / col / val only point at one of the two.
     int *rowptr = nullptr, *col = nullptr;
     void *val = nullptr;
-    bool owns_csr = false;
+    struct CsrUpload { DeviceArray<int> rowptr, col; DeviceBytes val; } upload;
     bool released_csr = false;      // the upload was freed after a re-laid-out copy took over
 
     // pageable host x / y that keep coming back (the reference's drivers reuse one X and one Y for every call) are
@@ -71,7 +134,7 @@ struct DeviceState {
     bool pin_host = false;
     // staging for host-side x / y; the pipelined host path (CSR-vector kernel) copies x in pieces on s_in,
     // computes row chunks as soon as their prefix of x has arrived, and returns finished chunks of y on s_out
-    void *x_stage = nullptr, *y_stage = nullptr;
+    struct Staging { DeviceBytes x, y; } stage;
     bool pipeline = false;
     cudaStream_t s_in = nullptr, s_out = nullptr;
     cudaEvent_t ev_in[kMaxPieces] = {}, ev_out[kPipeChunks] = {}, ev_start = nullptr, ev_x = nullptr;
@@ -81,67 +144,78 @@ struct DeviceState {
     int tpr = 0;
     // Active matrix view used by every layout builder and kernel: the CSR itself, or (x_bands > 1) its
     // band-major copy, in which virtual row b*m + r holds the entries of row r whose column lies in band
-    // b = col / band_cols.  Kernels then write the virtual y (v_y) and band_reduce_kernel folds it.
+    // b = col / band_cols.  Kernels then write the virtual y (v.y) and band_reduce_kernel folds it.
     int a_m = 0;
     int *a_rowptr = nullptr, *a_col = nullptr;
     void *a_val = nullptr;
     int x_bands = 1, band_cols = 0;
     double far_fraction = -1.0;     // share of entries far from the diagonal (automatic band decision)
-    int *v_rowptr = nullptr, *v_col = nullptr;
-    void *v_val = nullptr, *v_y = nullptr;
+    struct BandCopy { DeviceArray<int> rowptr, col; DeviceBytes val, y; } v;
     // Method_Balanced: row blocks; ref_splitter mirrors the reference with the caller's nthreads
-    int parts = 0;
-    int *splitter = nullptr, *ref_splitter = nullptr;
-    int ref_T = 0;
-    // Method_Balanced2 / Method_Balanced_Yid: tiles + carries
-    int tiles = 0, tile_items = 0;
-    int *tile_rows = nullptr;       // nnz-split: row containing the first nnz of each tile [tiles+1]
-    int2 *merge_coords = nullptr;   // merge-path: (row, nnz) start of each tile [tiles+1]
-    void *carry_val = nullptr;      // [tiles] partial sum that belongs to a row started earlier
-    int *carry_row = nullptr;       // [tiles] that row, or -1
-    void *carry2_val = nullptr;     // level-2 carry list of the two-level fix-up: 2 entries per group of 64 tiles
-    int *carry2_row = nullptr;
+    struct Splitters {
+        int parts = 0, ref_T = 0;
+        DeviceArray<int> splitter;      // [parts+1]
+        DeviceArray<int> ref_splitter;  // [ref_T+1]
+    } split;
+    // tiles of Method_Balanced2 / Method_Balanced_Yid, CSR5 and band segments, and their carries
+    struct Tiles {
+        int count = 0, items = 0;
+        DeviceArray<int> rows;          // nnz-split: row containing the first nnz of each tile [count+1]
+        DeviceArray<int2> merge_coords; // merge-path: (row, nnz) start of each tile [count+1]
+        DeviceBytes carry_val;          // [count] partial sum that belongs to a row started earlier
+        DeviceArray<int> carry_row;     // [count] that row, or -1
+        DeviceBytes carry2_val;         // level-2 carry list of the two-level fix-up: 2 entries per group of 64 tiles
+        DeviceArray<int> carry2_row;
+    } tile;
     // Method_SellCSigma
-    int sigma = 0, banner = 0, slices = 0, sell_variant = 0;
-    long long padded = 0;
-    int *sell_perm = nullptr, *sell_width = nullptr, *sell_full = nullptr, *sell_col = nullptr;
-    long long *sell_slice_ptr = nullptr;
-    void *sell_val = nullptr;
-    // Method_Parallel on short-row matrices with hubs: rows binned by length class (<= 8, <= 32, <= 128), one
-    // launch per bin with 1 / 4 / 16 lanes per row; longer rows are on the long-row list
-    bool binned = false;
-    int *bin_list = nullptr;        // row ids, bin after bin, ascending inside a bin
-    int bin_ptr[4] = {};
-    // hyper-sparse column bands as band segments (band_seg.cuh): x_bands = K but the active view stays the CSR
-    int coo_bands = 0, coo_tiles = 0;  // (option / info key names kept from round 1: "coo_bands")
-    int seg_ptr[kMaxPieces + 1] = {};  // first slot of every band in seg_col / seg_val (aligned to 4), [K] = end
-    int seg_cnt[kMaxPieces] = {};      // entries of every band
-    int seg_tile0[kMaxPieces + 1] = {};  // first tile of every band
-    long long seg_total = 0;           // segments = (band, row) pairs with at least one entry
-    int seg_groups = 0;                // 32-row groups of the merge pass
-    int seg_ctas = 0;                  // persistent CTAs per SM of pass 1
-    int seg_grid = 0;                  // persistent CTAs of pass 1 (device-wide occupancy, set at the first launch)
-    bool seg_cross = false;            // some segment crosses a tile boundary: the carry fix-up is needed
-    bool seg_mask64 = false;           // K > 32: 64-bit row masks
-    int *seg_col = nullptr;            // column index | segment-end bit 31
-    void *seg_ent_val = nullptr;       // values, band-major
-    void *seg_mask = nullptr;          // per row: bands in which it has a segment
-    int4 *seg_tile_ent = nullptr;      // per tile: (first slot, entries, L2-prefetch duty: first x element, elements)
-    int *seg_tile_seg0 = nullptr;      // per 256-entry chunk of a tile (8 per tile): index of its first segment sum
-    int *seg_gbase = nullptr;          // [seg_groups][K]: position of a row group's first segment sum in band b's list
-    int *seg_ticket = nullptr;         // ticket counter of pass 1's dynamic tile schedule
-    void *seg_sums = nullptr;          // [seg_total] segment sums, band-major (written by pass 1, read by pass 2)
+    struct Sell {
+        int sigma = 0, banner = 0, slices = 0, variant = 0;
+        long long padded = 0;
+        DeviceArray<int> perm, width, full, col;
+        DeviceArray<long long> slice_ptr;
+        DeviceBytes val;
+    } sell;
     // long rows / row tails left over by the main kernel of Method_Parallel and Method_SellCSigma (long_rows.cuh)
-    int long_thr = 0x7fffffff;      // CSR-vector kernels skip rows longer than this
-    int lr_rows = 0, lr_segs = 0;
-    bool lr_accumulate = false;     // true: the main kernel already wrote the head of the row (SELL)
-    int *lr_row = nullptr, *lr_start = nullptr, *lr_seg_ptr = nullptr, *lr_seg_row = nullptr;
-    void *lr_partial = nullptr;
+    struct LongRows {
+        int thr = 0x7fffffff;           // CSR-vector kernels skip rows longer than this
+        int rows = 0, segs = 0;
+        bool accumulate = false;        // true: the main kernel already wrote the head of the row (SELL)
+        DeviceArray<int> row, start, seg_ptr, seg_row;
+        DeviceBytes partial;
+        // Method_Parallel on short-row matrices with hubs: rows binned by length class (<= 8, <= 32, <= 128), one
+        // launch per bin with 1 / 4 / 16 lanes per row; longer rows are on the long-row list
+        bool binned = false;
+        DeviceArray<int> bin_list;      // row ids, bin after bin, ascending inside a bin
+        int bin_ptr[4] = {};
+    } lr;
     // Method_CSR5SPMV (omega = 32)
-    int c5_sigma = 0, c5_p = 0, c5_bit_y = 0, c5_bit_ss = 0, c5_num_offsets = 0, c5_tail_start = 0;
-    uint32_t *c5_tile_ptr = nullptr, *c5_tile_desc = nullptr;
-    int *c5_off_ptr = nullptr, *c5_off = nullptr, *c5_col = nullptr;
-    void *c5_val = nullptr;
+    struct Csr5 {
+        int sigma = 0, p = 0, bit_y = 0, bit_ss = 0, num_offsets = 0, tail_start = 0;
+        DeviceArray<uint32_t> tile_ptr, tile_desc;
+        DeviceArray<int> off_ptr, off, col;
+        DeviceBytes val;
+    } c5;
+    // hyper-sparse column bands as band segments (band_seg.cuh): x_bands = K but the active view stays the CSR
+    struct BandSegments {
+        int bands = 0;                  // K (option / info key names kept from round 1: "coo_bands")
+        int ptr[kMaxPieces + 1] = {};   // first slot of every band in col / ent_val (aligned to 4), [K] = end
+        int cnt[kMaxPieces] = {};       // entries of every band
+        int tile0[kMaxPieces + 1] = {}; // first tile of every band
+        long long total = 0;            // segments = (band, row) pairs with at least one entry
+        int groups = 0;                 // 32-row groups of the merge pass
+        int ctas = 0;                   // persistent CTAs per SM of pass 1
+        int grid = 0;                   // persistent CTAs of pass 1 (device-wide occupancy, set at the first launch)
+        bool cross = false;             // some segment crosses a tile boundary: the carry fix-up is needed
+        bool mask64 = false;            // K > 32: 64-bit row masks
+        DeviceArray<int> col;           // column index | segment-end bit 31
+        DeviceBytes ent_val;            // values, band-major
+        DeviceBytes mask;               // per row: bands in which it has a segment
+        DeviceArray<int4> tile_ent;     // per tile: (first slot, entries, L2-prefetch duty: first x element, elements)
+        DeviceArray<int> tile_seg0;     // per 256-entry chunk of a tile (8 per tile): index of its first segment sum
+        DeviceArray<int> gbase;         // [groups][K]: position of a row group's first segment sum in band b's list
+        DeviceArray<int> ticket;        // ticket counter of pass 1's dynamic tile schedule
+        DeviceBytes sums;               // [total] segment sums, band-major (written by pass 1, read by pass 2)
+    } seg;
 };
 
 // ------------------------------------------------------------------------------------------------

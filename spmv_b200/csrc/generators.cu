@@ -162,33 +162,36 @@ static bool alloc_csr(spmv_b200_csr *out, int m, int n, long long nnz, unsigned 
     return true;
 }
 
-static bool gen_stencil(int kind, int d0, int d1, int d2, unsigned long size, spmv_b200_csr *out)
+// a generator's failure exit once *out may hold allocations: *out is freed and zeroed
+static int gen_failed(spmv_b200_csr *out)
+{
+    spmv_b200_csr_free(out);
+    return -1;
+}
+
+static int gen_stencil(int kind, int d0, int d1, int d2, unsigned long size, spmv_b200_csr *out)
 {
     const long long m64 = (long long)d0 * d1 * (kind ? d2 : 1);
-    if (!out || d0 < 1 || d1 < 1 || d2 < 1 || m64 > 0x7fffffffLL / 32) { set_error("bad stencil shape"); return false; }
+    if (!out || d0 < 1 || d1 < 1 || d2 < 1 || m64 > 0x7fffffffLL / 32) { set_error("bad stencil shape"); return -1; }
     const int m = (int)m64;
     memset(out, 0, sizeof(*out));
-    int *cnt = nullptr, *rp = nullptr;
-    SB_TRY(cudaMalloc((void **)&cnt, ((size_t)m + 1) * sizeof(int)));
-    SB_TRY(cudaMalloc((void **)&rp, ((size_t)m + 1 + 8) * sizeof(int)));
+    DeviceArray<int> cnt, rp;
+    DeviceArray<unsigned char> tmp;
+    if (!cnt.alloc((size_t)m + 1) || !rp.alloc((size_t)m + 1)) return -1;
     stencil_count_kernel<<<grid_for(m + 1), 256>>>(kind, d0, d1, d2, m, cnt);
     size_t bytes = 0;
-    SB_TRY(cub::DeviceScan::ExclusiveSum(nullptr, bytes, cnt, rp, m + 1));
-    void *tmp = nullptr;
-    SB_TRY(cudaMalloc(&tmp, bytes ? bytes : 1));
-    SB_TRY(cub::DeviceScan::ExclusiveSum(tmp, bytes, cnt, rp, m + 1));
     int nnz = 0;
-    SB_TRY(cudaMemcpy(&nnz, rp + m, sizeof(int), cudaMemcpyDeviceToHost));
-    cudaFree(tmp);
-    cudaFree(cnt);
-    out->m = m; out->n = m; out->nnz = nnz; out->size = size; out->RowPtr = rp;
-    SB_TRY(cudaMalloc((void **)&out->ColIdx, ((size_t)nnz + 8) * sizeof(int)));
-    SB_TRY(cudaMalloc(&out->Val, ((size_t)nnz + 8) * size));
-    if (size == 8) stencil_fill_kernel<double><<<grid_for(m), 256>>>(kind, d0, d1, d2, m, rp, out->ColIdx, (double *)out->Val);
-    else stencil_fill_kernel<float><<<grid_for(m), 256>>>(kind, d0, d1, d2, m, rp, out->ColIdx, (float *)out->Val);
-    SB_TRY(cudaGetLastError());
-    SB_TRY(cudaDeviceSynchronize());
-    return true;
+    if (!SB_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, bytes, cnt.get(), rp.get(), m + 1)) || !tmp.alloc(bytes) ||
+        !SB_CUDA(cub::DeviceScan::ExclusiveSum(tmp.get(), bytes, cnt.get(), rp.get(), m + 1)) ||
+        !SB_CUDA(cudaMemcpy(&nnz, rp + m, sizeof(int), cudaMemcpyDeviceToHost)))
+        return -1;
+    if (!alloc_csr(out, m, m, nnz, size) ||
+        !SB_CUDA(cudaMemcpy(out->RowPtr, rp, ((size_t)m + 1) * sizeof(int), cudaMemcpyDeviceToDevice)))
+        return gen_failed(out);
+    if (size == 8) stencil_fill_kernel<double><<<grid_for(m), 256>>>(kind, d0, d1, d2, m, out->RowPtr, out->ColIdx, (double *)out->Val);
+    else stencil_fill_kernel<float><<<grid_for(m), 256>>>(kind, d0, d1, d2, m, out->RowPtr, out->ColIdx, (float *)out->Val);
+    if (!SB_CUDA(cudaGetLastError()) || !SB_CUDA(cudaDeviceSynchronize())) return gen_failed(out);
+    return 0;
 }
 
 }  // namespace sb
@@ -199,12 +202,12 @@ extern "C" {
 
 int spmv_b200_gen_laplacian2d(int nx, int ny, unsigned long size, spmv_b200_csr *out)
 {
-    return gen_stencil(0, nx, ny, 1, size == 8 ? 8 : 4, out) ? 0 : -1;
+    return gen_stencil(0, nx, ny, 1, size == 8 ? 8 : 4, out);
 }
 
 int spmv_b200_gen_stencil27(int nx, int ny, int nz, unsigned long size, spmv_b200_csr *out)
 {
-    return gen_stencil(1, nx, ny, nz, size == 8 ? 8 : 4, out) ? 0 : -1;
+    return gen_stencil(1, nx, ny, nz, size == 8 ? 8 : 4, out);
 }
 
 int spmv_b200_gen_uniform(int m, int n, int k, unsigned long long seed, long long row0, int eighths,
@@ -212,10 +215,10 @@ int spmv_b200_gen_uniform(int m, int n, int k, unsigned long long seed, long lon
 {
     size = size == 8 ? 8 : 4;
     if (!out || m < 0 || n < 1 || k < 1 || k > kMaxRowK || (long long)m * k > 0x7fffffffLL - 8192) { set_error("bad uniform shape"); return -1; }
-    if (!alloc_csr(out, m, n, (long long)m * k, size)) return -1;
+    if (!alloc_csr(out, m, n, (long long)m * k, size)) return gen_failed(out);
     if (size == 8) uniform_kernel<double><<<grid_for(m + 1), 256>>>(m, n, k, seed, row0, eighths, out->RowPtr, out->ColIdx, (double *)out->Val);
     else uniform_kernel<float><<<grid_for(m + 1), 256>>>(m, n, k, seed, row0, eighths, out->RowPtr, out->ColIdx, (float *)out->Val);
-    if (!SB_CUDA(cudaGetLastError()) || !SB_CUDA(cudaDeviceSynchronize())) return -1;
+    if (!SB_CUDA(cudaGetLastError()) || !SB_CUDA(cudaDeviceSynchronize())) return gen_failed(out);
     return 0;
 }
 
@@ -226,26 +229,21 @@ int spmv_b200_gen_rmat(int scale, int edge_factor, unsigned long long seed, unsi
     const int m = 1 << scale;
     const long long edges = (long long)m * edge_factor;
     if (edges > 0x7fffffffLL - 8192) { set_error("rmat too large"); return -1; }
-    if (!alloc_csr(out, m, m, edges, size)) return -1;
-    unsigned long long *keys = nullptr, *sorted = nullptr;
-    if (!SB_CUDA(cudaMalloc((void **)&keys, (size_t)edges * 8)) || !SB_CUDA(cudaMalloc((void **)&sorted, (size_t)edges * 8))) return -1;
+    DeviceArray<unsigned long long> keys, sorted;
+    DeviceArray<unsigned char> tmp;
+    if (!alloc_csr(out, m, m, edges, size) || !keys.alloc((size_t)edges) || !sorted.alloc((size_t)edges)) return gen_failed(out);
     const double a = 0.57, b = 0.19, c = 0.19;
     rmat_edges_kernel<<<grid_for(edges), 256>>>(edges, scale, seed, a, a + b, a + b + c, keys);
     size_t bytes = 0;
-    cub::DeviceRadixSort::SortKeys(nullptr, bytes, keys, sorted, (int)edges, 0, 32 + scale);
-    void *tmp = nullptr;
-    bool ok = SB_CUDA(cudaMalloc(&tmp, bytes ? bytes : 1)) &&
-              SB_CUDA(cub::DeviceRadixSort::SortKeys(tmp, bytes, keys, sorted, (int)edges, 0, 32 + scale));
+    cub::DeviceRadixSort::SortKeys(nullptr, bytes, keys.get(), sorted.get(), (int)edges, 0, 32 + scale);
+    bool ok = tmp.alloc(bytes) && SB_CUDA(cub::DeviceRadixSort::SortKeys(tmp.get(), bytes, keys.get(), sorted.get(), (int)edges, 0, 32 + scale));
     if (ok) {
         const long long n = edges > m + 1 ? edges : m + 1;
         if (size == 8) rmat_finish_kernel<double><<<grid_for(n), 256>>>(edges, m, seed, sorted, out->RowPtr, out->ColIdx, (double *)out->Val);
         else rmat_finish_kernel<float><<<grid_for(n), 256>>>(edges, m, seed, sorted, out->RowPtr, out->ColIdx, (float *)out->Val);
         ok = SB_CUDA(cudaGetLastError()) && SB_CUDA(cudaDeviceSynchronize());
     }
-    cudaFree(tmp);
-    cudaFree(keys);
-    cudaFree(sorted);
-    return ok ? 0 : -1;
+    return ok ? 0 : gen_failed(out);
 }
 
 int spmv_b200_gen_x(void *device_dst, long long n, unsigned long long seed, int ones, unsigned long size)
