@@ -35,6 +35,26 @@ SPMV_B200_API void spmv_b200_clear_error(void);
  * it borrowed at create and the values given (NULL = re-read the array given at create), same method, precision and
  * stream.  Costs one create.  Returns 0, or -1 (spmv_b200_last_error()). */
 SPMV_B200_API int spmv_b200_update_values(spmv_Handle_t handle, void *Matrix_Val);
+/* A handle created with option "refresh" = 1 can take new values without a rebuild: create then keeps, for every value
+ * array it stores, a source map (4 bytes per stored slot: where in the caller's Matrix_Val, in the caller's order, the
+ * value of that slot comes from).  spmv_b200_set_values(handle, Matrix_Val) then writes the new values into every layout
+ * in place.  Matrix_Val holds nnz values of the handle's precision in the order of the ColIdx given at create (before
+ * any option-"reorder" permutation), as a HOST or DEVICE pointer; NULL = re-read the array given at create (the
+ * reference's usage: change that array in place, then call).  With an adopted device CSR only NULL or that same adopted
+ * pointer is accepted: the library never writes the caller's arrays.
+ * The call is stream-ordered on the handle's stream: every product enqueued before it uses the old values, every one
+ * enqueued after it the new ones (device or host x / y, the pipelined host path, spmv_b200_spmv_bands /
+ * spmv_b200_spmv_finish, y peers).  A DEVICE source (on the handle's device) returns without a host synchronisation
+ * and allocates nothing; the caller keeps the array unchanged until the stream has passed the refresh, as for a device
+ * x in spmv().  A HOST source has been copied out on return, so the caller may reuse the array at once; it goes
+ * through a staging array of nnz values, allocated at the first such call and owned by the handle, unless the handle's
+ * own CSR upload takes it as it is.  Afterwards every spmv() result is bit for bit what a handle newly created with
+ * these values under the same options computes.  spmv_b200_info(h, "refreshable") says whether a handle can be
+ * refreshed (0 without the option, or when a map could not be allocated at create; the handle still works).
+ * m == 0 or nnz == 0: returns 0 and does nothing.  Returns 0, or -1 (spmv_b200_last_error()): NULL handle, failed
+ * create, no option "refresh", another pointer than an adopted one, a device pointer on another device.
+ * Refresh kernels are not counted by spmv_b200_launch_count(). */
+SPMV_B200_API int spmv_b200_set_values(spmv_Handle_t handle, const void *Matrix_Val);
 
 /* ---- streams -----------------------------------------------------------------------------------
  * spmv() with HOST x/y is synchronous (reference semantics).  With DEVICE x/y it is enqueued on the
@@ -81,6 +101,9 @@ SPMV_B200_API void spmv_b200_sync(spmv_Handle_t handle);
  *                     "auto_method") too.  0 (default) = run what Function says
  *   "pipeline"        1 (default) = spmv() with HOST x and y on a Method_Parallel handle overlaps the PCIe
  *                     copies with the kernels (x in pieces, y in row chunks); 0 = copy, run, copy
+ *   "refresh"         1 = create also keeps a source map of every value array the handle stores, so that
+ *                     spmv_b200_set_values can refresh the values in place (4 bytes per stored slot); 0 (default) = no
+ *                     maps, create is unchanged
  * Returns 0, or -1 for an unknown key. */
 SPMV_B200_API int spmv_b200_set_option(const char *key, long long value);
 SPMV_B200_API long long spmv_b200_get_option(const char *key);
@@ -90,7 +113,7 @@ SPMV_B200_API long long spmv_b200_get_option(const char *key);
  * SPMV_B200_KERNEL_*), "requested", "m", "n", "nnz", "tpr", "parts", "tiles", "sigma", "banner",
  * "slices", "padded_nnz", "csr5_p", "csr5_sigma", "csr5_num_offsets", "csr5_tail_start", "device",
  * "has_empty_rows", "x_bands", "seg_bands", "segments", "band_cols", "active_rows", "owns_csr", "released_csr",
- * "layout_fallbacks", "auto_method", "values_snapshotted", "pipeline", "dev_l2_bytes".  Returns -1 for an unknown key /
+ * "layout_fallbacks", "auto_method", "values_snapshotted", "refreshable", "pipeline", "dev_l2_bytes".  Returns -1 for an unknown key /
  * NULL handle.
  *
  * spmv_b200_structure: copy a device layout array to HOST memory.  Returns its size in bytes (call

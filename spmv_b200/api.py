@@ -39,7 +39,8 @@ EXPORTED_FUNCTIONS = [
     "spmv_b200_set_y_peers", "spmv_b200_ipc_export", "spmv_b200_ipc_open", "spmv_b200_ipc_close",
     "spmv_b200_recommend_method", "spmv_b200_bands", "spmv_b200_band_columns", "spmv_b200_spmv_bands",
     "spmv_b200_spmv_finish", "spmv_b200_memcpy_async", "spmv_b200_stream_write32", "spmv_b200_stream_wait32_geq",
-    "spmv_b200_reorder", "spmv_b200_permute_csr", "spmv_b200_update_values", "spmv_b200_live_allocations"]
+    "spmv_b200_reorder", "spmv_b200_permute_csr", "spmv_b200_update_values", "spmv_b200_live_allocations",
+    "spmv_b200_set_values"]
 EXPORTED_DATA = ["Methods_names", "Vectorized_names", "funcNames"]
 
 
@@ -114,6 +115,7 @@ def lib() -> C.CDLL:
     L.spmv_b200_spmv_bands.argtypes = [spmv_Handle_t, i, i, vp]
     L.spmv_b200_spmv_finish.argtypes = [spmv_Handle_t, vp]
     L.spmv_b200_update_values.argtypes = [spmv_Handle_t, vp]
+    L.spmv_b200_set_values.argtypes = [spmv_Handle_t, vp]
     L.spmv_b200_reorder.argtypes = [i, vp, vp, vp]
     L.spmv_b200_permute_csr.argtypes = [i, vp, vp, vp, ul, vp, vp, vp, vp]
     L.spmv_b200_memcpy_async.argtypes = [vp, vp, C.c_size_t, vp]
@@ -236,6 +238,29 @@ class Handle:
         if lib().spmv_b200_update_values(self.h, _addr(Matrix_Val) if Matrix_Val is not None else None) != 0:
             raise RuntimeError("spmv_b200_update_values failed: " + last_error())
 
+    def set_values(self, Matrix_Val=None):
+        """New values on the same pattern, in place and stream-ordered (spmv_b200_set_values; the handle must have been
+        created with option "refresh").  Matrix_Val: nnz values of the handle's precision in the order of the ColIdx
+        given at create, as numpy, CPU torch or CUDA torch; None re-reads the array given at create.  A CUDA source is
+        kept alive here until the next set_values or destroy, since the refresh reads it on the stream."""
+        addr = None
+        if Matrix_Val is not None:
+            if isinstance(Matrix_Val, np.ndarray):
+                floating, itemsize = Matrix_Val.dtype.kind == "f", Matrix_Val.dtype.itemsize
+                count, contiguous = Matrix_Val.size, Matrix_Val.flags.c_contiguous
+            else:
+                floating, itemsize = Matrix_Val.is_floating_point(), Matrix_Val.element_size()
+                count, contiguous = Matrix_Val.numel(), Matrix_Val.is_contiguous()
+            nnz = self.info("nnz")
+            if not floating or itemsize != self.size:
+                raise ValueError(f"set_values: the handle holds {8 * self.size}-bit floats, got {Matrix_Val.dtype}")
+            if count != nnz or not contiguous:
+                raise ValueError(f"set_values: need {nnz} contiguous values, got {count}")
+            addr = _addr(Matrix_Val)
+        if lib().spmv_b200_set_values(self.h, addr) != 0:
+            raise RuntimeError(last_error())
+        self.values_source = Matrix_Val if getattr(Matrix_Val, "is_cuda", False) else None
+
     def bands(self) -> int:
         """Column bands that can be staged one by one (1: use spmv())."""
         return int(lib().spmv_b200_bands(self.h))
@@ -264,6 +289,7 @@ class Handle:
         if getattr(self, "h", None):
             spmv_destory_handle(self.h)
             self.h = None
+        self.values_source = None
 
     def __del__(self):
         try:

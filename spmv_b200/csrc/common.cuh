@@ -115,6 +115,10 @@ struct DeviceState {
     int dev_sms = 0;
     long long dev_l2 = 0;
     int layout_fallbacks = 0;       // optional layouts (band copy, band segments, row bins) that could not be built
+    // option "refresh": every value array below keeps its source map (refresh.cuh) in its own group, so that dropping a
+    // layout drops its map too.  Cleared at create when a map could not be built: the handle then cannot be refreshed
+    bool refresh = false;
+    bool map_failed = false;
     int n_peers = 0;                // spmv_b200_set_y_peers
     void *peers[kMaxPeers] = {};
 
@@ -122,7 +126,7 @@ struct DeviceState {
     // array).  rowptr / col / val only point at one of the two.
     int *rowptr = nullptr, *col = nullptr;
     void *val = nullptr;
-    struct CsrUpload { DeviceArray<int> rowptr, col; DeviceBytes val; } upload;
+    struct CsrUpload { DeviceArray<int> rowptr, col; DeviceBytes val; DeviceArray<int> map; } upload;  // map: under "reorder" only
     bool released_csr = false;      // the upload was freed after a re-laid-out copy took over
 
     // pageable host x / y that keep coming back (the reference's drivers reuse one X and one Y for every call) are
@@ -134,7 +138,7 @@ struct DeviceState {
     bool pin_host = false;
     // staging for host-side x / y; the pipelined host path (CSR-vector kernel) copies x in pieces on s_in,
     // computes row chunks as soon as their prefix of x has arrived, and returns finished chunks of y on s_out
-    struct Staging { DeviceBytes x, y; } stage;
+    struct Staging { DeviceBytes x, y, val; } stage;  // val: host values of spmv_b200_set_values, when no upload takes them
     bool pipeline = false;
     cudaStream_t s_in = nullptr, s_out = nullptr;
     cudaEvent_t ev_in[kMaxPieces] = {}, ev_out[kPipeChunks] = {}, ev_start = nullptr, ev_x = nullptr;
@@ -150,7 +154,7 @@ struct DeviceState {
     void *a_val = nullptr;
     int x_bands = 1, band_cols = 0;
     double far_fraction = -1.0;     // share of entries far from the diagonal (automatic band decision)
-    struct BandCopy { DeviceArray<int> rowptr, col; DeviceBytes val, y; } v;
+    struct BandCopy { DeviceArray<int> rowptr, col, map; DeviceBytes val, y; } v;
     // Method_Balanced: row blocks; ref_splitter mirrors the reference with the caller's nthreads
     struct Splitters {
         int parts = 0, ref_T = 0;
@@ -171,7 +175,7 @@ struct DeviceState {
     struct Sell {
         int sigma = 0, banner = 0, slices = 0, variant = 0;
         long long padded = 0;
-        DeviceArray<int> perm, width, full, col;
+        DeviceArray<int> perm, width, full, col, map;
         DeviceArray<long long> slice_ptr;
         DeviceBytes val;
     } sell;
@@ -192,7 +196,7 @@ struct DeviceState {
     struct Csr5 {
         int sigma = 0, p = 0, bit_y = 0, bit_ss = 0, num_offsets = 0, tail_start = 0;
         DeviceArray<uint32_t> tile_ptr, tile_desc;
-        DeviceArray<int> off_ptr, off, col;
+        DeviceArray<int> off_ptr, off, col, map;
         DeviceBytes val;
     } c5;
     // hyper-sparse column bands as band segments (band_seg.cuh): x_bands = K but the active view stays the CSR
@@ -209,6 +213,7 @@ struct DeviceState {
         bool mask64 = false;            // K > 32: 64-bit row masks
         DeviceArray<int> col;           // column index | segment-end bit 31
         DeviceBytes ent_val;            // values, band-major
+        DeviceArray<int> map;           // source map of ent_val [ptr[K]]
         DeviceBytes mask;               // per row: bands in which it has a segment
         DeviceArray<int4> tile_ent;     // per tile: (first slot, entries, L2-prefetch duty: first x element, elements)
         DeviceArray<int> tile_seg0;     // per 256-entry chunk of a tile (8 per tile): index of its first segment sum

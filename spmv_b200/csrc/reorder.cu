@@ -42,7 +42,41 @@ void permute_values(int m, const int *rowptr, const int *col, const V *val, cons
     }
 }
 
+template <typename V>
+int permute_csr(int m, const int *RowPtr, const int *ColIdx, const V *Val, const int *index, int *RowPtr_out, int *ColIdx_out,
+                V *Val_out)
+{
+    if (m < 0 || !RowPtr || !index || !RowPtr_out) return -1;
+    const int nnz = RowPtr[m] - RowPtr[0];
+    if (nnz > 0 && (!ColIdx || !Val || !ColIdx_out || !Val_out)) return -1;
+    std::vector<int> inv((size_t)m, -1);
+    for (int i = 0; i < m; ++i) {
+        if (index[i] < 0 || index[i] >= m || inv[index[i]] != -1) return -1;  // not a permutation
+        inv[index[i]] = i;
+    }
+    for (int j = RowPtr[0]; j < RowPtr[m]; ++j)
+        if (ColIdx[j] < 0 || ColIdx[j] >= m) return -1;  // a symmetric permutation needs a square pattern
+    RowPtr_out[0] = 0;
+    for (int i = 0; i < m; ++i) RowPtr_out[i + 1] = RowPtr_out[i] + (RowPtr[index[i] + 1] - RowPtr[index[i]]);
+    permute_values<V>(m, RowPtr, ColIdx, Val, index, inv.data(), RowPtr_out, ColIdx_out, Val_out);
+    return 0;
+}
+
 }  // namespace
+
+namespace sb {
+
+// Options "reorder" + "refresh": pos_out[d] = 1 + the caller's position of the entry A' stores at d (the source map of
+// the permuted upload, refresh.cuh), placed exactly as spmv_b200_permute_csr places the values.
+int permute_positions(int m, const int *RowPtr, const int *ColIdx, const int *index, int *RowPtr_out, int *ColIdx_out, int *pos_out)
+{
+    if (m < 0 || !RowPtr || RowPtr[m] < 0) return -1;
+    std::vector<int> pos((size_t)RowPtr[m]);  // the values are read as Val[j], j in [RowPtr[0], RowPtr[m])
+    std::iota(pos.begin(), pos.end(), 1);
+    return permute_csr<int>(m, RowPtr, ColIdx, pos.data(), index, RowPtr_out, ColIdx_out, pos_out);
+}
+
+}  // namespace sb
 
 extern "C" {
 
@@ -82,23 +116,9 @@ int spmv_b200_reorder(int m, const int *RowPtr, const int *ColIdx, int *index_ou
 int spmv_b200_permute_csr(int m, const int *RowPtr, const int *ColIdx, const void *Val, unsigned long size,
                           const int *index, int *RowPtr_out, int *ColIdx_out, void *Val_out)
 {
-    if (m < 0 || !RowPtr || !index || !RowPtr_out) return -1;
-    const int nnz = RowPtr[m] - RowPtr[0];
-    if (nnz > 0 && (!ColIdx || !Val || !ColIdx_out || !Val_out)) return -1;
-    std::vector<int> inv((size_t)m, -1);
-    for (int i = 0; i < m; ++i) {
-        if (index[i] < 0 || index[i] >= m || inv[index[i]] != -1) return -1;  // not a permutation
-        inv[index[i]] = i;
-    }
-    for (int j = RowPtr[0]; j < RowPtr[m]; ++j)
-        if (ColIdx[j] < 0 || ColIdx[j] >= m) return -1;  // a symmetric permutation needs a square pattern
-    RowPtr_out[0] = 0;
-    for (int i = 0; i < m; ++i) RowPtr_out[i + 1] = RowPtr_out[i] + (RowPtr[index[i] + 1] - RowPtr[index[i]]);
     if (size == sizeof(double))
-        permute_values<double>(m, RowPtr, ColIdx, (const double *)Val, index, inv.data(), RowPtr_out, ColIdx_out, (double *)Val_out);
-    else
-        permute_values<float>(m, RowPtr, ColIdx, (const float *)Val, index, inv.data(), RowPtr_out, ColIdx_out, (float *)Val_out);
-    return 0;
+        return permute_csr<double>(m, RowPtr, ColIdx, (const double *)Val, index, RowPtr_out, ColIdx_out, (double *)Val_out);
+    return permute_csr<float>(m, RowPtr, ColIdx, (const float *)Val, index, RowPtr_out, ColIdx_out, (float *)Val_out);
 }
 
 }  // extern "C"

@@ -20,8 +20,12 @@
 #include "csr5.cuh"
 #include "long_rows.cuh"
 #include "band_seg.cuh"
+#include "refresh.cuh"
 
 namespace sb {
+
+int permute_positions(int m, const int *RowPtr, const int *ColIdx, const int *index, int *RowPtr_out, int *ColIdx_out,
+                      int *pos_out);  // reorder.cu
 
 // ------------------------------------------------------------------------------------------------
 // error latch, launch counter, options
@@ -56,7 +60,7 @@ struct Options {
                                        {"force_merge", 0}, {"sell_cap", 1024},
                                        {"long_thr", 0},    {"pipeline", 1},   {"sell_variant", -1},
                                        {"seg_bands", 0},    {"seg_prefetch", 1}, {"seg_ctas", 2},  {"auto", 0},     {"reorder", 0},    {"row_bins", 1},
-                                       {"pin_host", 1}};
+                                       {"pin_host", 1},     {"refresh", 0}};
     std::map<std::string, bool> user_set;
 };
 static Options &options()
@@ -152,6 +156,39 @@ static void note_host_buffer(DeviceState *st, int which, const void *p, size_t b
     if (a.type != cudaMemoryTypeUnregistered) { slot.seen = -1; return; }  // already pinned by the caller
     if (cudaHostRegister(const_cast<void *>(p), bytes, cudaHostRegisterDefault) == cudaSuccess) slot.registered = true;
     else { cudaGetLastError(); slot.seen = -1; }  // e.g. registered through another handle: leave it alone
+}
+
+// Option "refresh": a source map that cannot be made costs the handle its refresh, never its layout.
+static void map_failure(DeviceState *st)
+{
+    cudaGetLastError();
+    spmv_b200_clear_error();
+    st->map_failed = true;
+}
+
+// Source map of the value array `val` a builder reads: the band-major copy's, the permuted upload's (option
+// "reorder"), or -- the CSR in the caller's own order -- k + 1 at k, made in `tmp`.
+static const int *source_map_of(DeviceState *st, const void *val, DeviceArray<int> &tmp)
+{
+    if (val == st->v.val.get()) return st->v.map;
+    if (st->upload.map) return st->upload.map;
+    if (!tmp.alloc((size_t)st->nnz)) return nullptr;
+    map_iota_kernel<<<blocks_for(st->nnz), kThreads, 0, st->stream>>>(st->nnz, tmp);
+    return tmp;
+}
+
+// The source map of a layout's value array: `move(src, map)` enqueues the builder's value-moving kernel again with
+// T = int, reading the source map of `val` (what the builder read the values from) and writing `map` in place of
+// the values.  Padding slots get the builder's own zero, which is the map's "no source".
+template <typename Move>
+static void build_map(DeviceState *st, const void *val, DeviceArray<int> &map, size_t count, Move move)
+{
+    if (!st->refresh || st->map_failed) return;
+    DeviceArray<int> tmp;
+    const int *src = source_map_of(st, val, tmp);
+    if (src && map.alloc(count) && move(src, map.get()) && SB_CUDA(cudaGetLastError())) return;
+    map.reset();
+    map_failure(st);
 }
 
 static void free_state(DeviceState *st)
@@ -267,6 +304,10 @@ static bool build_band_major(DeviceState *st)
         ok = SB_CUDA(cudaGetLastError()) && SB_CUDA(cudaStreamSynchronize(st->stream));
     }
     if (!ok) return give_up();
+    build_map(st, st->val, st->v.map, (size_t)st->nnz, [&](const int *src, int *map) {
+        band_scatter_kernel<int><<<blocks_for(m), kThreads, 0, st->stream>>>(m, K, band_cols, st->rowptr, st->col, src, st->v.rowptr, st->v.col, map);
+        return true;
+    });
     st->x_bands = K;
     st->band_cols = band_cols;
     st->a_m = (int)vm; st->a_rowptr = st->v.rowptr; st->a_col = st->v.col; st->a_val = st->v.val.get();
@@ -486,6 +527,11 @@ static bool build_sell(DeviceState *st)
         st->sell.slices, st->a_rowptr, st->a_col, (const T *)st->a_val, st->sell.perm, st->sell.slice_ptr, st->sell.col,
         st->sell.val.as<T>());
     SB_TRY(cudaGetLastError());
+    build_map(st, st->a_val, st->sell.map, (size_t)st->sell.padded, [&](const int *src, int *map) {
+        sell_fill_kernel<int><<<blocks_for((long long)st->sell.slices * 32), kThreads, 0, st->stream>>>(
+            st->sell.slices, st->a_rowptr, st->a_col, src, st->sell.perm, st->sell.slice_ptr, st->sell.col, map);
+        return true;
+    });
     return true;
 }
 
@@ -536,6 +582,10 @@ static bool build_csr5(DeviceState *st)
     c5_transpose_kernel<T><<<blocks_for(st->nnz), kThreads, 0, st->stream>>>(
         st->nnz, sigma, p, st->c5.tile_ptr, st->a_col, (const T *)st->a_val, st->c5.col, st->c5.val.as<T>());
     SB_TRY(cudaGetLastError());
+    build_map(st, st->a_val, st->c5.map, (size_t)st->nnz, [&](const int *src, int *map) {
+        c5_transpose_kernel<int><<<blocks_for(st->nnz), kThreads, 0, st->stream>>>(st->nnz, sigma, p, st->c5.tile_ptr, st->a_col, src, st->c5.col, map);
+        return true;
+    });
     return alloc_carries(st, p);
 }
 
@@ -608,6 +658,12 @@ static bool build_band_seg_t(DeviceState *st)
         if (ok) {
             bseg_gather_kernel<T><<<blocks_for(nnz), kThreads, 0, st->stream>>>(nnz, idx_out, key_out, ent_row, st->col, (const T *)st->val, d_tab,
                                                                                d_tab + (K + 1), st->seg.col, st->seg.ent_val.as<T>());
+            build_map(st, st->val, st->seg.map, (size_t)slot, [&](const int *src, int *map) {  // the gaps between bands stay 0
+                if (!SB_CUDA(cudaMemsetAsync(map, 0, (size_t)slot * sizeof(int), st->stream))) return false;
+                bseg_gather_kernel<int><<<blocks_for(nnz), kThreads, 0, st->stream>>>(nnz, idx_out, key_out, ent_row, st->col, src, d_tab,
+                                                                                     d_tab + (K + 1), st->seg.col, map);
+                return true;
+            });
             bseg_tile_kernel<<<blocks_for((long long)tiles * 32), kThreads, 0, st->stream>>>(tiles, K, st->band_cols, st->n, st->vsize, d_tab + 3 * (K + 1), d_tab + (K + 1), d_tab + 2 * (K + 1),
                                                                                              st->seg.col, st->seg.tile_ent, tile_segs, d_cross);
             bseg_group_count_kernel<MaskT><<<blocks_for((long long)st->seg.groups * 32), kThreads, 0, st->stream>>>(m, K, st->seg.groups, st->seg.mask.as<MaskT>(), blk_cnt);
@@ -738,8 +794,9 @@ static int auto_pick_method(DeviceState *st)
     return Method_SellCSigma;
 }
 
+// reorder_map: the source map of the permuted values under options "reorder" and "refresh" (host, nnz ints)
 static bool build_state(DeviceState *st, spmv_Handle *h, int m, int n, int *RowPtr, int *ColIdx, void *Val,
-                        int method)
+                        int method, const int *reorder_map = nullptr)
 {
     st->requested = method;
     int ndev = 0;
@@ -791,6 +848,9 @@ static bool build_state(DeviceState *st, spmv_Handle *h, int m, int n, int *RowP
         if (st->nnz > 0) {
             SB_TRY(cudaMemcpy(st->col, ColIdx, (size_t)st->nnz * sizeof(int), cudaMemcpyHostToDevice));
             SB_TRY(cudaMemcpy(st->val, Val, (size_t)st->nnz * st->vsize, cudaMemcpyHostToDevice));
+            if (reorder_map && !st->map_failed &&
+                !(up.map.alloc((size_t)st->nnz) && SB_CUDA(cudaMemcpy(up.map, reorder_map, (size_t)st->nnz * sizeof(int), cudaMemcpyHostToDevice))))
+                map_failure(st);
         }
     }
 
@@ -827,6 +887,14 @@ static bool build_state(DeviceState *st, spmv_Handle *h, int m, int n, int *RowP
         st->rowptr = st->col = nullptr;
         st->val = nullptr;
         st->released_csr = true;
+    }
+    if (st->map_failed) {  // a handle that cannot refresh every array it stores keeps none of the maps
+        st->refresh = false;
+        st->upload.map.reset();
+        st->v.map.reset();
+        st->sell.map.reset();
+        st->c5.map.reset();
+        st->seg.map.reset();
     }
     return true;
 }
@@ -1219,6 +1287,7 @@ static void create_into(spmv_Handle *h, BASIC_INT_TYPE m, BASIC_INT_TYPE n, BASI
     // deviation, include/spmv.h)
     DeviceState *st = new DeviceState();
     h->extraHandle = st;
+    st->refresh = opt("refresh") != 0;
     // Option "reorder": the reference's level-3 hook (common.c:144-156, compiled out upstream).  Same condition as
     // there (square, > 8096 rows, > 100000 non-zeros), HOST arrays only; the device layout is then built from
     // A' = P A P^T and the permutation is handed to the caller in handle->index (reorder.cu).
@@ -1239,7 +1308,13 @@ static void create_into(spmv_Handle *h, BASIC_INT_TYPE m, BASIC_INT_TYPE n, BASI
             index[m] = m;
             h->index = index;           // freed by spmv_clear_handle
             h->Level_3_opt_used = 1;
-            st->ok = build_state(st, h, m, n, p_rowptr.data(), p_col.data(), p_val.data(), method);
+            std::vector<int> p_map;     // option "refresh": where every permuted value comes from
+            if (st->refresh) {
+                p_map.resize(nnz);
+                // (rewrites p_rowptr / p_col with what they already hold: the same permutation)
+                if (permute_positions(m, RowPtr, ColIdx, index, p_rowptr.data(), p_col.data(), p_map.data()) != 0) st->map_failed = true;
+            }
+            st->ok = build_state(st, h, m, n, p_rowptr.data(), p_col.data(), p_val.data(), method, p_map.empty() ? nullptr : p_map.data());
             return;
         }
         free(index);
@@ -1338,6 +1413,73 @@ int spmv_b200_update_values(spmv_Handle_t handle, void *Matrix_Val)
     DeviceState *fresh = state_of(handle);
     if (fresh) fresh->stream = stream;
     return fresh && fresh->ok ? 0 : -1;
+}
+
+// Option "refresh": new values on the handle's stream, through the source maps kept at create (refresh.cuh).  The
+// owned upload in the caller's order takes the values as they are (one copy); every other value array is gathered
+// from them in one launch.
+int spmv_b200_set_values(spmv_Handle_t handle, const void *Matrix_Val)
+{
+    DeviceState *st = state_of(handle);
+    if (!st) { set_error("spmv_b200_set_values: NULL handle"); return -1; }
+    if (!st->ok) { set_error("spmv_b200_set_values: the handle's create failed"); return -1; }
+    if (!st->refresh) {
+        set_error("spmv_b200_set_values: the handle keeps no source maps (create it with option \"refresh\" = 1; "
+                  "spmv_b200_info(h, \"refreshable\") = 0)");
+        return -1;
+    }
+    std::lock_guard<std::mutex> lock(st->mu);
+    DeviceGuard guard(st->device);
+    if (st->m == 0 || st->nnz == 0) return 0;
+    const void *src = Matrix_Val ? Matrix_Val : handle->Matrix_Val;
+    if (st->val && !st->upload.val.get() && src != st->val) {  // an adopted device CSR is the caller's: never written
+        set_error("spmv_b200_set_values: the handle adopted the caller's device Matrix_Val %p; refresh it in place and pass "
+                  "NULL or that pointer (got %p)", st->val, src);
+        return -1;
+    }
+    cudaPointerAttributes a;
+    bool on_device = false;
+    if (cudaPointerGetAttributes(&a, src) != cudaSuccess) cudaGetLastError();
+    else on_device = a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
+    if (on_device && a.type == cudaMemoryTypeDevice && a.device != st->device) {
+        set_error("spmv_b200_set_values: Matrix_Val is on device %d, the handle on device %d", a.device, st->device);
+        return -1;
+    }
+    RefreshTable tab = {};
+    long long quads = 0;
+    auto add = [&](void *dst, const int *map, long long count) {
+        if (!map || count <= 0 || tab.n == kRefreshMaxTargets) return;
+        tab.t[tab.n++] = {dst, map, count, quads};
+        quads += (count + 3) / 4;
+    };
+    add(st->upload.val.get(), st->upload.map, st->nnz);
+    add(st->v.val.get(), st->v.map, st->nnz);
+    add(st->sell.val.get(), st->sell.map, st->sell.padded);
+    add(st->c5.val.get(), st->c5.map, st->nnz);
+    add(st->seg.ent_val.get(), st->seg.map, st->seg.ptr[st->seg.bands]);
+    const size_t bytes = (size_t)st->nnz * st->vsize;
+    const void *from = src;  // what the gather reads
+    void *copy_to = nullptr;
+    if (st->upload.val.get() && !st->upload.map) copy_to = st->upload.val.get();  // the identity target
+    else if (!on_device && tab.n > 0) {
+        if (!st->stage.val.get() && !st->stage.val.alloc((size_t)st->nnz, st->vsize)) return -1;
+        copy_to = st->stage.val.get();
+    }
+    if (copy_to) {
+        if (!SB_CUDA(cudaMemcpyAsync(copy_to, src, bytes, cudaMemcpyDefault, st->stream))) return -1;
+        from = copy_to;
+    }
+    if (!on_device) {  // the caller may reuse a host array at once: wait for its copy alone
+        if (!st->ev_x && !SB_CUDA(cudaEventCreateWithFlags(&st->ev_x, cudaEventDisableTiming))) return -1;
+        if (!SB_CUDA(cudaEventRecord(st->ev_x, st->stream))) return -1;
+    }
+    if (tab.n > 0) {  // (not on the spmv() path: not in spmv_b200_launch_count)
+        if (st->vsize == 8) value_refresh_kernel<double><<<blocks_for(quads), kThreads, 0, st->stream>>>(tab, (const double *)from);
+        else value_refresh_kernel<float><<<blocks_for(quads), kThreads, 0, st->stream>>>(tab, (const float *)from);
+        if (!SB_CUDA(cudaGetLastError())) return -1;
+    }
+    if (!on_device && !SB_CUDA(cudaEventSynchronize(st->ev_x))) return -1;
+    return 0;
 }
 
 // ================================================================================================
@@ -1570,6 +1712,7 @@ long long spmv_b200_info(spmv_Handle_t handle, const char *key)
     if (k == "csr5_tail_start") return st->c5.tail_start;
     if (k == "pipeline") return st->pipeline;
     if (k == "values_snapshotted") return 1;
+    if (k == "refreshable") return st->refresh;
     if (k == "binned") return st->lr.binned;
     if (k == "pinned_host_buffers") return (int)st->pin[0].registered + (int)st->pin[1].registered;
     if (k == "long_rows") return st->lr.rows;
