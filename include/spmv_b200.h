@@ -67,7 +67,7 @@ SPMV_B200_API void spmv_b200_sync(spmv_Handle_t handle);
  *   "sell_sigma"      sorting window of Method_SellCSigma (multiple of 32, <= 4096; default 256)
  *   "csr5_sigma"      nnz per lane of a CSR5 tile (4, 8 or 16; default 0 = 16, or 8 below 2^25 non-zeros)
  *   "block_nnz"       nnz per row block of Method_Balanced (default 512)
- *   "tile_items"      items per thread of the merge-path / equal-nnz tiles (4..16; default 8)
+ *   "tile_items"      items per thread of the merge-path / equal-nnz tiles (4 or 8; default 8, any other value is 8)
  *   "tpr"             force threads-per-row of Method_Parallel (power of two <= 32; 0 = from mean)
  *   "x_bands"         column bands of the band-major layout that keeps the gathered slice of x inside L2
  *                     (0 = automatic from n and the L2 size, 1 = off, 2..64 forced); every method except
@@ -76,6 +76,10 @@ SPMV_B200_API void spmv_b200_sync(spmv_Handle_t handle);
  *                     merged per row in a second pass), for matrices whose bands would hold fewer than 4 non-zeros
  *                     per row (0 = automatic, -1 = never, 2..64 forced); replaces the kernel of every method except
  *                     Method_Serial
+ *   "seg_ctas"        persistent CTAs per SM of the band-segment pass 1 (2 = default, or 3); read at a handle's FIRST
+ *                     band-segment launch, not at create
+ *   "seg_prefetch"    L2 prefetch of the next band's slice of x in the band-segment pass 1 (0 = never, 1 = automatic
+ *                     (default), 2 = always); read once per process, at the first band-segment launch; no effect on y
  *   "force_merge"     1 = Method_Balanced2 always runs the merge-path kernel (default: only when a row is
  *                     long enough to starve a row block, the reference's own Balanced2 -> Balanced rule)
  *   "sell_variant"    SELL kernel flavour: -1 = automatic (default: 2 on diagonal-local matrices, else 0),
@@ -110,9 +114,11 @@ SPMV_B200_API long long spmv_b200_get_option(const char *key);
 
 /* ---- introspection -----------------------------------------------------------------------------
  * spmv_b200_info: scalar facts about a handle.  Keys: "kernel" (internal kernel family, see
- * SPMV_B200_KERNEL_*), "requested", "m", "n", "nnz", "tpr", "parts", "tiles", "sigma", "banner",
- * "slices", "padded_nnz", "csr5_p", "csr5_sigma", "csr5_num_offsets", "csr5_tail_start", "device",
- * "has_empty_rows", "x_bands", "seg_bands", "segments", "band_cols", "active_rows", "owns_csr", "released_csr",
+ * SPMV_B200_KERNEL_*), "requested", "m", "n", "nnz", "tpr", "parts", "tiles", "tile_items", "sigma", "banner",
+ * "slices", "sell_variant" (0 or 2: the SELL kernel flavour that runs), "padded_nnz", "csr5_p", "csr5_sigma",
+ * "csr5_num_offsets", "csr5_tail_start", "device", "has_empty_rows", "x_bands", "seg_bands", "segments", "seg_cross",
+ * "seg_ctas" (persistent CTAs per SM of the band-segment pass 1; 0 until the handle's first launch), "band_cols",
+ * "active_rows", "owns_csr", "released_csr",
  * "layout_fallbacks", "auto_method", "values_snapshotted", "refreshable", "pipeline", "dev_l2_bytes".  Returns -1 for an unknown key /
  * NULL handle.
  *

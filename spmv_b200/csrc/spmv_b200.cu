@@ -1703,6 +1703,7 @@ long long spmv_b200_info(spmv_Handle_t handle, const char *key)
     if (k == "sigma") return st->sell.sigma;
     if (k == "banner") return st->sell.banner;
     if (k == "slices") return st->sell.slices;
+    if (k == "sell_variant") return st->sell.variant;
     if (k == "padded_nnz") return st->sell.padded;
     if (k == "csr5_p") return st->c5.p;
     if (k == "csr5_sigma") return st->c5.sigma;
@@ -1725,6 +1726,7 @@ long long spmv_b200_info(spmv_Handle_t handle, const char *key)
     if (k == "seg_bands") return st->seg.bands;
     if (k == "segments") return st->seg.total;
     if (k == "seg_cross") return st->seg.cross;
+    if (k == "seg_ctas") return st->seg.ctas;
     if (k == "layout_fallbacks") return st->layout_fallbacks;
     if (k == "band_cols") return st->band_cols;
     if (k == "far_permille") return (long long)(st->far_fraction * 1000.0);
