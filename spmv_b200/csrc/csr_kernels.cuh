@@ -75,15 +75,12 @@ csr_reforder_kernel(int m, const int *__restrict__ rowptr, const int *__restrict
 // that allocate in L1 (L2 evict-first): the tpr lanes of a row walk it with stride tpr, so one 32-byte sector
 // serves several lanes and is fetched from L2 once.  (Measured and dropped in round 1, fraction of the HBM peak for
 // aligned 4-element chunk loads / a plain scalar loop / this: C1 0.50 / 0.60 / 0.62, C2 0.385 / 0.36 / 0.40,
-// C4 0.69 / 0.74 / 0.89.  The template parameter is kept as the name of the scheme.)
+// C4 0.69 / 0.74 / 0.89.)
 // ------------------------------------------------------------------------------------------------
-template <typename T, int MODE>
-__device__ __forceinline__ T row_partial(int start, int end, int sl, int tpr, int nnz4,
-                                         const int *__restrict__ col, const T *__restrict__ val,
-                                         const T *__restrict__ x, uint64_t pl, uint64_t pf)
+template <typename T>
+__device__ __forceinline__ T row_partial(int start, int end, int sl, int tpr, const int *__restrict__ col,
+                                         const T *__restrict__ val, const T *__restrict__ x, uint64_t pl, uint64_t pf)
 {
-    static_assert(MODE == 4, "only the batched scheme is instantiated");
-    (void)nnz4;
     // A lane adds at most kBlock / 2 batches into one FMA chain: a lane that walks a very long row alone (small
     // tpr on a skewed matrix) folds block sums instead of piling ~sqrt(len) ulps into a single chain, which would
     // miss the 8*eps*sum|a x| bound.  Fixed order either way: bitwise reproducible.
@@ -119,9 +116,9 @@ __device__ __forceinline__ T row_partial(int start, int end, int sl, int tpr, in
 // the OpenMP row loop becomes a grid of sub-warps, TPR lanes per row with TPR = 2^k ~ mean row
 // length / 4 chosen at create.  Fixed butterfly reduction => bitwise reproducible.
 // ------------------------------------------------------------------------------------------------
-template <typename T, int TPR, int VEC, bool PEERS, bool FUSE>
+template <typename T, int TPR, bool PEERS, bool FUSE>
 __global__ void __launch_bounds__(kThreads)
-csr_vector_kernel(int row0, int m, int nnz, int long_thr, const int *__restrict__ rowptr, const int *__restrict__ col,
+csr_vector_kernel(int row0, int m, int long_thr, const int *__restrict__ rowptr, const int *__restrict__ col,
                   const T *__restrict__ val, const T *__restrict__ x, T *__restrict__ y, const PeerList<T> peers,
                   int fuse_bands, int band_m, const T *__restrict__ vy)
 {
@@ -148,7 +145,7 @@ csr_vector_kernel(int row0, int m, int nnz, int long_thr, const int *__restrict_
             for (int b = 1; b < fuse_bands; ++b) prev += ldg_stream(vy + (size_t)b * band_m + out_row);
         }
     }
-    T sum = row_partial<T, VEC>(start, end, sl, TPR, nnz & ~3, col, val, x, pl, pf);
+    T sum = row_partial<T>(start, end, sl, TPR, col, val, x, pl, pf);
     sum = group_sum_c<T, TPR>(sum);
     if (valid && sl == 0) store_y<PEERS>(y, peers, out_row, FUSE ? prev + sum : sum);
 }
@@ -158,7 +155,7 @@ csr_vector_kernel(int row0, int m, int nnz, int long_thr, const int *__restrict_
 // so a warp only ever holds rows of similar length (no lane group waiting for a 100-entry neighbour).
 template <typename T, int TPR, bool PEERS>
 __global__ void __launch_bounds__(kThreads)
-csr_vector_list_kernel(int count, int nnz, const int *__restrict__ list, const int *__restrict__ rowptr,
+csr_vector_list_kernel(int count, const int *__restrict__ list, const int *__restrict__ rowptr,
                        const int *__restrict__ col, const T *__restrict__ val, const T *__restrict__ x,
                        T *__restrict__ y, const PeerList<T> peers)
 {
@@ -170,7 +167,7 @@ csr_vector_list_kernel(int count, int nnz, const int *__restrict__ list, const i
     const int row = valid ? list[idx] : 0;
     const int start = valid ? rowptr[row] : 0;
     const int end = valid ? rowptr[row + 1] : 0;
-    T sum = row_partial<T, 4>(start, end, sl, TPR, nnz & ~3, col, val, x, pl, pf);
+    T sum = row_partial<T>(start, end, sl, TPR, col, val, x, pl, pf);
     sum = group_sum_c<T, TPR>(sum);
     if (valid && sl == 0) store_y<PEERS>(y, peers, row, sum);
 }
@@ -193,8 +190,8 @@ __global__ void row_bin_kernel(int m, const int *__restrict__ rowptr, unsigned c
 // mean row length, so short-row and long-row regions of one matrix each get a fitting geometry.
 // Block 0 starts at row 0 (the reference leaves leading empty rows unwritten).
 // ------------------------------------------------------------------------------------------------
-template <typename T, int VEC, bool PEERS, int TPR>
-__device__ __forceinline__ void row_block_body(int r0, int r1, int lane, int nnz4, const int *__restrict__ rowptr,
+template <typename T, bool PEERS, int TPR>
+__device__ __forceinline__ void row_block_body(int r0, int r1, int lane, const int *__restrict__ rowptr,
                                                const int *__restrict__ col, const T *__restrict__ val,
                                                const T *__restrict__ x, T *__restrict__ y, const PeerList<T> &peers,
                                                uint64_t pl, uint64_t pf)
@@ -207,15 +204,15 @@ __device__ __forceinline__ void row_block_body(int r0, int r1, int lane, int nnz
         const bool valid = row < r1;
         const int start = valid ? rowptr[row] : 0;
         const int end = valid ? rowptr[row + 1] : 0;
-        T sum = row_partial<T, VEC>(start, end, sl, TPR, nnz4, col, val, x, pl, pf);
+        T sum = row_partial<T>(start, end, sl, TPR, col, val, x, pl, pf);
         sum = group_sum_c<T, TPR>(sum);
         if (valid && sl == 0) store_y<PEERS>(y, peers, row, sum);
     }
 }
 
-template <typename T, int VEC, bool PEERS>
+template <typename T, bool PEERS>
 __global__ void __launch_bounds__(kThreads)
-row_block_kernel(int parts, int nnz, const int *__restrict__ splitter, const int *__restrict__ rowptr,
+row_block_kernel(int parts, const int *__restrict__ splitter, const int *__restrict__ rowptr,
                  const int *__restrict__ col, const T *__restrict__ val, const T *__restrict__ x,
                  T *__restrict__ y, const PeerList<T> peers)
 {
@@ -229,11 +226,10 @@ row_block_kernel(int parts, int nnz, const int *__restrict__ splitter, const int
     if (nrows <= 0) return;
     const int nz = rowptr[r1] - rowptr[r0];
     const int avg = (nz + nrows - 1) / nrows;
-    const int nnz4 = nnz & ~3;
     // lanes per row from the block's own mean row length (warp-uniform): compile-time bodies so that the row
     // walk unrolls and the butterfly has a fixed depth
-#define SB_BODY(N) row_block_body<T, VEC, PEERS, N>(r0, r1, lane, nnz4, rowptr, col, val, x, y, peers, pl, pf)
-    constexpr int per_lane = VEC == 4 ? 7 : 4;  // batches of 8 per lane (mode 4) / one 4-element chunk per lane
+#define SB_BODY(N) row_block_body<T, PEERS, N>(r0, r1, lane, rowptr, col, val, x, y, peers, pl, pf)
+    constexpr int per_lane = 7;  // entries per lane, as pick_tpr chooses lanes for Method_Parallel
     if (avg <= per_lane) SB_BODY(1);
     else if (avg <= 2 * per_lane) SB_BODY(2);
     else if (avg <= 4 * per_lane) SB_BODY(4);
@@ -269,13 +265,6 @@ __global__ void empty_rows_kernel(int m, const int *__restrict__ rowptr, int *__
 {
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
     if (r < m && rowptr[r] == rowptr[r + 1]) *flag = 1;
-}
-
-template <typename T>
-__global__ void fill_zero_kernel(long long n, T *__restrict__ y)
-{
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) y[i] = 0;
 }
 
 // ------------------------------------------------------------------------------------------------

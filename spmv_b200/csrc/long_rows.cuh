@@ -24,19 +24,6 @@ __global__ void long_cover_threshold_kernel(int m, int row0, int thr, const int 
     if (r >= row0) covered[r] = len > thr ? 0 : len;
 }
 
-// non-zeros that sit in rows of at most thr entries (integer counter, builder only)
-__global__ void short_nnz_kernel(int m, int thr, const int *__restrict__ rowptr, unsigned long long *__restrict__ out)
-{
-    const int r = blockIdx.x * blockDim.x + threadIdx.x;
-    unsigned long long v = 0;
-    if (r < m) {
-        const int len = rowptr[r + 1] - rowptr[r];
-        if (len <= thr) v = (unsigned long long)len;
-    }
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(kFull, v, o);
-    if ((threadIdx.x & 31) == 0 && v) atomicAdd(out, v);
-}
-
 __global__ void long_count_kernel(int m, const int *__restrict__ rowptr, const int *__restrict__ covered,
                                   int *__restrict__ cnt_rows, int *__restrict__ cnt_segs)
 {

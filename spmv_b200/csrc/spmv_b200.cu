@@ -95,6 +95,13 @@ static bool is_device_ptr(const void *p)
 
 static inline int blocks_for(long long threads) { return (int)((threads + kThreads - 1) / kThreads); }
 
+// f(T()) with the handle's value type: T = double for fp64, float for fp32
+template <typename F>
+static auto with_precision(const DeviceState *st, F f)
+{
+    return st->vsize == 8 ? f(double()) : f(float());
+}
+
 struct DeviceGuard {  // library code is device-agnostic: run on the handle's device, then restore
     int prev = -1, want;
     explicit DeviceGuard(int dev) : want(dev)
@@ -105,18 +112,36 @@ struct DeviceGuard {  // library code is device-agnostic: run on the handle's de
     ~DeviceGuard() { if (prev >= 0 && prev != want) cudaSetDevice(prev); }
 };
 
-// Zero a one-element device counter, enqueue `launch(counter)` on s, and read the counter back after a stream sync.
+// Copy `count` values from the device to the host on the handle's stream and wait for them: every scalar a builder
+// reads back, so that create is ordered on st->stream alone.
+template <typename V>
+static bool read_back(const DeviceState *st, V *host, const V *device, size_t count = 1)
+{
+    SB_TRY(cudaMemcpyAsync(host, device, count * sizeof(V), cudaMemcpyDeviceToHost, st->stream));
+    SB_TRY(cudaStreamSynchronize(st->stream));
+    return true;
+}
+
+// Zero a one-element device counter, enqueue `launch(counter)` on the handle's stream, and read the counter back.
 template <typename C, typename Launch>
-static bool read_counter(cudaStream_t s, C *value, Launch launch)
+static bool read_counter(const DeviceState *st, C *value, Launch launch)
 {
     DeviceArray<C> counter;
     if (!counter.alloc(1)) return false;
-    SB_TRY(cudaMemsetAsync(counter, 0, sizeof(C), s));
+    SB_TRY(cudaMemsetAsync(counter, 0, sizeof(C), st->stream));
     launch(counter.get());
     SB_TRY(cudaGetLastError());
-    SB_TRY(cudaMemcpyAsync(value, counter, sizeof(C), cudaMemcpyDeviceToHost, s));
-    SB_TRY(cudaStreamSynchronize(s));
-    return true;
+    return read_back(st, value, counter.get());
+}
+
+// An optional step failed: forget its CUDA and library errors and reset what it built.  Whether that counts as a
+// layout fallback (spmv_b200_info "layout_fallbacks") is the caller's to say.
+template <typename... Built>
+static void abandon(Built &...built)
+{
+    cudaGetLastError();
+    spmv_b200_clear_error();
+    ((built = {}), ...);
 }
 
 template <typename V>
@@ -161,8 +186,7 @@ static void note_host_buffer(DeviceState *st, int which, const void *p, size_t b
 // Option "refresh": a source map that cannot be made costs the handle its refresh, never its layout.
 static void map_failure(DeviceState *st)
 {
-    cudaGetLastError();
-    spmv_b200_clear_error();
+    abandon();
     st->map_failed = true;
 }
 
@@ -246,7 +270,7 @@ static bool build_band_major(DeviceState *st)
         // whether banding can pay (below) and which SELL kernel flavour runs (build_sell).
         const int halfwidth = (int)(0.125 * usable / st->vsize);
         unsigned long long h_far = 0;
-        const bool probed = read_counter(st->stream, &h_far, [&](unsigned long long *far) {
+        const bool probed = read_counter(st, &h_far, [&](unsigned long long *far) {
             band_locality_kernel<<<blocks_for(st->m), kThreads, 0, st->stream>>>(
                 st->m, (double)st->n / st->m, halfwidth, st->rowptr, st->col, far);
         });
@@ -284,9 +308,7 @@ static bool build_band_major(DeviceState *st)
     // The band-major copy is a speed-up only: when it cannot be allocated (or built) the handle keeps running the
     // plain CSR view it already holds -- never fail a handle over an optional layout.
     auto give_up = [&]() {
-        cudaGetLastError();
-        st->v = {};
-        spmv_b200_clear_error();
+        abandon(st->v);
         st->layout_fallbacks++;
         return true;
     };
@@ -320,7 +342,7 @@ static bool build_splitter(DeviceState *st, int m, const int *rowptr, int parts,
     if (!out.alloc((size_t)parts + 1)) return false;
     splitter_kernel<<<blocks_for(parts + 1), kThreads, 0, st->stream>>>(parts, st->nnz, m, rowptr, out);
     SB_TRY(cudaGetLastError());
-    return read_counter(st->stream, starved, [&](int *flag) {
+    return read_counter(st, starved, [&](int *flag) {
         splitter_starved_kernel<<<blocks_for(parts), kThreads, 0, st->stream>>>(parts, m, out, flag);
     });
 }
@@ -363,8 +385,7 @@ static bool build_long_rows(DeviceState *st, DeviceArray<int> covered, bool accu
              exclusive_scan(cnt_s.get(), scan_s.get(), m + 1, st->stream);
     }
     int totals[2] = {0, 0};
-    if (ok) ok = SB_CUDA(cudaMemcpy(&totals[0], scan_r + m, sizeof(int), cudaMemcpyDeviceToHost)) &&
-                 SB_CUDA(cudaMemcpy(&totals[1], scan_s + m, sizeof(int), cudaMemcpyDeviceToHost));
+    if (ok) ok = read_back(st, &totals[0], scan_r + m) && read_back(st, &totals[1], scan_s + m);
     st->lr.rows = totals[0];
     st->lr.segs = totals[1];
     st->lr.accumulate = accumulate;
@@ -423,9 +444,7 @@ static bool build_long_rows_threshold(DeviceState *st)
         int h_ptr[5] = {0, 0, 0, 0, 0};
         if (ok) {
             sorted_key_ptr_kernel<<<1, kThreads, 0, st->stream>>>(m, 4, key_out, d_ptr);  // first sorted row of every bin
-            ok = SB_CUDA(cudaGetLastError()) &&
-                 SB_CUDA(cudaMemcpyAsync(h_ptr, d_ptr, sizeof(h_ptr), cudaMemcpyDeviceToHost, st->stream)) &&
-                 SB_CUDA(cudaStreamSynchronize(st->stream));
+            ok = SB_CUDA(cudaGetLastError()) && read_back(st, h_ptr, d_ptr.get(), 5);
         }
         if (!ok) return false;
         for (int b = 0; b < 4; ++b) st->lr.bin_ptr[b] = h_ptr[b];  // bin b = list[bin_ptr[b], bin_ptr[b+1]); bin 3 is unused
@@ -445,9 +464,7 @@ static bool build_pipeline(DeviceState *st)
     if (!d.alloc(kPipeChunks)) return false;
     SB_TRY(cudaMemsetAsync(d, 0, kPipeChunks * sizeof(int), st->stream));
     chunk_xmax_kernel<<<blocks_for(st->m), kThreads, 0, st->stream>>>(st->m, kPipeChunks, st->rowptr, st->col, d);
-    const bool ok = SB_CUDA(cudaGetLastError()) &&
-                    SB_CUDA(cudaMemcpyAsync(st->chunk_xmax, d, kPipeChunks * sizeof(int), cudaMemcpyDeviceToHost, st->stream)) &&
-                    SB_CUDA(cudaStreamSynchronize(st->stream));
+    const bool ok = SB_CUDA(cudaGetLastError()) && read_back(st, st->chunk_xmax, d.get(), kPipeChunks);
     st->pipeline = ok;
     return ok;
 }
@@ -521,7 +538,7 @@ static bool build_sell(DeviceState *st)
     SB_TRY(cudaGetLastError());
     if (cap && !build_long_rows(st, std::move(covered), /*accumulate=*/true)) return false;
     if (!exclusive_scan(count.get(), st->sell.slice_ptr.get(), st->sell.slices + 1, st->stream)) return false;
-    SB_TRY(cudaMemcpy(&st->sell.padded, st->sell.slice_ptr + st->sell.slices, sizeof(long long), cudaMemcpyDeviceToHost));
+    if (!read_back(st, &st->sell.padded, st->sell.slice_ptr + st->sell.slices)) return false;
     if (!st->sell.col.alloc((size_t)st->sell.padded) || !st->sell.val.alloc((size_t)st->sell.padded, sizeof(T))) return false;
     sell_fill_kernel<T><<<blocks_for((long long)st->sell.slices * 32), kThreads, 0, st->stream>>>(
         st->sell.slices, st->a_rowptr, st->a_col, (const T *)st->a_val, st->sell.perm, st->sell.slice_ptr, st->sell.col,
@@ -568,8 +585,8 @@ static bool build_csr5(DeviceState *st)
     SB_TRY(cudaGetLastError());
     if (!exclusive_scan(off_cnt.get(), st->c5.off_ptr.get(), p + 1, st->stream)) return false;
     uint32_t tail_word = 0;
-    SB_TRY(cudaMemcpy(&st->c5.num_offsets, st->c5.off_ptr + p, sizeof(int), cudaMemcpyDeviceToHost));
-    SB_TRY(cudaMemcpy(&tail_word, st->c5.tile_ptr + (p - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    if (!read_back(st, &st->c5.num_offsets, st->c5.off_ptr + p) || !read_back(st, &tail_word, st->c5.tile_ptr + (p - 1)))
+        return false;
     st->c5.tail_start = (int)(tail_word & 0x7FFFFFFFu);  // anonymouslib_avx2.h:177
     if (st->c5.num_offsets > 0) {
         if (!st->c5.off.alloc((size_t)st->c5.num_offsets)) return false;
@@ -619,9 +636,7 @@ static bool build_band_seg_t(DeviceState *st)
         }
         if (ok) {
             sorted_key_ptr_kernel<<<1, kThreads, 0, st->stream>>>(nnz, K, key_out, d_tab);
-            ok = SB_CUDA(cudaGetLastError()) &&
-                 SB_CUDA(cudaMemcpyAsync(h_ptr, d_tab, ((size_t)K + 1) * sizeof(int), cudaMemcpyDeviceToHost, st->stream)) &&
-                 SB_CUDA(cudaStreamSynchronize(st->stream));
+            ok = SB_CUDA(cudaGetLastError()) && read_back(st, h_ptr, d_tab.get(), (size_t)K + 1);
         }
         if (!ok) return false;
         // band b occupies slots [seg.ptr[b], seg.ptr[b] + seg.cnt[b]); starts aligned to 4 entries (16 bytes of ColIdx)
@@ -673,10 +688,8 @@ static bool build_band_seg_t(DeviceState *st)
                 bseg_transpose_kernel<<<blocks_for((long long)gk), kThreads, 0, st->stream>>>(K, st->seg.groups, blk_scan, st->seg.gbase);
                 ok = SB_CUDA(cudaGetLastError());
             }
-            ok = ok &&
-                 SB_CUDA(cudaMemcpy(&h_segs[0], st->seg.tile_seg0 + (size_t)tiles * kSegChunks, sizeof(int), cudaMemcpyDeviceToHost)) &&
-                 SB_CUDA(cudaMemcpy(&h_segs[1], blk_scan + gk, sizeof(int), cudaMemcpyDeviceToHost)) &&
-                 SB_CUDA(cudaMemcpy(&h_cross, d_cross, sizeof(int), cudaMemcpyDeviceToHost));
+            ok = ok && read_back(st, &h_segs[0], st->seg.tile_seg0 + (size_t)tiles * kSegChunks) &&
+                 read_back(st, &h_segs[1], blk_scan + gk) && read_back(st, &h_cross, d_cross.get());
         }
         if (!ok) return false;
     }
@@ -696,25 +709,26 @@ static bool build_band_seg(DeviceState *st)
     return st->seg.bands <= 32 ? build_band_seg_t<T, uint32_t>(st) : build_band_seg_t<T, unsigned long long>(st);
 }
 
+// Mirror of the reference's demotion / promotion rule with the CALLER's nthreads (a10, parallel_balanced2_spmv.c:72-94)
+// for clients that read handle->spmvMethod: Method_Balanced2 when some partition of the reference's csrSplitter owns
+// no whole row, else Method_Balanced.
+static bool apply_reference_balance_rule(DeviceState *st, spmv_Handle *h)
+{
+    st->split.ref_T = (int)(h->nthreads ? (h->nthreads > (1u << 24) ? (1u << 24) : h->nthreads) : 1);
+    int ref_starved = 0;
+    if (!build_splitter(st, st->m, st->rowptr, st->split.ref_T, st->split.ref_splitter, &ref_starved)) return false;
+    h->spmvMethod = ref_starved ? Method_Balanced2 : Method_Balanced;
+    return true;
+}
+
 template <typename T>
 static bool build_method(DeviceState *st, spmv_Handle *h, int method)
 {
     if (st->seg.bands > 1 && method != Method_Serial) {
-        if (build_band_seg<T>(st)) {
-            if (method == Method_Balanced || method == Method_Balanced2) {
-                // keep what a client reads from the handle: the reference's Balanced <-> Balanced2 rule (a10)
-                st->split.ref_T = (int)(h->nthreads ? (h->nthreads > (1u << 24) ? (1u << 24) : h->nthreads) : 1);
-                int ref_starved = 0;
-                if (!build_splitter(st, st->m, st->rowptr, st->split.ref_T, st->split.ref_splitter, &ref_starved)) return false;
-                h->spmvMethod = ref_starved ? Method_Balanced2 : Method_Balanced;
-            }
-            return true;
-        }
+        if (build_band_seg<T>(st))
+            return (method != Method_Balanced && method != Method_Balanced2) || apply_reference_balance_rule(st, h);
         // an optional layout: fall back to the method's own kernel on the plain CSR view
-        cudaGetLastError();
-        st->seg = {};
-        st->tile = {};
-        spmv_b200_clear_error();
+        abandon(st->seg, st->tile);
         st->x_bands = 1;
         st->kernel = SPMV_B200_KERNEL_NONE;
         st->layout_fallbacks++;
@@ -727,21 +741,14 @@ static bool build_method(DeviceState *st, spmv_Handle *h, int method)
         st->tpr = pick_tpr(st->nnz, st->a_m);
         st->kernel = SPMV_B200_KERNEL_CSR_VECTOR;
         if (!build_long_rows_threshold(st)) {  // bins / long-row list are speed-ups: plain CSR-vector still works
-            cudaGetLastError();
-            st->lr = {};
-            spmv_b200_clear_error();
+            abandon(st->lr);
             st->layout_fallbacks++;
         }
-        if (!build_pipeline(st)) { cudaGetLastError(); st->pipeline = false; spmv_b200_clear_error(); }
+        if (!build_pipeline(st)) abandon(st->pipeline);
         return true;
     case Method_Balanced:
     case Method_Balanced2: {
-        // mirror of the reference's demotion / promotion rule with the CALLER's nthreads (a10,
-        // parallel_balanced2_spmv.c:72-94) for clients that read handle->spmvMethod
-        st->split.ref_T = (int)(h->nthreads ? (h->nthreads > (1u << 24) ? (1u << 24) : h->nthreads) : 1);
-        int ref_starved = 0;
-        if (!build_splitter(st, st->m, st->rowptr, st->split.ref_T, st->split.ref_splitter, &ref_starved)) return false;
-        h->spmvMethod = ref_starved ? Method_Balanced2 : Method_Balanced;
+        if (!apply_reference_balance_rule(st, h)) return false;
         // the GPU geometry: row blocks of ~block_nnz non-zeros, one warp each
         long long block_nnz = opt("block_nnz");
         if (block_nnz < 32) block_nnz = 32;
@@ -779,19 +786,32 @@ static bool build_method(DeviceState *st, spmv_Handle *h, int method)
 //   * fewer than 8192 rows: Method_Parallel (nothing to amortise a layout build).
 // The statistics are the ones create gathers on the device anyway (far_fraction of the locality probe) plus one pass
 // over RowPtr.  Method_Serial is never overridden: it promises the reference's bits.
+// spmv_b200_recommend_method applies the same rule on the host, where the locality share is unknown (far_fraction
+// < 0) and short rows alone never pick Method_Parallel.  heavy(cut, &count) counts the non-zeros in rows longer than
+// cut; it is called only from 8192 rows on, and a count that fails picks Method_Parallel.
+template <typename CountHeavy>
+static int pick_method(long long m, long long nnz, double far_fraction, CountHeavy heavy)
+{
+    if (m < 8192 || nnz <= 0) return Method_Parallel;
+    const double mean = (double)nnz / m;
+    long long count = 0;
+    if (!heavy((int)(4.0 * mean) + 16, &count)) return Method_Parallel;
+    if (4 * count > nnz) return Method_CSR5SPMV;
+    if (far_fraction >= 0.0 && mean <= 8.0 && far_fraction <= 0.25) return Method_Parallel;
+    return Method_SellCSigma;
+}
+
 static int auto_pick_method(DeviceState *st)
 {
-    if (st->m < 8192 || st->nnz <= 0) return Method_Parallel;
-    const double mean = (double)st->nnz / st->m;
-    const int cut = (int)(4.0 * mean) + 16;
-    unsigned long long h_heavy = 0;
-    const bool ok = read_counter(st->stream, &h_heavy, [&](unsigned long long *heavy) {
-        heavy_rows_kernel<<<blocks_for(st->m), kThreads, 0, st->stream>>>(st->m, cut, st->rowptr, heavy);
+    return pick_method(st->m, st->nnz, st->far_fraction, [&](int cut, long long *count) {
+        unsigned long long h_heavy = 0;
+        const bool ok = read_counter(st, &h_heavy, [&](unsigned long long *heavy) {
+            heavy_rows_kernel<<<blocks_for(st->m), kThreads, 0, st->stream>>>(st->m, cut, st->rowptr, heavy);
+        });
+        if (!ok) abandon();
+        *count = (long long)h_heavy;
+        return ok;
     });
-    if (!ok) { cudaGetLastError(); spmv_b200_clear_error(); return Method_Parallel; }
-    if (4.0 * (double)h_heavy > (double)st->nnz) return Method_CSR5SPMV;
-    if (mean <= 8.0 && st->far_fraction <= 0.25) return Method_Parallel;
-    return Method_SellCSigma;
 }
 
 // reorder_map: the source map of the permuted values under options "reorder" and "refresh" (host, nnz ints)
@@ -816,10 +836,7 @@ static bool build_state(DeviceState *st, spmv_Handle *h, int m, int n, int *RowP
     const bool dev_csr = is_device_ptr(RowPtr);
     int ends[2] = {0, 0};
     if (dev_csr) {
-        if (m > 0) {
-            SB_TRY(cudaMemcpy(&ends[0], RowPtr, sizeof(int), cudaMemcpyDeviceToHost));
-            SB_TRY(cudaMemcpy(&ends[1], RowPtr + m, sizeof(int), cudaMemcpyDeviceToHost));
-        }
+        if (m > 0 && !(read_back(st, &ends[0], RowPtr) && read_back(st, &ends[1], RowPtr + m))) return false;
     } else if (m > 0) {
         ends[0] = RowPtr[0];
         ends[1] = RowPtr[m];
@@ -856,12 +873,11 @@ static bool build_state(DeviceState *st, spmv_Handle *h, int m, int n, int *RowP
 
     st->a_m = st->m; st->a_rowptr = st->rowptr; st->a_col = st->col; st->a_val = st->val;
     if (method != Method_Serial) {  // Method_Serial keeps the reference's exact summation order: never banded
-        const bool okb = st->vsize == 8 ? build_band_major<double>(st) : build_band_major<float>(st);
-        if (!okb) return false;
+        if (!with_precision(st, [&](auto t) { return build_band_major<decltype(t)>(st); })) return false;
     }
     if (m > 0) {
         int e = 0;
-        const bool ok = read_counter(st->stream, &e, [&](int *flag) {
+        const bool ok = read_counter(st, &e, [&](int *flag) {
             empty_rows_kernel<<<blocks_for(st->a_m), kThreads, 0, st->stream>>>(st->a_m, st->a_rowptr, flag);
         });
         if (!ok) return false;
@@ -877,8 +893,7 @@ static bool build_state(DeviceState *st, spmv_Handle *h, int m, int n, int *RowP
         if (st->auto_method == Method_SellCSigma || st->auto_method == Method_CSR5SPMV || st->auto_method == Method_Parallel)
             h->spmvMethod = (SPMV_METHODS)st->auto_method;  // what actually runs, for clients that read the field
     }
-    const bool ok = st->vsize == 8 ? build_method<double>(st, h, method) : build_method<float>(st, h, method);
-    if (!ok) return false;
+    if (!with_precision(st, [&](auto t) { return build_method<decltype(t)>(st, h, method); })) return false;
     SB_TRY(cudaStreamSynchronize(st->stream));
     // Our own upload of the CSR is dead weight once every kernel of the handle reads a re-laid-out copy (the
     // band-major copy or the COO bands): give those gigabytes back (an adopted device CSR is the caller's).
@@ -902,16 +917,29 @@ static bool build_state(DeviceState *st, spmv_Handle *h, int m, int n, int *RowP
 // ------------------------------------------------------------------------------------------------
 // launch dispatch (a3: the reference's spmv_functions[] table, common.c:85-94)
 // ------------------------------------------------------------------------------------------------
-template <typename T, int VEC>
-static void launch_vector(DeviceState *st, int tpr, int row0, int row1, const T *x, T *y, const PeerList<T> &peers, int fuse_bands)
+// the extra y destinations of spmv_b200_set_y_peers (fused all-gather); PeerList<T>{} is "none"
+template <typename T>
+static PeerList<T> peers_of(const DeviceState *st)
 {
+    PeerList<T> peers;
+    peers.n = st->n_peers;
+    for (int i = 0; i < kMaxPeers; ++i) peers.p[i] = (T *)st->peers[i];
+    return peers;
+}
+
+// CSR-vector over rows [row0, row1) of the active view; fuse_bands > 0: they belong to the last band and y is the
+// FINAL y
+template <typename T>
+static void launch_vector(DeviceState *st, int row0, int row1, const T *x, T *y, const PeerList<T> &peers, int fuse_bands = 0)
+{
+    const int tpr = st->tpr;
     const int grid = blocks_for((long long)(row1 - row0) * tpr);
     if (grid <= 0) return;
-#define SB_ARGS row0, row1, st->nnz, st->lr.thr, st->a_rowptr, st->a_col, (const T *)st->a_val, x, y, peers, fuse_bands, st->m, st->v.y.as<T>()
+#define SB_ARGS row0, row1, st->lr.thr, st->a_rowptr, st->a_col, (const T *)st->a_val, x, y, peers, fuse_bands, st->m, st->v.y.as<T>()
 #define SB_CASE(N) case N: \
-        if (fuse_bands > 0) csr_vector_kernel<T, N, VEC, false, true><<<grid, kThreads, 0, st->stream>>>(SB_ARGS); \
-        else if (peers.n > 0) csr_vector_kernel<T, N, VEC, true, false><<<grid, kThreads, 0, st->stream>>>(SB_ARGS); \
-        else csr_vector_kernel<T, N, VEC, false, false><<<grid, kThreads, 0, st->stream>>>(SB_ARGS); \
+        if (fuse_bands > 0) csr_vector_kernel<T, N, false, true><<<grid, kThreads, 0, st->stream>>>(SB_ARGS); \
+        else if (peers.n > 0) csr_vector_kernel<T, N, true, false><<<grid, kThreads, 0, st->stream>>>(SB_ARGS); \
+        else csr_vector_kernel<T, N, false, false><<<grid, kThreads, 0, st->stream>>>(SB_ARGS); \
         break;
     switch (tpr) { SB_CASE(1) SB_CASE(2) SB_CASE(4) SB_CASE(8) SB_CASE(16) default: SB_CASE(32) }
 #undef SB_CASE
@@ -919,11 +947,15 @@ static void launch_vector(DeviceState *st, int tpr, int row0, int row1, const T 
     count_launch();
 }
 
-// rows [row0, row1) of the active view; fuse_bands > 0: they belong to the last band and y is the FINAL y
+// y_out = the band partials of the virtual y (v.y) added in band order, copied to the peers too
 template <typename T>
-static void launch_vector_mode(DeviceState *st, int row0, int row1, const T *x, T *y, const PeerList<T> &peers, int fuse_bands = 0)
+static bool launch_band_fold(DeviceState *st, T *y_out)
 {
-    launch_vector<T, 4>(st, st->tpr, row0, row1, x, y, peers, fuse_bands);
+    const PeerList<T> peers = peers_of<T>(st);
+    if (peers.n > 0) band_reduce_kernel<T, true><<<blocks_for(st->m), kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), y_out, peers);
+    else band_reduce_kernel<T, false><<<blocks_for(st->m), kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), y_out, peers);
+    count_launch();
+    return SB_CUDA(cudaGetLastError());
 }
 
 // CSR-vector over rows [row0, m) only (the CSR tail of SELL)
@@ -991,9 +1023,7 @@ static bool launch_seg_finish(DeviceState *st, T *y_out)
 {
     cudaStream_t s = st->stream;
     if (st->seg.cross) launch_carry_fixup<T>(st, s, st->tile.count * kSegChunks, st->tile.carry_row, st->tile.carry_val.as<T>(), st->seg.sums.as<T>());
-    PeerList<T> pr;
-    pr.n = st->n_peers;
-    for (int i = 0; i < kMaxPeers; ++i) pr.p[i] = (T *)st->peers[i];
+    const PeerList<T> pr = peers_of<T>(st);
 #define SB_MERGE(M, P) bseg_merge_kernel<T, M, P><<<blocks_for((long long)st->seg.groups * 32), kThreads, 0, s>>>(0, st->m, st->seg.bands, st->seg.mask.as<M>(), \
                                                                                      st->seg.gbase, st->seg.sums.as<T>(), y_out, pr)
     if (st->seg.mask64) { if (pr.n > 0) SB_MERGE(unsigned long long, true); else SB_MERGE(unsigned long long, false); }
@@ -1022,10 +1052,7 @@ static bool launch(DeviceState *st, const T *x, T *y_out)
     T *y = banded ? st->v.y.as<T>() : y_out;
     const T *val = (const T *)st->a_val;
     // extra y destinations (fused all-gather): written by whichever kernel produces the FINAL y
-    PeerList<T> peers, none;
-    none.n = 0;
-    peers.n = st->n_peers;
-    for (int i = 0; i < kMaxPeers; ++i) { peers.p[i] = (T *)st->peers[i]; none.p[i] = nullptr; }
+    const PeerList<T> peers = peers_of<T>(st), none{};
     const PeerList<T> &direct = banded ? none : peers;  // kernels write virtual y when banded
     bool scattered = peers.n == 0;
     switch (st->kernel) {
@@ -1046,21 +1073,21 @@ static bool launch(DeviceState *st, const T *x, T *y_out)
                 if (count <= 0) continue;
                 const int grid = blocks_for((long long)count * lanes[b]);
                 const int *list = st->lr.bin_list + st->lr.bin_ptr[b];
-#define SB_BIN(N) if (direct.n > 0) csr_vector_list_kernel<T, N, true><<<grid, kThreads, 0, s>>>(count, st->nnz, list, st->a_rowptr, st->a_col, val, x, y, direct); \
-                  else csr_vector_list_kernel<T, N, false><<<grid, kThreads, 0, s>>>(count, st->nnz, list, st->a_rowptr, st->a_col, val, x, y, direct)
+#define SB_BIN(N) if (direct.n > 0) csr_vector_list_kernel<T, N, true><<<grid, kThreads, 0, s>>>(count, list, st->a_rowptr, st->a_col, val, x, y, direct); \
+                  else csr_vector_list_kernel<T, N, false><<<grid, kThreads, 0, s>>>(count, list, st->a_rowptr, st->a_col, val, x, y, direct)
                 if (b == 0) { SB_BIN(1); } else if (b == 1) { SB_BIN(4); } else { SB_BIN(16); }
 #undef SB_BIN
                 count_launch();
             }
         } else {
-            launch_vector_mode<T>(st, 0, m, x, y, direct);
+            launch_vector<T>(st, 0, m, x, y, direct);
         }
         scattered = scattered || !banded;
         break;
     case SPMV_B200_KERNEL_ROW_BLOCKS: {
         const int grid = blocks_for((long long)st->split.parts * 32);
-#define SB_RB(V, P) row_block_kernel<T, V, P><<<grid, kThreads, 0, s>>>(st->split.parts, st->nnz, st->split.splitter, st->a_rowptr, st->a_col, val, x, y, direct)
-        if (direct.n > 0) SB_RB(4, true); else SB_RB(4, false);
+#define SB_RB(P) row_block_kernel<T, P><<<grid, kThreads, 0, s>>>(st->split.parts, st->split.splitter, st->a_rowptr, st->a_col, val, x, y, direct)
+        if (direct.n > 0) SB_RB(true); else SB_RB(false);
 #undef SB_RB
         scattered = scattered || !banded;
         count_launch();
@@ -1137,12 +1164,7 @@ static bool launch(DeviceState *st, const T *x, T *y_out)
         else long_final_kernel<T, false><<<fgrid, kThreads, 0, s>>>(st->lr.rows, st->lr.accumulate, single, st->lr.row, st->lr.seg_ptr, st->lr.partial.as<T>(), y, direct);
         count_launch(2);
     }
-    if (banded) {
-        if (peers.n > 0) band_reduce_kernel<T, true><<<blocks_for(st->m), kThreads, 0, s>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), y_out, peers);
-        else band_reduce_kernel<T, false><<<blocks_for(st->m), kThreads, 0, s>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), y_out, peers);
-        scattered = true;
-        count_launch();
-    }
+    if (banded) return launch_band_fold<T>(st, y_out);  // writes the peers too
     if (!scattered) {  // kernel family without a fused epilogue: one stream-ordered copy to the peers
         peer_copy_kernel<T><<<blocks_for(st->m), kThreads, 0, s>>>(st->m, y_out, peers);
         count_launch();
@@ -1171,9 +1193,7 @@ static bool run_pipelined(DeviceState *st, const T *hx, T *hy)
     const int m = st->m, n = st->n;
     const bool banded = st->x_bands > 1;
     const int pieces = banded ? st->x_bands : kPipeChunks;
-    PeerList<T> none;
-    none.n = 0;
-    for (int i = 0; i < kMaxPeers; ++i) none.p[i] = nullptr;
+    const PeerList<T> none{};
     // whatever the caller queued on the compute stream before this call stays ahead of the copies
     SB_TRY(cudaEventRecord(st->ev_start, s));
     SB_TRY(cudaStreamWaitEvent(st->s_in, st->ev_start, 0));
@@ -1203,12 +1223,12 @@ static bool run_pipelined(DeviceState *st, const T *hx, T *hy)
         const int K = st->x_bands;
         for (int b = 0; b + 1 < K; ++b) {
             if (!need_piece(b)) return false;
-            launch_vector_mode<T>(st, b * m, (b + 1) * m, xd, st->v.y.as<T>(), none);
+            launch_vector<T>(st, b * m, (b + 1) * m, xd, st->v.y.as<T>(), none);
         }
         if (!need_piece(K - 1)) return false;
         for (int c = 0; c < kPipeChunks; ++c) {
             const int r0 = (int)((long long)m * c / kPipeChunks), r1 = (int)((long long)m * (c + 1) / kPipeChunks);
-            launch_vector_mode<T>(st, (K - 1) * m + r0, (K - 1) * m + r1, xd, yd, none, K - 1);
+            launch_vector<T>(st, (K - 1) * m + r0, (K - 1) * m + r1, xd, yd, none, K - 1);
             if (!chunk_out(c, r0, r1)) return false;
         }
     } else {
@@ -1217,7 +1237,7 @@ static bool run_pipelined(DeviceState *st, const T *hx, T *hy)
             int p = 0;
             while (p < pieces - 1 && piece_hi(p) < st->chunk_xmax[c]) ++p;
             if (!need_piece(p)) return false;
-            launch_vector_mode<T>(st, r0, r1, xd, yd, none);
+            launch_vector<T>(st, r0, r1, xd, yd, none);
             if (!chunk_out(c, r0, r1)) return false;
         }
     }
@@ -1355,8 +1375,10 @@ void spmv(const spmv_Handle_t handle, BASIC_INT_TYPE m, const BASIC_INT_TYPE *Ro
     if (!x_dev && !st->stage.x.get() && !st->stage.x.alloc(st->n, st->vsize)) return;
     if (!y_dev && !st->stage.y.get() && !st->stage.y.alloc(st->m, st->vsize)) return;
     if (!x_dev && !y_dev && st->pipeline && st->n_peers == 0 && st->kernel == SPMV_B200_KERNEL_CSR_VECTOR && xb && yb) {
-        if (st->vsize == 8) run_pipelined<double>(st, (const double *)Vector_Val_X, (double *)Vector_Val_Y);
-        else run_pipelined<float>(st, (const float *)Vector_Val_X, (float *)Vector_Val_Y);
+        with_precision(st, [&](auto t) {
+            using T = decltype(t);
+            return run_pipelined<T>(st, (const T *)Vector_Val_X, (T *)Vector_Val_Y);
+        });
         return;
     }
     if (!x_dev) {
@@ -1370,9 +1392,7 @@ void spmv(const spmv_Handle_t handle, BASIC_INT_TYPE m, const BASIC_INT_TYPE *Ro
         }
     }
     if (!y_dev) yd = st->stage.y.get();
-    const bool ok = st->vsize == 8 ? launch<double>(st, (const double *)xd, (double *)yd)
-                                   : launch<float>(st, (const float *)xd, (float *)yd);
-    if (!ok) return;
+    if (!with_precision(st, [&](auto t) { using T = decltype(t); return launch<T>(st, (const T *)xd, (T *)yd); })) return;
     if (!y_dev) {
         if (yb && !SB_CUDA(cudaMemcpyAsync(Vector_Val_Y, yd, yb, cudaMemcpyDeviceToHost, st->stream))) return;
         SB_CUDA(cudaStreamSynchronize(st->stream));  // host y is complete on return, as in the reference
@@ -1474,8 +1494,10 @@ int spmv_b200_set_values(spmv_Handle_t handle, const void *Matrix_Val)
         if (!SB_CUDA(cudaEventRecord(st->ev_x, st->stream))) return -1;
     }
     if (tab.n > 0) {  // (not on the spmv() path: not in spmv_b200_launch_count)
-        if (st->vsize == 8) value_refresh_kernel<double><<<blocks_for(quads), kThreads, 0, st->stream>>>(tab, (const double *)from);
-        else value_refresh_kernel<float><<<blocks_for(quads), kThreads, 0, st->stream>>>(tab, (const float *)from);
+        with_precision(st, [&](auto t) {
+            using T = decltype(t);
+            value_refresh_kernel<T><<<blocks_for(quads), kThreads, 0, st->stream>>>(tab, (const T *)from);
+        });
         if (!SB_CUDA(cudaGetLastError())) return -1;
     }
     if (!on_device && !SB_CUDA(cudaEventSynchronize(st->ev_x))) return -1;
@@ -1554,43 +1576,15 @@ int spmv_b200_spmv_bands(spmv_Handle_t handle, int band_first, int band_count, c
     if (!is_device_ptr(x_device)) { set_error("spmv_b200_spmv_bands: x must be a device pointer"); return -1; }
     std::lock_guard<std::mutex> lock(st->mu);
     DeviceGuard guard(st->device);
-    bool ok;
-    if (st->kernel == SPMV_B200_KERNEL_BAND_SEG) {
-        ok = st->vsize == 8 ? launch_seg_bands<double>(st, band_first, band_count, (const double *)x_device)
-                            : launch_seg_bands<float>(st, band_first, band_count, (const float *)x_device);
-    } else {
+    const bool ok = with_precision(st, [&](auto t) {
+        using T = decltype(t);
+        if (st->kernel == SPMV_B200_KERNEL_BAND_SEG) return launch_seg_bands<T>(st, band_first, band_count, (const T *)x_device);
         const int r0 = band_first * st->m, r1 = (band_first + band_count) * st->m;  // virtual rows of these bands
-        if (st->vsize == 8) {
-            PeerList<double> none;
-            none.n = 0;
-            for (int i = 0; i < kMaxPeers; ++i) none.p[i] = nullptr;
-            launch_vector_mode<double>(st, r0, r1, (const double *)x_device, st->v.y.as<double>(), none);
-        } else {
-            PeerList<float> none;
-            none.n = 0;
-            for (int i = 0; i < kMaxPeers; ++i) none.p[i] = nullptr;
-            launch_vector_mode<float>(st, r0, r1, (const float *)x_device, st->v.y.as<float>(), none);
-        }
-        ok = SB_CUDA(cudaGetLastError());
-    }
+        launch_vector<T>(st, r0, r1, (const T *)x_device, st->v.y.as<T>(), PeerList<T>{});
+        return SB_CUDA(cudaGetLastError());
+    });
     return ok ? 0 : -1;
 }
-
-}  // extern "C"
-
-template <typename T>
-static bool finish_banded(DeviceState *st, T *y)
-{
-    PeerList<T> peers;
-    peers.n = st->n_peers;
-    for (int i = 0; i < kMaxPeers; ++i) peers.p[i] = (T *)st->peers[i];
-    if (peers.n > 0) band_reduce_kernel<T, true><<<blocks_for(st->m), kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), y, peers);
-    else band_reduce_kernel<T, false><<<blocks_for(st->m), kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), y, peers);
-    count_launch();
-    return SB_CUDA(cudaGetLastError());
-}
-
-extern "C" {
 
 int spmv_b200_spmv_finish(spmv_Handle_t handle, void *y_device)
 {
@@ -1599,11 +1593,10 @@ int spmv_b200_spmv_finish(spmv_Handle_t handle, void *y_device)
     if (!is_device_ptr(y_device)) { set_error("spmv_b200_spmv_finish: y must be a device pointer"); return -1; }
     std::lock_guard<std::mutex> lock(st->mu);
     DeviceGuard guard(st->device);
-    bool ok;
-    if (st->kernel == SPMV_B200_KERNEL_BAND_SEG)
-        ok = st->vsize == 8 ? launch_seg_finish<double>(st, (double *)y_device) : launch_seg_finish<float>(st, (float *)y_device);
-    else
-        ok = st->vsize == 8 ? finish_banded<double>(st, (double *)y_device) : finish_banded<float>(st, (float *)y_device);
+    const bool ok = with_precision(st, [&](auto t) {
+        using T = decltype(t);
+        return st->kernel == SPMV_B200_KERNEL_BAND_SEG ? launch_seg_finish<T>(st, (T *)y_device) : launch_band_fold<T>(st, (T *)y_device);
+    });
     return ok ? 0 : -1;
 }
 
@@ -1800,17 +1793,14 @@ int spmv_b200_partition_rows(const int *RowPtr, int m, int parts, int *splitter_
 int spmv_b200_recommend_method(int m, const int *RowPtr)
 {
     if (!RowPtr || m < 0) return -1;
-    if (m < 8192) return Method_Parallel;
     const long long nnz = (long long)RowPtr[m] - RowPtr[0];
-    if (nnz <= 0) return Method_Parallel;
-    const double mean = (double)nnz / m;
-    const long long cut = (long long)(4.0 * mean) + 16;
-    long long heavy = 0;  // non-zeros in rows much longer than the mean
-    for (int r = 0; r < m; ++r) {
-        const long long len = (long long)RowPtr[r + 1] - RowPtr[r];
-        if (len > cut) heavy += len;
-    }
-    return (4 * heavy > nnz) ? Method_CSR5SPMV : Method_SellCSigma;
+    return pick_method(m, nnz, /*far_fraction: unknown*/ -1.0, [&](int cut, long long *heavy) {
+        for (int r = 0; r < m; ++r) {
+            const long long len = (long long)RowPtr[r + 1] - RowPtr[r];
+            if (len > cut) *heavy += len;
+        }
+        return true;
+    });
 }
 
 void *spmv_b200_malloc(size_t bytes)
