@@ -8,6 +8,7 @@
 #include <string>
 #include <map>
 #include <utility>
+#include <type_traits>
 #include <cmath>
 #include <vector>
 #include <cub/device/device_scan.cuh>
@@ -95,11 +96,28 @@ static bool is_device_ptr(const void *p)
 
 static inline int blocks_for(long long threads) { return (int)((threads + kThreads - 1) / kThreads); }
 
+// Column bands: the n columns cut into K bands of band_cols = ceil(n / K).  Band b of K holds the columns [lo, hi);
+// the last band ends at n, so K = 1 is all n columns.
+static int cols_per_band(const DeviceState *st, int K) { return (int)(((long long)st->n + K - 1) / K); }
+static std::pair<long long, long long> band_columns(const DeviceState *st, int b, int K)
+{
+    const long long n = st->n, lo = (long long)b * st->band_cols, hi = lo + st->band_cols;
+    return {lo < n ? lo : n, b == K - 1 || hi > n ? n : hi};
+}
+
 // f(T()) with the handle's value type: T = double for fp64, float for fp32
 template <typename F>
 static auto with_precision(const DeviceState *st, F f)
 {
     return st->vsize == 8 ? f(double()) : f(float());
+}
+
+// f(std::integral_constant<int, V>()) for the first V of the list equal to v, or for the last V when none is
+template <int V, int... Rest, typename F>
+static auto with_value(int v, F f)
+{
+    if constexpr (sizeof...(Rest) == 0) return f(std::integral_constant<int, V>());
+    else return v == V ? f(std::integral_constant<int, V>()) : with_value<Rest...>(v, f);
 }
 
 struct DeviceGuard {  // library code is device-agnostic: run on the handle's device, then restore
@@ -302,7 +320,7 @@ static bool build_band_major(DeviceState *st)
     if (bands > kMaxBands) bands = kMaxBands;
     if ((long long)st->m * bands > 0x7fffffffLL - 8192) return true;
     const int K = (int)bands, m = st->m;
-    const int band_cols = (int)(((long long)st->n + K - 1) / K);
+    const int band_cols = cols_per_band(st, K);
     const size_t vm = (size_t)m * K;
     DeviceArray<int> counts;
     // The band-major copy is a speed-up only: when it cannot be allocated (or built) the handle keeps running the
@@ -612,7 +630,7 @@ template <typename T, typename MaskT>
 static bool build_band_seg_t(DeviceState *st)
 {
     const int K = st->seg.bands, nnz = st->nnz, m = st->m;
-    st->band_cols = (int)(((long long)st->n + K - 1) / K);
+    st->band_cols = cols_per_band(st, K);
     st->seg.mask64 = sizeof(MaskT) == 8;
     int tiles = 0, h_cross = 0, h_segs[2] = {0, 0};
     {  // the temporaries (about 15 bytes per entry) are freed before the segment sums are allocated
@@ -932,18 +950,12 @@ static PeerList<T> peers_of(const DeviceState *st)
 template <typename T>
 static void launch_vector(DeviceState *st, int row0, int row1, const T *x, T *y, const PeerList<T> &peers, int fuse_bands = 0)
 {
-    const int tpr = st->tpr;
-    const int grid = blocks_for((long long)(row1 - row0) * tpr);
+    const int grid = blocks_for((long long)(row1 - row0) * st->tpr);
     if (grid <= 0) return;
-#define SB_ARGS row0, row1, st->lr.thr, st->a_rowptr, st->a_col, (const T *)st->a_val, x, y, peers, fuse_bands, st->m, st->v.y.as<T>()
-#define SB_CASE(N) case N: \
-        if (fuse_bands > 0) csr_vector_kernel<T, N, false, true><<<grid, kThreads, 0, st->stream>>>(SB_ARGS); \
-        else if (peers.n > 0) csr_vector_kernel<T, N, true, false><<<grid, kThreads, 0, st->stream>>>(SB_ARGS); \
-        else csr_vector_kernel<T, N, false, false><<<grid, kThreads, 0, st->stream>>>(SB_ARGS); \
-        break;
-    switch (tpr) { SB_CASE(1) SB_CASE(2) SB_CASE(4) SB_CASE(8) SB_CASE(16) default: SB_CASE(32) }
-#undef SB_CASE
-#undef SB_ARGS
+    const auto kernel = with_value<1, 2, 4, 8, 16, 32>(st->tpr, [&](auto N) {
+        return fuse_bands > 0 ? csr_vector_kernel<T, N, false, true> : peers.n > 0 ? csr_vector_kernel<T, N, true, false> : csr_vector_kernel<T, N, false, false>;
+    });
+    kernel<<<grid, kThreads, 0, st->stream>>>(row0, row1, st->lr.thr, st->a_rowptr, st->a_col, (const T *)st->a_val, x, y, peers, fuse_bands, st->m, st->v.y.as<T>());
     count_launch();
 }
 
@@ -952,8 +964,8 @@ template <typename T>
 static bool launch_band_fold(DeviceState *st, T *y_out)
 {
     const PeerList<T> peers = peers_of<T>(st);
-    if (peers.n > 0) band_reduce_kernel<T, true><<<blocks_for(st->m), kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), y_out, peers);
-    else band_reduce_kernel<T, false><<<blocks_for(st->m), kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), y_out, peers);
+    const auto kernel = peers.n > 0 ? band_reduce_kernel<T, true> : band_reduce_kernel<T, false>;
+    kernel<<<blocks_for(st->m), kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), y_out, peers);
     count_launch();
     return SB_CUDA(cudaGetLastError());
 }
@@ -990,14 +1002,14 @@ static bool launch_seg_bands(DeviceState *st, int b0, int count, const T *x)
 {
     const int t0 = st->seg.tile0[b0], t1 = st->seg.tile0[b0 + count];
     if (t1 <= t0) return true;
-    if (st->seg.grid == 0) {  // persistent CTAs: option seg_ctas per SM (shared memory AND registers allow 2 or 3)
-        st->seg.ctas = (int)opt("seg_ctas");
-        if (st->seg.ctas != 3) st->seg.ctas = 2;
-        const void *fn = st->seg.ctas == 3 ? (const void *)bseg_kernel<T, 3> : (const void *)bseg_kernel<T, 2>;
-        SB_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bseg_smem_bytes<T>()));
+    // persistent CTAs: option seg_ctas per SM (shared memory AND registers allow 2 or 3), read at the first launch
+    if (st->seg.grid == 0) st->seg.ctas = (int)opt("seg_ctas") == 3 ? 3 : 2;
+    const auto kernel = st->seg.ctas == 3 ? bseg_kernel<T, 3> : bseg_kernel<T, 2>;
+    if (st->seg.grid == 0) {
+        SB_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bseg_smem_bytes<T>()));
         // leave the rest of the unified array to L1: the gathers need lines for their outstanding misses
         const int carve = (int)((st->seg.ctas * (bseg_smem_bytes<T>() + 2048) * 100 + 228 * 1024 - 1) / (228 * 1024));
-        SB_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, carve > 100 ? 100 : carve));
+        SB_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, carve > 100 ? 100 : carve));
         st->seg.grid = st->seg.ctas * (st->dev_sms > 0 ? st->dev_sms : 1);
     }
     const int grid = t1 - t0 < st->seg.grid ? t1 - t0 : st->seg.grid;
@@ -1009,10 +1021,8 @@ static bool launch_seg_bands(DeviceState *st, int b0, int count, const T *x)
     const int pf_opt = opt_cached_seg_prefetch();
     const bool two_fit = 2.0 * (double)st->band_cols * st->vsize <= 0.53 * (double)st->dev_l2;
     const int pf_on = (((uintptr_t)x & 15u) == 0 && (pf_opt == 2 || (pf_opt == 1 && two_fit))) ? 1 : 0;
-#define SB_SEG(MINB) bseg_kernel<T, MINB><<<grid, kSegThreads, bseg_smem_bytes<T>(), st->stream>>>(t0, t1, pf_on, st->seg.ticket, st->seg.tile_ent, st->seg.tile_seg0, \
-        st->seg.col, st->seg.ent_val.as<T>(), x, st->seg.sums.as<T>(), st->tile.carry_val.as<T>(), st->tile.carry_row)
-    if (st->seg.ctas == 3) SB_SEG(3); else SB_SEG(2);
-#undef SB_SEG
+    kernel<<<grid, kSegThreads, bseg_smem_bytes<T>(), st->stream>>>(t0, t1, pf_on, st->seg.ticket, st->seg.tile_ent, st->seg.tile_seg0, st->seg.col,
+        st->seg.ent_val.as<T>(), x, st->seg.sums.as<T>(), st->tile.carry_val.as<T>(), st->tile.carry_row);
     count_launch();
     return SB_CUDA(cudaGetLastError());
 }
@@ -1024,11 +1034,12 @@ static bool launch_seg_finish(DeviceState *st, T *y_out)
     cudaStream_t s = st->stream;
     if (st->seg.cross) launch_carry_fixup<T>(st, s, st->tile.count * kSegChunks, st->tile.carry_row, st->tile.carry_val.as<T>(), st->seg.sums.as<T>());
     const PeerList<T> pr = peers_of<T>(st);
-#define SB_MERGE(M, P) bseg_merge_kernel<T, M, P><<<blocks_for((long long)st->seg.groups * 32), kThreads, 0, s>>>(0, st->m, st->seg.bands, st->seg.mask.as<M>(), \
-                                                                                     st->seg.gbase, st->seg.sums.as<T>(), y_out, pr)
-    if (st->seg.mask64) { if (pr.n > 0) SB_MERGE(unsigned long long, true); else SB_MERGE(unsigned long long, false); }
-    else { if (pr.n > 0) SB_MERGE(uint32_t, true); else SB_MERGE(uint32_t, false); }
-#undef SB_MERGE
+    auto merge = [&](auto mask_word) {  // row masks of 32 or 64 bands
+        using M = decltype(mask_word);
+        const auto kernel = pr.n > 0 ? bseg_merge_kernel<T, M, true> : bseg_merge_kernel<T, M, false>;
+        kernel<<<blocks_for((long long)st->seg.groups * 32), kThreads, 0, s>>>(0, st->m, st->seg.bands, st->seg.mask.as<M>(), st->seg.gbase, st->seg.sums.as<T>(), y_out, pr);
+    };
+    if (st->seg.mask64) merge((unsigned long long)0); else merge(uint32_t(0));
     count_launch();
     return SB_CUDA(cudaGetLastError());
 }
@@ -1051,10 +1062,9 @@ static bool launch(DeviceState *st, const T *x, T *y_out)
     const bool banded = st->x_bands > 1;
     T *y = banded ? st->v.y.as<T>() : y_out;
     const T *val = (const T *)st->a_val;
-    // extra y destinations (fused all-gather): written by whichever kernel produces the FINAL y
-    const PeerList<T> peers = peers_of<T>(st), none{};
-    const PeerList<T> &direct = banded ? none : peers;  // kernels write virtual y when banded
-    bool scattered = peers.n == 0;
+    // extra y destinations (fused all-gather), written with the final y: by the band fold when banded, else here
+    const PeerList<T> fused = banded ? PeerList<T>{} : peers_of<T>(st);
+    bool wrote_fused = false;  // the case's kernels (and the long-row pass) wrote every final value to `fused` too
     switch (st->kernel) {
     case SPMV_B200_KERNEL_CSR_REFORDER: {
         constexpr int L = sizeof(T) == 8 ? 4 : 8;
@@ -1071,57 +1081,45 @@ static bool launch(DeviceState *st, const T *x, T *y_out)
             for (int b = 0; b < 3; ++b) {
                 const int count = st->lr.bin_ptr[b + 1] - st->lr.bin_ptr[b];
                 if (count <= 0) continue;
-                const int grid = blocks_for((long long)count * lanes[b]);
-                const int *list = st->lr.bin_list + st->lr.bin_ptr[b];
-#define SB_BIN(N) if (direct.n > 0) csr_vector_list_kernel<T, N, true><<<grid, kThreads, 0, s>>>(count, list, st->a_rowptr, st->a_col, val, x, y, direct); \
-                  else csr_vector_list_kernel<T, N, false><<<grid, kThreads, 0, s>>>(count, list, st->a_rowptr, st->a_col, val, x, y, direct)
-                if (b == 0) { SB_BIN(1); } else if (b == 1) { SB_BIN(4); } else { SB_BIN(16); }
-#undef SB_BIN
+                const auto kernel = with_value<1, 4, 16>(lanes[b], [&](auto N) {
+                    return fused.n > 0 ? csr_vector_list_kernel<T, N, true> : csr_vector_list_kernel<T, N, false>;
+                });
+                kernel<<<blocks_for((long long)count * lanes[b]), kThreads, 0, s>>>(count, st->lr.bin_list + st->lr.bin_ptr[b], st->a_rowptr, st->a_col, val, x, y, fused);
                 count_launch();
             }
         } else {
-            launch_vector<T>(st, 0, m, x, y, direct);
+            launch_vector<T>(st, 0, m, x, y, fused);
         }
-        scattered = scattered || !banded;
+        wrote_fused = true;
         break;
     case SPMV_B200_KERNEL_ROW_BLOCKS: {
-        const int grid = blocks_for((long long)st->split.parts * 32);
-#define SB_RB(P) row_block_kernel<T, P><<<grid, kThreads, 0, s>>>(st->split.parts, st->split.splitter, st->a_rowptr, st->a_col, val, x, y, direct)
-        if (direct.n > 0) SB_RB(true); else SB_RB(false);
-#undef SB_RB
-        scattered = scattered || !banded;
+        const auto kernel = fused.n > 0 ? row_block_kernel<T, true> : row_block_kernel<T, false>;
+        kernel<<<blocks_for((long long)st->split.parts * 32), kThreads, 0, s>>>(st->split.parts, st->split.splitter, st->a_rowptr, st->a_col, val, x, y, fused);
+        wrote_fused = true;
         count_launch();
         break;
     }
     case SPMV_B200_KERNEL_MERGE_PATH: {
-        if (st->tile.items == 4)
-            merge_path_kernel<T, 4><<<st->tile.count, kThreads, 0, s>>>(m, st->nnz, st->tile.merge_coords, st->a_rowptr, st->a_col, val, x, y, st->tile.carry_val.as<T>(), st->tile.carry_row);
-        else
-            merge_path_kernel<T, 8><<<st->tile.count, kThreads, 0, s>>>(m, st->nnz, st->tile.merge_coords, st->a_rowptr, st->a_col, val, x, y, st->tile.carry_val.as<T>(), st->tile.carry_row);
+        const auto kernel = st->tile.items == 4 ? merge_path_kernel<T, 4> : merge_path_kernel<T, 8>;
+        kernel<<<st->tile.count, kThreads, 0, s>>>(m, st->nnz, st->tile.merge_coords, st->a_rowptr, st->a_col, val, x, y, st->tile.carry_val.as<T>(), st->tile.carry_row);
         launch_carry_fixup<T>(st, s, st->tile.count, st->tile.carry_row, st->tile.carry_val.as<T>(), y);
         count_launch();
         break;
     }
     case SPMV_B200_KERNEL_NNZ_SPLIT: {
-        if (st->tile.items == 4)
-            nnz_split_kernel<T, 4><<<st->tile.count, kThreads, 0, s>>>(m, st->nnz, st->tile.rows, st->a_rowptr, st->a_col, val, x, y, st->tile.carry_val.as<T>(), st->tile.carry_row);
-        else
-            nnz_split_kernel<T, 8><<<st->tile.count, kThreads, 0, s>>>(m, st->nnz, st->tile.rows, st->a_rowptr, st->a_col, val, x, y, st->tile.carry_val.as<T>(), st->tile.carry_row);
+        const auto kernel = st->tile.items == 4 ? nnz_split_kernel<T, 4> : nnz_split_kernel<T, 8>;
+        kernel<<<st->tile.count, kThreads, 0, s>>>(m, st->nnz, st->tile.rows, st->a_rowptr, st->a_col, val, x, y, st->tile.carry_val.as<T>(), st->tile.carry_row);
         launch_carry_fixup<T>(st, s, st->tile.count, st->tile.carry_row, st->tile.carry_val.as<T>(), y);
         count_launch();
         break;
     }
     case SPMV_B200_KERNEL_SELL: {
         if (st->sell.slices > 0) {
-            const PeerList<T> &sp = (st->sell.banner == m) ? direct : none;
-            const int sgrid = blocks_for((long long)st->sell.slices * 32);
-#define SB_SELL(P, U, MINB) sell_kernel<T, P, U, MINB><<<sgrid, kThreads, 0, s>>>( \
-                st->sell.slices, st->sell.slice_ptr, st->sell.full, st->sell.perm, st->sell.col, st->sell.val.as<T>(), x, y, sp)
-            if (sp.n > 0) SB_SELL(true, 8, 6);
-            else if (st->sell.variant == 2) SB_SELL(false, 4, 8);
-            else SB_SELL(false, 8, 6);
-#undef SB_SELL
-            scattered = scattered || (!banded && st->sell.banner == m);
+            wrote_fused = st->sell.banner == m;  // no CSR tail: the SELL kernel writes every final value
+            const PeerList<T> sp = wrote_fused ? fused : PeerList<T>{};
+            const auto kernel = sp.n > 0 ? sell_kernel<T, true, 8, 6> : st->sell.variant == 2 ? sell_kernel<T, false, 4, 8> : sell_kernel<T, false, 8, 6>;
+            kernel<<<blocks_for((long long)st->sell.slices * 32), kThreads, 0, s>>>(
+                st->sell.slices, st->sell.slice_ptr, st->sell.full, st->sell.perm, st->sell.col, st->sell.val.as<T>(), x, y, sp);
             count_launch();
         }
         if (st->sell.banner < m) {
@@ -1137,10 +1135,9 @@ static bool launch(DeviceState *st, const T *x, T *y_out)
         }
         const T *tval = st->c5.val.as<T>();
         if (p > 1) {
-            const int grid = blocks_for((long long)(p - 1) * 32);
-#define SB_C5(SG) csr5_kernel<T, SG><<<grid, kThreads, 0, s>>>(p, st->c5.bit_y, st->c5.bit_ss, st->c5.tile_ptr, st->c5.tile_desc, st->c5.off_ptr, st->c5.off, st->c5.col, tval, x, y, st->tile.carry_val.as<T>(), st->tile.carry_row)
-            if (st->c5.sigma == 4) SB_C5(4); else if (st->c5.sigma == 8) SB_C5(8); else SB_C5(16);
-#undef SB_C5
+            const auto kernel = with_value<4, 8, 16>(st->c5.sigma, [](auto SG) { return csr5_kernel<T, SG>; });
+            kernel<<<blocks_for((long long)(p - 1) * 32), kThreads, 0, s>>>(
+                p, st->c5.bit_y, st->c5.bit_ss, st->c5.tile_ptr, st->c5.tile_desc, st->c5.off_ptr, st->c5.off, st->c5.col, tval, x, y, st->tile.carry_val.as<T>(), st->tile.carry_row);
             count_launch();
         }
         const int tail_nz0 = (p - 1) * kC5Omega * st->c5.sigma;
@@ -1155,18 +1152,17 @@ static bool launch(DeviceState *st, const T *x, T *y_out)
         return false;
     }
     if (st->lr.rows > 0) {  // hub rows / SELL overflow: segment sums, then one ordered add per row
-        const int single = direct.n == 0;  // with peer destinations every final value goes through long_final_kernel
+        const int single = fused.n == 0;  // with peer destinations every final value goes through long_final_kernel
         long_seg_kernel<T><<<blocks_for((long long)st->lr.segs * 32), kThreads, 0, s>>>(
             st->lr.segs, st->lr.seg_row, st->lr.row, st->lr.start, st->lr.seg_ptr, st->a_rowptr, st->a_col, val, x, st->lr.partial.as<T>(),
             y, single, st->lr.accumulate);
-        const int fgrid = blocks_for((long long)st->lr.rows * 32);
-        if (direct.n > 0) long_final_kernel<T, true><<<fgrid, kThreads, 0, s>>>(st->lr.rows, st->lr.accumulate, single, st->lr.row, st->lr.seg_ptr, st->lr.partial.as<T>(), y, direct);
-        else long_final_kernel<T, false><<<fgrid, kThreads, 0, s>>>(st->lr.rows, st->lr.accumulate, single, st->lr.row, st->lr.seg_ptr, st->lr.partial.as<T>(), y, direct);
+        const auto final_kernel = fused.n > 0 ? long_final_kernel<T, true> : long_final_kernel<T, false>;
+        final_kernel<<<blocks_for((long long)st->lr.rows * 32), kThreads, 0, s>>>(st->lr.rows, st->lr.accumulate, single, st->lr.row, st->lr.seg_ptr, st->lr.partial.as<T>(), y, fused);
         count_launch(2);
     }
-    if (banded) return launch_band_fold<T>(st, y_out);  // writes the peers too
-    if (!scattered) {  // kernel family without a fused epilogue: one stream-ordered copy to the peers
-        peer_copy_kernel<T><<<blocks_for(st->m), kThreads, 0, s>>>(st->m, y_out, peers);
+    if (banded) return launch_band_fold<T>(st, y_out);  // y and the peers
+    if (fused.n > 0 && !wrote_fused) {  // kernels without a fused epilogue: one stream-ordered copy to the peers
+        peer_copy_kernel<T><<<blocks_for(st->m), kThreads, 0, s>>>(st->m, y_out, fused);
         count_launch();
     }
     return SB_CUDA(cudaGetLastError());
@@ -1198,13 +1194,12 @@ static bool run_pipelined(DeviceState *st, const T *hx, T *hy)
     SB_TRY(cudaEventRecord(st->ev_start, s));
     SB_TRY(cudaStreamWaitEvent(st->s_in, st->ev_start, 0));
     SB_TRY(cudaStreamWaitEvent(st->s_out, st->ev_start, 0));
-    auto piece_lo = [&](int p) -> long long { return banded ? (long long)p * st->band_cols : (long long)n * p / pieces; };
-    auto piece_hi = [&](int p) -> long long {
-        long long hi = banded ? (long long)(p + 1) * st->band_cols : (long long)n * (p + 1) / pieces;
-        return (p == pieces - 1 || hi > n) ? n : hi;
+    auto piece = [&](int p) -> std::pair<long long, long long> {  // columns [lo, hi) of x in piece p
+        if (banded) return band_columns(st, p, pieces);
+        return {(long long)n * p / pieces, p == pieces - 1 ? n : (long long)n * (p + 1) / pieces};
     };
     for (int p = 0; p < pieces; ++p) {
-        const long long lo = piece_lo(p), hi = piece_hi(p);
+        const auto [lo, hi] = piece(p);
         if (hi > lo) SB_TRY(cudaMemcpyAsync(xd + lo, hx + lo, (size_t)(hi - lo) * sizeof(T), cudaMemcpyHostToDevice, st->s_in));
         SB_TRY(cudaEventRecord(st->ev_in[p], st->s_in));
     }
@@ -1235,7 +1230,7 @@ static bool run_pipelined(DeviceState *st, const T *hx, T *hy)
         for (int c = 0; c < kPipeChunks; ++c) {
             const int r0 = (int)((long long)m * c / kPipeChunks), r1 = (int)((long long)m * (c + 1) / kPipeChunks);
             int p = 0;
-            while (p < pieces - 1 && piece_hi(p) < st->chunk_xmax[c]) ++p;
+            while (p < pieces - 1 && piece(p).second < st->chunk_xmax[c]) ++p;
             if (!need_piece(p)) return false;
             launch_vector<T>(st, r0, r1, xd, yd, none);
             if (!chunk_out(c, r0, r1)) return false;
@@ -1560,11 +1555,9 @@ int spmv_b200_band_columns(spmv_Handle_t handle, int band, long long *col_lo, lo
     if (!st || !st->ok || band < 0) return -1;
     const int K = stageable(st) ? st->x_bands : 1;
     if (band >= K) return -1;
-    const long long lo = K == 1 ? 0 : (long long)band * st->band_cols;
-    long long hi = K == 1 ? st->n : lo + st->band_cols;
-    if (band == K - 1 || hi > st->n) hi = st->n;
-    if (col_lo) *col_lo = lo < st->n ? lo : st->n;
-    if (col_hi) *col_hi = hi;
+    const auto cols = band_columns(st, band, K);
+    if (col_lo) *col_lo = cols.first;
+    if (col_hi) *col_hi = cols.second;
     return 0;
 }
 
