@@ -94,6 +94,25 @@ class DeviceBytes {
 };
 
 // ------------------------------------------------------------------------------------------------
+// The options of one create (include/spmv_b200.h), read once at its start by read_create_options, which applies every
+// key's rule: the builders see only these values.  seg_ctas and seg_prefetch are read at launch.
+// ------------------------------------------------------------------------------------------------
+struct CreateOptions {
+    int sell_sigma;         // a multiple of 32 in [32, 4096]
+    int sell_variant;       // 0, 2, or -1 = automatic
+    int sell_cap;           // [32, 2^20], or 0 = off
+    int csr5_sigma;         // 4, 8, 16, or 0 = automatic
+    long long block_nnz;    // >= 32
+    int tile_items;         // 4 or 8
+    int tpr;                // forced lanes per row (1, 2, 4, 8, 16, 32), or 0 = from the mean
+    bool row_bins;          // Method_Parallel may bin its rows: "row_bins" on and the raw "tpr" 0
+    long long long_thr;     // 0 = automatic, < 0 = off, else forced
+    int x_bands;            // 0 = automatic, 1 = off, 2 .. kMaxBands forced
+    int seg_bands;          // 0 = automatic, -1 = never, 2 .. kSegMaxBands forced (overrides x_bands)
+    bool force_merge, pipeline, auto_pick, reorder, pin_host, refresh;
+};
+
+// ------------------------------------------------------------------------------------------------
 // Device-resident state hanging off spmv_Handle::extraHandle.  The device arrays are grouped by the builder that
 // fills them, each group with the sizes that describe its arrays.
 // ------------------------------------------------------------------------------------------------
@@ -115,8 +134,10 @@ struct DeviceState {
     int dev_sms = 0;
     long long dev_l2 = 0;
     int layout_fallbacks = 0;       // optional layouts (band copy, band segments, row bins) that could not be built
+    CreateOptions opts = {};        // the options in force at create
     // option "refresh": every value array below keeps its source map (refresh.cuh) in its own group, so that dropping a
-    // layout drops its map too.  Cleared at create when a map could not be built: the handle then cannot be refreshed
+    // layout drops its map too.  Starts as opts.refresh; cleared at create when a map could not be built: the handle
+    // then cannot be refreshed
     bool refresh = false;
     bool map_failed = false;
     int n_peers = 0;                // spmv_b200_set_y_peers
@@ -135,7 +156,6 @@ struct DeviceState {
     // buffer while the handle lives.  Undone at clear / destroy or when the caller switches buffers
     struct PinSlot { const void *ptr = nullptr; size_t bytes = 0; int seen = 0; bool registered = false; };
     PinSlot pin[2];
-    bool pin_host = false;
     // staging for host-side x / y; the pipelined host path (CSR-vector kernel) copies x in pieces on s_in,
     // computes row chunks as soon as their prefix of x has arrived, and returns finished chunks of y on s_out
     struct Staging { DeviceBytes x, y, val; } stage;  // val: host values of spmv_b200_set_values, when no upload takes them
@@ -201,7 +221,7 @@ struct DeviceState {
     } c5;
     // hyper-sparse column bands as band segments (band_seg.cuh): x_bands = K but the active view stays the CSR
     struct BandSegments {
-        int bands = 0;                  // K (option / info key names kept from round 1: "coo_bands")
+        int bands = 0;                  // K, or 0 = no band segments (option and info key "seg_bands")
         int ptr[kMaxPieces + 1] = {};   // first slot of every band in col / ent_val (aligned to 4), [K] = end
         int cnt[kMaxPieces] = {};       // entries of every band
         int tile0[kMaxPieces + 1] = {}; // first tile of every band

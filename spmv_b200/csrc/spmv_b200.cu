@@ -3,6 +3,7 @@
 // adopts) the CSR arrays once and builds the device layout of the requested SPMV_METHODS value;
 // spmv() launches the matching sm_100a kernel family.  There is no CPU compute path in this file.
 #include <cstdarg>
+#include <algorithm>
 #include <atomic>
 #include <mutex>
 #include <string>
@@ -81,6 +82,37 @@ static long long opt(const char *key)
         if (const char *e = getenv(env.c_str())) return atoll(e);
     }
     return it->second;
+}
+
+// Every option a create reads, each read once and with its rule applied (the meaning of each field: CreateOptions)
+static CreateOptions read_create_options()
+{
+    CreateOptions o;
+    o.sell_sigma = (int)(std::clamp(opt("sell_sigma"), (long long)kSellC, (long long)kSellMaxSigma) / kSellC * kSellC);
+    const long long variant = opt("sell_variant");
+    o.sell_variant = variant == 0 || variant == 2 ? (int)variant : -1;
+    const long long cap = opt("sell_cap");  // 0 = off (the reference's widths), else the widest slice allowed
+    o.sell_cap = cap <= 0 ? 0 : (int)std::clamp(cap, 32LL, 1LL << 20);
+    const long long c5 = opt("csr5_sigma");
+    o.csr5_sigma = c5 == 4 || c5 == 8 || c5 == 16 ? (int)c5 : 0;
+    o.block_nnz = std::max(opt("block_nnz"), 32LL);
+    o.tile_items = opt("tile_items") == 4 ? 4 : 8;
+    const long long tpr = opt("tpr");
+    o.tpr = tpr == 1 || tpr == 2 || tpr == 4 || tpr == 8 || tpr == 16 || tpr == 32 ? (int)tpr : 0;
+    // any tpr but 0 switches the row bins off, also a value such as 3 that takes the tpr from the mean
+    o.row_bins = tpr == 0 && opt("row_bins") != 0;
+    o.long_thr = opt("long_thr");
+    const long long x_bands = opt("x_bands");
+    o.x_bands = x_bands == 0 ? 0 : (int)std::clamp(x_bands, 1LL, (long long)kMaxBands);
+    const long long seg_bands = opt("seg_bands");
+    o.seg_bands = seg_bands == 0 ? 0 : seg_bands < 2 ? -1 : (int)std::min(seg_bands, (long long)kSegMaxBands);
+    o.force_merge = opt("force_merge") != 0;
+    o.pipeline = opt("pipeline") != 0;
+    o.auto_pick = opt("auto") != 0;
+    o.reorder = opt("reorder") != 0;
+    o.pin_host = opt("pin_host") != 0;
+    o.refresh = opt("refresh") != 0;
+    return o;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -258,14 +290,12 @@ static void apply_device_limits(DeviceState *st)
     if (cudaGetDeviceProperties(&prop, st->device) != cudaSuccess) { cudaGetLastError(); return; }
     st->dev_sms = prop.multiProcessorCount;
     st->dev_l2 = prop.l2CacheSize;
-    st->pin_host = opt("pin_host") != 0;
 }
 
-static int pick_tpr(long long nnz, int m)
+static int pick_tpr(const DeviceState *st)
 {
-    const long long forced = opt("tpr");
-    if (forced == 1 || forced == 2 || forced == 4 || forced == 8 || forced == 16 || forced == 32) return (int)forced;
-    const double mean = m > 0 ? (double)nnz / m : 0.0;
+    if (st->opts.tpr) return st->opts.tpr;
+    const double mean = st->a_m > 0 ? (double)st->nnz / st->a_m : 0.0;
     int tpr = 1;
     // measured on B200 (scripts/sweep.py): ~7 entries per lane is the sweet spot -- fewer lanes per row
     // means more independent x gathers in flight per thread (mean 5 -> 1, 10.7 -> 2, 27 -> 4, 32 -> 8)
@@ -273,53 +303,62 @@ static int pick_tpr(long long nnz, int m)
     return tpr;
 }
 
-// Decide the number of column bands and, when > 1, build the band-major copy and make it the active view.
-template <typename T>
-static bool build_band_major(DeviceState *st)
+// the bytes of x that random gathers can keep in L2
+static double l2_reach(long long dev_l2) { return dev_l2 > 0 ? 0.5 * (double)dev_l2 : 63.0 * 1048576.0; }
+
+// Locality probe (m > 0, nnz > 0): the share of entries further than 1/8 of the L2 reach from the (scaled) diagonal.
+// > 25 % = gather-dominated (bound by L2 requests), else diagonal-local (bound by DRAM).  It decides whether banding
+// can pay (decide_bands), which SELL kernel flavour runs (build_sell) and the method option "auto" picks.
+static bool probe_locality(DeviceState *st)
 {
-    st->a_m = st->m; st->a_rowptr = st->rowptr; st->a_col = st->col; st->a_val = st->val;
-    if (st->m == 0 || st->nnz == 0) return true;
-    long long bands = opt("x_bands");  // 0 = automatic, 1 = off, >= 2 forced
-    const double xbytes = (double)st->n * st->vsize;
-    const double usable = st->dev_l2 > 0 ? 0.5 * (double)st->dev_l2 : 63.0 * 1048576.0;  // random-access reach
-    {
-        // locality probe: the share of entries further than 1/8 of the L2 reach from the (scaled) diagonal.
-        // > 25 % = gather-dominated (bound by L2 requests), else diagonal-local (bound by DRAM).  It decides
-        // whether banding can pay (below) and which SELL kernel flavour runs (build_sell).
-        const int halfwidth = (int)(0.125 * usable / st->vsize);
-        unsigned long long h_far = 0;
-        const bool probed = read_counter(st, &h_far, [&](unsigned long long *far) {
-            band_locality_kernel<<<blocks_for(st->m), kThreads, 0, st->stream>>>(
-                st->m, (double)st->n / st->m, halfwidth, st->rowptr, st->col, far);
-        });
-        if (!probed) return false;  // a 8-byte allocation or a trivial kernel failed: the device is unusable
-        st->far_fraction = (double)h_far / (double)st->nnz;
-    }
-    if (bands == 0) {
-        bands = 1;
+    const int halfwidth = (int)(0.125 * l2_reach(st->dev_l2) / st->vsize);
+    unsigned long long h_far = 0;
+    const bool probed = read_counter(st, &h_far, [&](unsigned long long *far) {
+        band_locality_kernel<<<blocks_for(st->m), kThreads, 0, st->stream>>>(
+            st->m, (double)st->n / st->m, halfwidth, st->rowptr, st->col, far);
+    });
+    if (!probed) return false;  // a 8-byte allocation or a trivial kernel failed: the device is unusable
+    st->far_fraction = (double)h_far / (double)st->nnz;
+    return true;
+}
+
+// The column bands of a matrix with m > 0 rows and nnz > 0 entries: {K of the band-major copy (1 = none), bands of
+// the band segments (0 = none)}.
+static std::pair<int, int> decide_bands(long long m, long long n, long long nnz, int vsize, long long dev_l2,
+                                        double far_fraction, const CreateOptions &o)
+{
+    if (o.seg_bands >= 2) return {1, o.seg_bands};  // forced band segments: no band-major copy
+    int K = o.x_bands, seg = 0;
+    if (K == 0) {
+        K = 1;
+        const double xbytes = (double)n * vsize, usable = l2_reach(dev_l2);
         // x up to ~1.2x the reach still gathers at >= 85 % of the L2 rate (profiles/r01_gather_probe.txt) and
         // banding costs 15-20 % (virtual row pointers, partial y): R-MAT s24 fp32 (x = 64 MiB) measured 7-15 %
         // FASTER unbanded, uniform fp64 (x = 128 MiB) 1.9x faster banded.  Banding only pays when the accesses
         // are NOT already diagonal-local.
-        if (xbytes > 1.2 * usable && st->far_fraction > 0.25) {
+        if (xbytes > 1.2 * usable && far_fraction > 0.25) {
             const long long k = (long long)ceil(xbytes / (0.75 * usable));
-            if (k <= kMaxBands && (double)st->nnz / ((double)k * st->m) >= 4.0) bands = k;
-            else if (opt("seg_bands") == 0) {
+            if (k <= kMaxBands && (double)nnz / ((double)k * m) >= 4.0) K = (int)k;
+            else if (o.seg_bands == 0) {
                 // hyper-sparse bands (< 4 entries per virtual row) would cost more in row pointers than they save:
                 // band segments (band_seg.cuh).  More bands = a smaller slice of x = fewer L2 misses of the gathers,
                 // but more and shorter segments for the merge pass.  Measured on the C5 shard (x = 2 GiB, 16 per
                 // row; scripts/c5_sweep.sh): 32 bands 5.24 ms, 40: 4.94, 44: 4.88, 48: 4.78, 52: 4.92, 56: 4.96,
                 // 64: 5.19 -- a slice of about 2/3 of the reach
                 const long long kc = (long long)ceil(xbytes / (0.68 * usable));
-                st->seg.bands = (int)(kc < 2 ? 2 : (kc > kSegMaxBands ? kSegMaxBands : kc));
+                seg = (int)(kc < 2 ? 2 : (kc > kSegMaxBands ? kSegMaxBands : kc));
             }
         }
     }
-    if (opt("seg_bands") >= 2) { st->seg.bands = (int)(opt("seg_bands") > kSegMaxBands ? kSegMaxBands : opt("seg_bands")); bands = 1; }
-    if (bands <= 1) return true;
-    if (bands > kMaxBands) bands = kMaxBands;
-    if ((long long)st->m * bands > 0x7fffffffLL - 8192) return true;
-    const int K = (int)bands, m = st->m;
+    if (m * K > 0x7fffffffLL - 8192) K = 1;  // the m·K virtual rows must stay 32-bit
+    return {K, seg};
+}
+
+// Build the band-major copy of K > 1 column bands and make it the active view.
+template <typename T>
+static void build_band_major(DeviceState *st, int K)
+{
+    const int m = st->m;
     const int band_cols = cols_per_band(st, K);
     const size_t vm = (size_t)m * K;
     DeviceArray<int> counts;
@@ -328,7 +367,6 @@ static bool build_band_major(DeviceState *st)
     auto give_up = [&]() {
         abandon(st->v);
         st->layout_fallbacks++;
-        return true;
     };
     if (!counts.alloc(vm + 1) || !st->v.rowptr.alloc(vm + 1 + 8) || !st->v.col.alloc((size_t)st->nnz + 8) ||
         !st->v.val.alloc((size_t)st->nnz + 8, sizeof(T)) || !st->v.y.alloc(vm, sizeof(T)))
@@ -351,7 +389,6 @@ static bool build_band_major(DeviceState *st)
     st->x_bands = K;
     st->band_cols = band_cols;
     st->a_m = (int)vm; st->a_rowptr = st->v.rowptr; st->a_col = st->v.col; st->a_val = st->v.val.get();
-    return true;
 }
 
 // a9 on the device for `parts` partitions; *starved = some partition owns no whole row (a10)
@@ -434,7 +471,7 @@ static bool build_long_rows_at(DeviceState *st, int thr)
 
 static bool build_long_rows_threshold(DeviceState *st)
 {
-    long long thr = opt("long_thr");  // 0 = automatic, < 0 = off
+    long long thr = st->opts.long_thr;  // 0 = automatic, < 0 = off
     if (thr < 0) { st->lr.thr = 0x7fffffff; return true; }
     const bool automatic = thr == 0;
     if (automatic) { thr = 256LL * st->tpr; if (thr < 512) thr = 512; if (thr > 4096) thr = 4096; }
@@ -443,7 +480,7 @@ static bool build_long_rows_threshold(DeviceState *st)
     // waiting for the longest row of their warp.  Bin the rows by length class instead -- stable radix sort of the
     // row ids by bin -- and give every bin its own launch; rows beyond 128 entries go to the long-row path.
     // (C3: 1.26 ms with one lane-group size, 1.20 ms re-split at 128 entries, see DESIGN.md for the binned figure)
-    if (automatic && st->lr.rows > 0 && st->tpr <= 4 && opt("tpr") == 0 && opt("row_bins") != 0) {
+    if (automatic && st->lr.rows > 0 && st->tpr <= 4 && st->opts.row_bins) {
         st->lr = {};
         if (!build_long_rows_at(st, 128)) return false;
         const int m = st->a_m;
@@ -476,7 +513,7 @@ static bool build_long_rows_threshold(DeviceState *st)
 static bool build_pipeline(DeviceState *st)
 {
     st->pipeline = false;
-    if (opt("pipeline") == 0 || st->lr.rows > 0 || st->m < (1 << 16)) return true;
+    if (!st->opts.pipeline || st->lr.rows > 0 || st->m < (1 << 16)) return true;
     if (st->x_bands > 1) { st->pipeline = st->x_bands <= kMaxPieces; return true; }
     DeviceArray<int> d;
     if (!d.alloc(kPipeChunks)) return false;
@@ -489,9 +526,7 @@ static bool build_pipeline(DeviceState *st)
 
 static bool build_tiles(DeviceState *st, bool merge)
 {
-    int ipt = (int)opt("tile_items");
-    if (ipt != 4 && ipt != 8) ipt = 8;
-    st->tile.items = ipt;
+    const int ipt = st->tile.items = st->opts.tile_items;
     const long long per_tile = (long long)kThreads * ipt;
     const long long total = merge ? (long long)st->a_m + st->nnz : (long long)st->nnz;
     st->tile.count = (int)((total + per_tile - 1) / per_tile);
@@ -514,24 +549,18 @@ static bool build_tiles(DeviceState *st, bool merge)
 template <typename T>
 static bool build_sell(DeviceState *st)
 {
-    long long sigma = opt("sell_sigma");
-    if (sigma < kSellC) sigma = kSellC;
-    if (sigma > kSellMaxSigma) sigma = kSellMaxSigma;
-    sigma = (sigma / kSellC) * kSellC;
-    st->sell.sigma = (int)sigma;
+    st->sell.sigma = st->opts.sell_sigma;
     const int windows = st->a_m / st->sell.sigma;
     st->sell.banner = windows * st->sell.sigma;  // reference sell_C_Sigma_spmv.c:148-156
     st->sell.slices = st->sell.banner / kSellC;
-    st->tpr = pick_tpr(st->nnz, st->a_m);  // for the CSR tail rows [banner, m)
+    st->tpr = pick_tpr(st);  // for the CSR tail rows [banner, m)
     st->kernel = SPMV_B200_KERNEL_SELL;
     // HBM-bound (diagonal-local) matrices want every warp slot filled: 4 columns per step in 32 registers
     // (C4: 0.86 -> 0.98 of the measured peak); gather-bound ones run best with 8 columns per step (C2: 0.43 vs 0.39)
-    st->sell.variant = (int)opt("sell_variant");
-    if (st->sell.variant != 0 && st->sell.variant != 2) st->sell.variant = (st->far_fraction > 0.25) ? 0 : 2;
+    st->sell.variant = st->opts.sell_variant >= 0 ? st->opts.sell_variant : st->far_fraction > 0.25 ? 0 : 2;
     // covered[r]: entries of row r stored in its slice (sell_width_kernel); tail rows [banner, m) stay CSR,
     // except hub rows, which csr_tail_kernel zeroes and the long-row path then adds as a whole
-    long long cap_opt = opt("sell_cap");  // 0 = off (the reference's widths), else the widest slice allowed
-    const int cap = cap_opt <= 0 ? 0 : (int)(cap_opt < 32 ? 32 : (cap_opt > (1 << 20) ? (1 << 20) : cap_opt));
+    const int cap = st->opts.sell_cap;
     DeviceArray<int> covered;
     if (cap) {
         if (!covered.alloc((size_t)st->a_m + 1)) return false;
@@ -573,9 +602,8 @@ static bool build_sell(DeviceState *st)
 template <typename T>
 static bool build_csr5(DeviceState *st)
 {
-    int sigma = (int)opt("csr5_sigma");  // 0 = automatic: 16, or 8 on small matrices (twice the tiles to fill the GPU)
-    if (sigma != 4 && sigma != 8 && sigma != 16) sigma = st->nnz < (1 << 25) ? 8 : 16;
-    st->c5.sigma = sigma;
+    // 0 = automatic: 16, or 8 on small matrices (twice the tiles to fill the GPU)
+    const int sigma = st->c5.sigma = st->opts.csr5_sigma ? st->opts.csr5_sigma : st->nnz < (1 << 25) ? 8 : 16;
     // anonymouslib_avx2.h:124-146 at omega = 32
     int base = 2, by = 1;
     while (base < kC5Omega * sigma) { base *= 2; by++; }
@@ -756,7 +784,7 @@ static bool build_method(DeviceState *st, spmv_Handle *h, int method)
         st->kernel = SPMV_B200_KERNEL_CSR_REFORDER;
         return true;
     case Method_Parallel:
-        st->tpr = pick_tpr(st->nnz, st->a_m);
+        st->tpr = pick_tpr(st);
         st->kernel = SPMV_B200_KERNEL_CSR_VECTOR;
         if (!build_long_rows_threshold(st)) {  // bins / long-row list are speed-ups: plain CSR-vector still works
             abandon(st->lr);
@@ -768,8 +796,7 @@ static bool build_method(DeviceState *st, spmv_Handle *h, int method)
     case Method_Balanced2: {
         if (!apply_reference_balance_rule(st, h)) return false;
         // the GPU geometry: row blocks of ~block_nnz non-zeros, one warp each
-        long long block_nnz = opt("block_nnz");
-        if (block_nnz < 32) block_nnz = 32;
+        const long long block_nnz = st->opts.block_nnz;
         st->split.parts = (int)(((long long)st->nnz + block_nnz - 1) / block_nnz);
         if (st->split.parts < 1) st->split.parts = 1;
         int starved = 0;
@@ -778,7 +805,7 @@ static bool build_method(DeviceState *st, spmv_Handle *h, int method)
         // starved block (some row spans more than a block) => merge-path; otherwise both methods run the
         // row-block kernel ("Balanced2 demoted to Balanced").  Option force_merge=1 keeps merge-path for
         // every Method_Balanced2 handle.
-        if (starved || (method == Method_Balanced2 && opt("force_merge") != 0)) return build_tiles(st, /*merge=*/true);
+        if (starved || (method == Method_Balanced2 && st->opts.force_merge)) return build_tiles(st, /*merge=*/true);
         st->kernel = SPMV_B200_KERNEL_ROW_BLOCKS;
         return true;
     }
@@ -890,8 +917,12 @@ static bool build_state(DeviceState *st, spmv_Handle *h, int m, int n, int *RowP
     }
 
     st->a_m = st->m; st->a_rowptr = st->rowptr; st->a_col = st->col; st->a_val = st->val;
-    if (method != Method_Serial) {  // Method_Serial keeps the reference's exact summation order: never banded
-        if (!with_precision(st, [&](auto t) { return build_band_major<decltype(t)>(st); })) return false;
+    // Method_Serial keeps the reference's exact summation order: never banded
+    if (method != Method_Serial && m > 0 && st->nnz > 0) {
+        if (!probe_locality(st)) return false;
+        const std::pair<int, int> bands = decide_bands(m, n, st->nnz, st->vsize, st->dev_l2, st->far_fraction, st->opts);
+        st->seg.bands = bands.second;
+        if (bands.first > 1) with_precision(st, [&](auto t) { build_band_major<decltype(t)>(st, bands.first); });
     }
     if (m > 0) {
         int e = 0;
@@ -906,7 +937,7 @@ static bool build_state(DeviceState *st, spmv_Handle *h, int m, int n, int *RowP
         return true;
     }
     st->auto_method = -1;
-    if (opt("auto") != 0 && method != Method_Serial) {
+    if (st->opts.auto_pick && method != Method_Serial) {
         method = st->auto_method = auto_pick_method(st);
         if (st->auto_method == Method_SellCSigma || st->auto_method == Method_CSR5SPMV || st->auto_method == Method_Parallel)
             h->spmvMethod = (SPMV_METHODS)st->auto_method;  // what actually runs, for clients that read the field
@@ -1302,13 +1333,14 @@ static void create_into(spmv_Handle *h, BASIC_INT_TYPE m, BASIC_INT_TYPE n, BASI
     // deviation, include/spmv.h)
     DeviceState *st = new DeviceState();
     h->extraHandle = st;
-    st->refresh = opt("refresh") != 0;
+    st->opts = read_create_options();
+    st->refresh = st->opts.refresh;
     // Option "reorder": the reference's level-3 hook (common.c:144-156, compiled out upstream).  Same condition as
     // there (square, > 8096 rows, > 100000 non-zeros), HOST arrays only; the device layout is then built from
     // A' = P A P^T and the permutation is handed to the caller in handle->index (reorder.cu).
     std::vector<int> p_rowptr, p_col;
     std::vector<double> p_val;  // (storage only: 8-byte aligned, holds fp32 or fp64 values)
-    if (opt("reorder") != 0 && m == n && m > 8096 && RowPtr && ColIdx && Matrix_Val && !is_device_ptr(RowPtr) &&
+    if (st->opts.reorder && m == n && m > 8096 && RowPtr && ColIdx && Matrix_Val && !is_device_ptr(RowPtr) &&
         RowPtr[0] == 0 && RowPtr[m] > 100000) {
         const size_t nnz = (size_t)RowPtr[m];
         int *index = (int *)malloc(((size_t)m + 1) * sizeof(int));
@@ -1363,7 +1395,7 @@ void spmv(const spmv_Handle_t handle, BASIC_INT_TYPE m, const BASIC_INT_TYPE *Ro
     const void *xd = Vector_Val_X;
     void *yd = Vector_Val_Y;
     const size_t xb = (size_t)st->n * st->vsize, yb = (size_t)st->m * st->vsize;
-    if (st->pin_host) {
+    if (st->opts.pin_host) {
         if (!x_dev && xb) note_host_buffer(st, 0, Vector_Val_X, xb);
         if (!y_dev && yb) note_host_buffer(st, 1, Vector_Val_Y, yb);
     }
