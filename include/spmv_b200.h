@@ -56,6 +56,30 @@ SPMV_B200_API int spmv_b200_update_values(spmv_Handle_t handle, void *Matrix_Val
  * Refresh kernels are not counted by spmv_b200_launch_count(). */
 SPMV_B200_API int spmv_b200_set_values(spmv_Handle_t handle, const void *Matrix_Val);
 
+/* ---- scaled products ----------------------------------------------------------------------------------
+ * y <- alpha * A x + beta * y, the update of a CG residual, a Jacobi or Chebyshev step, PageRank or a Lanczos step,
+ * and what MKL's mkl_sparse_?_mv and cuSPARSE's cusparseSpMV compute.  With s = the y that spmv() on this handle writes
+ * for this x, bit for bit, every row gets y[i] = fl(fl(alpha s[i]) + fl(beta y_old[i])): three roundings, no FMA, so
+ * the result is reproducible on a CPU.  beta == 0: y[i] = fl(alpha s[i]) and the old y is never read (it may hold
+ * anything, NaN included); alpha == 0: y[i] = fl(beta y_old[i]) and A and x are not read; both 0: every row +0.0.  So
+ * alpha = 1, beta = 0 is exactly spmv().  fp32 handles round alpha and beta to float first.  nnz == 0 follows the rule
+ * with s = +0; m == 0 does nothing.
+ * x and y may be HOST or DEVICE pointers as in spmv() (option "pin_host" applies; the pipelined host path does not):
+ * with device x and y the call is enqueued on the handle's stream, with a host y it is synchronous (and with beta != 0
+ * the old y is uploaded first).  y peers (spmv_b200_set_y_peers) receive the scaled values.  x and y must not overlap.
+ * The scaling is done by the kernel that stores each final y value -- the fold of the column bands, or the main kernel
+ * of an unbanded CSR-vector, row-block or 8-column SELL handle -- at the cost of one read of the old y when beta != 0;
+ * the other layouts (carry fix-ups, long-row list, row bins, SELL's 4-column flavour "sell_variant" 2, Method_Serial,
+ * nnz == 0) write A x into a scratch array of m values, allocated at the first such call and owned by the handle, and
+ * scale it in one more pass.
+ * spmv_b200_info(h, "axpby_path") says which: 0 = scratch pass, 1 = main kernel, 2 = fold (option "axpby_fused" = 0
+ * at create: always 0).  With device pointers the call can be captured in a CUDA graph after one call outside the
+ * capture (which may allocate the scratch array).
+ * Returns 0, or -1 (spmv_b200_last_error()): NULL handle, failed create, NULL y, NULL x with n > 0, or x == y (all
+ * with y untouched), or a failed allocation or launch (a failed scratch allocation also leaves y untouched; the
+ * handle keeps working). */
+SPMV_B200_API int spmv_b200_spmv_axpby(spmv_Handle_t handle, double alpha, const void *x, double beta, void *y);
+
 /* ---- streams -----------------------------------------------------------------------------------
  * spmv() with HOST x/y is synchronous (reference semantics).  With DEVICE x/y it is enqueued on the
  * handle's stream (default: the legacy default stream 0) and returns immediately. */
@@ -108,6 +132,9 @@ SPMV_B200_API void spmv_b200_sync(spmv_Handle_t handle);
  *   "refresh"         1 = create also keeps a source map of every value array the handle stores, so that
  *                     spmv_b200_set_values can refresh the values in place (4 bytes per stored slot); 0 (default) = no
  *                     maps, create is unchanged
+ *   "axpby_fused"     1 (default) = spmv_b200_spmv_axpby scales in the kernel that stores each final y value where the
+ *                     layout has such a kernel; 0 = always A x into the scratch array, then one scaling pass (the same
+ *                     bits; for timing one against the other)
  * Returns 0, or -1 for an unknown key. */
 SPMV_B200_API int spmv_b200_set_option(const char *key, long long value);
 SPMV_B200_API long long spmv_b200_get_option(const char *key);
@@ -119,7 +146,8 @@ SPMV_B200_API long long spmv_b200_get_option(const char *key);
  * "csr5_num_offsets", "csr5_tail_start", "device", "has_empty_rows", "x_bands", "seg_bands", "segments", "seg_cross",
  * "seg_ctas" (persistent CTAs per SM of the band-segment pass 1; 0 until the handle's first launch), "band_cols",
  * "active_rows", "owns_csr", "released_csr",
- * "layout_fallbacks", "auto_method", "values_snapshotted", "refreshable", "pipeline", "dev_l2_bytes".  Returns -1 for an unknown key /
+ * "layout_fallbacks", "auto_method", "values_snapshotted", "refreshable", "pipeline", "dev_l2_bytes", "axpby_path" (where
+ * spmv_b200_spmv_axpby scales: 0 = scratch pass, 1 = main kernel, 2 = fold).  Returns -1 for an unknown key /
  * NULL handle.
  *
  * spmv_b200_structure: copy a device layout array to HOST memory.  Returns its size in bytes (call

@@ -40,7 +40,7 @@ EXPORTED_FUNCTIONS = [
     "spmv_b200_recommend_method", "spmv_b200_bands", "spmv_b200_band_columns", "spmv_b200_spmv_bands",
     "spmv_b200_spmv_finish", "spmv_b200_memcpy_async", "spmv_b200_stream_write32", "spmv_b200_stream_wait32_geq",
     "spmv_b200_reorder", "spmv_b200_permute_csr", "spmv_b200_update_values", "spmv_b200_live_allocations",
-    "spmv_b200_set_values"]
+    "spmv_b200_set_values", "spmv_b200_spmv_axpby"]
 EXPORTED_DATA = ["Methods_names", "Vectorized_names", "funcNames"]
 
 
@@ -116,6 +116,7 @@ def lib() -> C.CDLL:
     L.spmv_b200_spmv_finish.argtypes = [spmv_Handle_t, vp]
     L.spmv_b200_update_values.argtypes = [spmv_Handle_t, vp]
     L.spmv_b200_set_values.argtypes = [spmv_Handle_t, vp]
+    L.spmv_b200_spmv_axpby.argtypes = [spmv_Handle_t, C.c_double, vp, C.c_double, vp]
     L.spmv_b200_reorder.argtypes = [i, vp, vp, vp]
     L.spmv_b200_permute_csr.argtypes = [i, vp, vp, vp, ul, vp, vp, vp, vp]
     L.spmv_b200_memcpy_async.argtypes = [vp, vp, C.c_size_t, vp]
@@ -205,6 +206,12 @@ class Handle:
     def spmv(self, x, y):
         rp, ci, va = self.keep
         spmv(self.h, self.m, rp, ci, va, x, y)
+        return y
+
+    def spmv_axpby(self, alpha, x, beta, y):
+        """y <- alpha A x + beta y in place (spmv_b200_spmv_axpby); host y: complete on return."""
+        if lib().spmv_b200_spmv_axpby(self.h, float(alpha), _addr(x), float(beta), _addr(y)) != 0:
+            raise RuntimeError("spmv_b200_spmv_axpby: " + last_error())
         return y
 
     def info(self, key: str) -> int:

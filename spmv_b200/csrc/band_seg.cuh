@@ -444,7 +444,7 @@ bseg_kernel(int tile_lo, int tile_hi, int pf_on, int *__restrict__ next_tile, co
 // (A ballot-free variant -- a rank byte per segment, every lane walking its own set bits -- was measured: 40 % fewer
 // instructions but 1.8x the DRAM traffic, because lanes then read different bands in the same instruction.)
 // ------------------------------------------------------------------------------------------------
-template <typename T, bool PEERS>
+template <typename T>
 __device__ __forceinline__ void merge_half(unsigned mk, int base, unsigned lt, const T *__restrict__ seg_val, T &sum)
 {
     // fully unrolled over 32 mask bits in batches of 8 loads; bits of bands that do not exist are never set
@@ -465,25 +465,44 @@ __device__ __forceinline__ void merge_half(unsigned mk, int base, unsigned lt, c
     }
 }
 
-template <typename T, typename MaskT, bool PEERS>
-__global__ void __launch_bounds__(kThreads)
-bseg_merge_kernel(int row0, int m, int bands, const MaskT *__restrict__ mask, const int *__restrict__ gbase,
-                  const T *__restrict__ seg_val, T *__restrict__ y, const PeerList<T> peers)
+template <typename T, typename MaskT, typename Store>
+__device__ __forceinline__ void bseg_merge_body(unsigned tid, int row0, int m, int bands,
+                                                const MaskT *__restrict__ mask, const int *__restrict__ gbase,
+                                                const T *__restrict__ seg_val, const Store &store)
 {
-    const int lane = threadIdx.x & 31;
-    const long long g = row0 / 32 + (((long long)blockIdx.x * kThreads + threadIdx.x) >> 5);  // row0: a multiple of 32
+    const int lane = tid & 31;
+    const long long g = row0 / 32 + (((long long)blockIdx.x * kThreads + tid) >> 5);  // row0: a multiple of 32
     const long long r = g * 32 + lane;
     if (g * 32 >= m) return;
     const MaskT mk = r < m ? __ldcs(mask + r) : (MaskT)0;
     const int base_lo = lane < bands ? __ldcs(gbase + (size_t)g * bands + lane) : 0;
     const unsigned lt = (1u << lane) - 1u;
     T sum = 0;
-    merge_half<T, PEERS>((unsigned)mk, base_lo, lt, seg_val, sum);
+    merge_half<T>((unsigned)mk, base_lo, lt, seg_val, sum);
     if (sizeof(MaskT) == 8) {
         const int base_hi = lane + 32 < bands ? __ldcs(gbase + (size_t)g * bands + 32 + lane) : 0;
-        merge_half<T, PEERS>((unsigned)((unsigned long long)mk >> 32), base_hi, lt, seg_val, sum);
+        merge_half<T>((unsigned)((unsigned long long)mk >> 32), base_hi, lt, seg_val, sum);
     }
-    if (r < m) store_y<PEERS>(y, peers, r, sum);
+    // the old y is loaded after the merge, not before it: held across the merge it costs the fp64 / 64-band kernel 8
+    // registers (40 instead of 32) and a quarter of its warps, for every beta
+    if (r < m) store.put(r, sum, store.early(true, r));
+}
+
+template <typename T, typename MaskT, bool PEERS>
+__global__ void __launch_bounds__(kThreads)
+bseg_merge_kernel(int row0, int m, int bands, const MaskT *__restrict__ mask, const int *__restrict__ gbase,
+                  const T *__restrict__ seg_val, T *__restrict__ y, const PeerList<T> peers)
+{
+    bseg_merge_body<T>(threadIdx.x, row0, m, bands, mask, gbase, seg_val, PeerStore<PEERS, T>{y, peers});
+}
+
+// spmv_b200_spmv_axpby on a band-segment handle: pass 2, scaled
+template <typename T, typename MaskT>
+__global__ void __launch_bounds__(kThreads)
+bseg_merge_axpby_kernel(int row0, int m, int bands, const MaskT *__restrict__ mask, const int *__restrict__ gbase,
+                        const T *__restrict__ seg_val, const ScaledStore<T> store)
+{
+    bseg_merge_body<T>(threadIdx.x, row0, m, bands, mask, gbase, seg_val, store);
 }
 
 }  // namespace sb

@@ -110,6 +110,7 @@ struct CreateOptions {
     int x_bands;            // 0 = automatic, 1 = off, 2 .. kMaxBands forced
     int seg_bands;          // 0 = automatic, -1 = never, 2 .. kSegMaxBands forced (overrides x_bands)
     bool force_merge, pipeline, auto_pick, reorder, pin_host, refresh;
+    bool axpby_fused;       // false: spmv_b200_spmv_axpby takes the scratch pass on every layout
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -158,7 +159,9 @@ struct DeviceState {
     PinSlot pin[2];
     // staging for host-side x / y; the pipelined host path (CSR-vector kernel) copies x in pieces on s_in,
     // computes row chunks as soon as their prefix of x has arrived, and returns finished chunks of y on s_out
-    struct Staging { DeviceBytes x, y, val; } stage;  // val: host values of spmv_b200_set_values, when no upload takes them
+    // val: host values of spmv_b200_set_values, when no upload takes them; s: A x of spmv_b200_spmv_axpby on the handles
+    // whose last store has no scaled kernel (its scratch pass), allocated at the first such call
+    struct Staging { DeviceBytes x, y, val, s; } stage;
     bool pipeline = false;
     cudaStream_t s_in = nullptr, s_out = nullptr;
     cudaEvent_t ev_in[kMaxPieces] = {}, ev_out[kPipeChunks] = {}, ev_start = nullptr, ev_x = nullptr;
@@ -366,6 +369,41 @@ __device__ __forceinline__ void store_y(T *y, const PeerList<T> &peers, long lon
             if (i < peers.n) stg_y(peers.p[i] + row, v);
     }
 }
+
+// ---- the final store of a row value v = (A x)[row]: a template parameter of every kernel body that writes final y
+// values.  PeerStore is spmv()'s (y = v, and the peer copies); ScaledStore is spmv_b200_spmv_axpby's (y <- alpha v +
+// beta y).  early(pred, row) reads what put needs; most bodies call it before the row walk, so that a load of the old y
+// is in flight while the row is summed.  put(row, v, early) writes.  The kernels read threadIdx.x themselves and hand it to the body (`tid`): only a
+// read in the __global__ function carries the range __launch_bounds__ gives it, so the spmv() kernels keep their code.
+struct NoEarly {};
+template <bool PEERS, typename T>
+struct PeerStore {
+    T *y;
+    const PeerList<T> &peers;
+    __device__ __forceinline__ NoEarly early(bool, long long) const { return {}; }
+    __device__ __forceinline__ void put(long long row, T v, NoEarly) const { store_y<PEERS>(y, peers, row, v); }
+};
+
+// round-to-nearest products and sums that nvcc never contracts into an FMA
+__device__ __forceinline__ double mul_rn(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ float mul_rn(float a, float b) { return __fmul_rn(a, b); }
+__device__ __forceinline__ double add_rn(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ float add_rn(float a, float b) { return __fadd_rn(a, b); }
+
+// y[row] = fl(fl(alpha v) + fl(beta y_old)), three roundings and no FMA (what numpy computes from spmv()'s bits); beta ==
+// 0: fl(alpha v), and the old y is never read, so whatever it holds does not propagate.  (alpha == 0 never reaches a
+// kernel that computes v: the host then writes fl(beta y_old), or +0, without reading A or x.)
+template <typename T>
+struct ScaledStore {
+    T *y;
+    T alpha, beta;
+    __device__ __forceinline__ T early(bool pred, long long row) const { return pred && beta != (T)0 ? __ldcs(y + row) : (T)0; }
+    __device__ __forceinline__ void put(long long row, T v, T y_old) const
+    {
+        const T av = mul_rn(alpha, v);
+        stg_y(y + row, beta != (T)0 ? add_rn(av, mul_rn(beta, y_old)) : av);
+    }
+};
 
 __device__ __forceinline__ double fma_t(double a, double b, double c) { return fma(a, b, c); }
 __device__ __forceinline__ float fma_t(float a, float b, float c) { return fmaf(a, b, c); }

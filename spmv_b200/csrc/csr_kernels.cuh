@@ -116,11 +116,11 @@ __device__ __forceinline__ T row_partial(int start, int end, int sl, int tpr, co
 // the OpenMP row loop becomes a grid of sub-warps, TPR lanes per row with TPR = 2^k ~ mean row
 // length / 4 chosen at create.  Fixed butterfly reduction => bitwise reproducible.
 // ------------------------------------------------------------------------------------------------
-template <typename T, int TPR, bool PEERS, bool FUSE>
-__global__ void __launch_bounds__(kThreads)
-csr_vector_kernel(int row0, int m, int long_thr, const int *__restrict__ rowptr, const int *__restrict__ col,
-                  const T *__restrict__ val, const T *__restrict__ x, T *__restrict__ y, const PeerList<T> peers,
-                  int fuse_bands, int band_m, const T *__restrict__ vy)
+template <typename T, int TPR, bool FUSE, typename Store>
+__device__ __forceinline__ void csr_vector_body(unsigned tid, int row0, int m, int long_thr,
+                                                const int *__restrict__ rowptr, const int *__restrict__ col,
+                                                const T *__restrict__ val, const T *__restrict__ x, const Store &store,
+                                                int fuse_bands, int band_m, const T *__restrict__ vy)
 {
     // rows [row0, m): the whole matrix in one launch, or one band / row chunk of the pipelined host path.
     // FUSE (pipelined host path only; a separate instantiation so that the plain kernel keeps its 40 registers):
@@ -128,9 +128,9 @@ csr_vector_kernel(int row0, int m, int long_thr, const int *__restrict__ rowptr,
     // (vy, complete: written by an earlier launch) are folded in here, in band order, and the final value goes
     // to row (virtual row - fuse_bands*band_m) of y -- band_reduce_kernel without its own pass.
     const uint64_t pl = policy_evict_last(), pf = policy_evict_first();
-    const long long gt = (long long)blockIdx.x * kThreads + threadIdx.x;
+    const long long gt = (long long)blockIdx.x * kThreads + tid;
     const long long row_l = row0 + gt / TPR;
-    const int sl = threadIdx.x & (TPR - 1);
+    const int sl = tid & (TPR - 1);
     bool valid = row_l < m;
     const int row = valid ? (int)row_l : 0;
     int start = valid ? rowptr[row] : 0;
@@ -145,9 +145,31 @@ csr_vector_kernel(int row0, int m, int long_thr, const int *__restrict__ rowptr,
             for (int b = 1; b < fuse_bands; ++b) prev += ldg_stream(vy + (size_t)b * band_m + out_row);
         }
     }
+    const auto early = store.early(valid && sl == 0, out_row);
     T sum = row_partial<T>(start, end, sl, TPR, col, val, x, pl, pf);
     sum = group_sum_c<T, TPR>(sum);
-    if (valid && sl == 0) store_y<PEERS>(y, peers, out_row, FUSE ? prev + sum : sum);
+    if (valid && sl == 0) store.put(out_row, FUSE ? prev + sum : sum, early);
+}
+
+template <typename T, int TPR, bool PEERS, bool FUSE>
+__global__ void __launch_bounds__(kThreads)
+csr_vector_kernel(int row0, int m, int long_thr, const int *__restrict__ rowptr, const int *__restrict__ col,
+                  const T *__restrict__ val, const T *__restrict__ x, T *__restrict__ y, const PeerList<T> peers,
+                  int fuse_bands, int band_m, const T *__restrict__ vy)
+{
+    csr_vector_body<T, TPR, FUSE>(threadIdx.x, row0, m, long_thr, rowptr, col, val, x, PeerStore<PEERS, T>{y, peers},
+                                  fuse_bands, band_m, vy);
+}
+
+// spmv_b200_spmv_axpby on an unbanded Method_Parallel handle with one lane per row, without row bins or long-row list:
+// y <- alpha A x + beta y (instantiated for TPR = 1 only, see axpby_path)
+template <typename T, int TPR>
+__global__ void __launch_bounds__(kThreads)
+csr_vector_axpby_kernel(int row0, int m, int long_thr, const int *__restrict__ rowptr, const int *__restrict__ col,
+                        const T *__restrict__ val, const T *__restrict__ x, const ScaledStore<T> store)
+{
+    csr_vector_body<T, TPR, false>(threadIdx.x, row0, m, long_thr, rowptr, col, val, x, store, 0, 0,
+                                   (const T *)nullptr);
 }
 
 // The same row walk over a LIST of rows: Method_Parallel on matrices whose rows are short but not uniformly so
@@ -346,15 +368,31 @@ __global__ void band_scatter_kernel(int m, int bands, int band_cols, const int *
     }
 }
 
+template <typename T, typename Store>
+__device__ __forceinline__ void band_reduce_body(int row0, int row1, int m, int bands, const T *__restrict__ yv,
+                                                 const Store &store)
+{
+    const int r = row0 + blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= row1) return;
+    const auto early = store.early(true, r);
+    T s = ldg_stream(yv + r);
+    for (int b = 1; b < bands; ++b) s += ldg_stream(yv + (size_t)b * m + r);
+    store.put(r, s, early);
+}
+
 template <typename T, bool PEERS>
 __global__ void band_reduce_kernel(int row0, int row1, int m, int bands, const T *__restrict__ yv, T *__restrict__ y,
                                    const PeerList<T> peers)
 {
-    const int r = row0 + blockIdx.x * blockDim.x + threadIdx.x;
-    if (r >= row1) return;
-    T s = ldg_stream(yv + r);
-    for (int b = 1; b < bands; ++b) s += ldg_stream(yv + (size_t)b * m + r);
-    store_y<PEERS>(y, peers, r, s);
+    band_reduce_body<T>(row0, row1, m, bands, yv, PeerStore<PEERS, T>{y, peers});
+}
+
+// spmv_b200_spmv_axpby on a band-major handle: the fold of the band partials, scaled
+template <typename T>
+__global__ void band_reduce_axpby_kernel(int row0, int row1, int m, int bands, const T *__restrict__ yv,
+                                         const ScaledStore<T> store)
+{
+    band_reduce_body<T>(row0, row1, m, bands, yv, store);
 }
 
 // Largest column index used by each of `chunks` equal row chunks (+1): the prefix of x a chunk needs.  Lets the
@@ -389,6 +427,18 @@ __global__ void peer_copy_kernel(long long m, const T *__restrict__ y, const Pee
 #pragma unroll
     for (int i = 0; i < kMaxPeers; ++i)
         if (i < peers.n) stg_y(peers.p[i] + r, v);
+}
+
+// spmv_b200_spmv_axpby on the handles whose last store is not a scaled kernel's: s = A x as spmv() writes it (into a
+// scratch array of the handle), y <- alpha s + beta y.  s = NULL is alpha == 0: y = fl(beta y_old).
+template <typename T>
+__global__ void axpby_kernel(long long m, const T *__restrict__ s, const ScaledStore<T> store)
+{
+    const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= m) return;
+    const T y_old = store.early(true, r);
+    if (s) store.put(r, ldg_stream(s + r), y_old);
+    else stg_y(store.y + r, mul_rn(store.beta, y_old));
 }
 
 }  // namespace sb

@@ -141,20 +141,21 @@ __global__ void sell_fill_kernel(int slices, const int *__restrict__ rowptr, con
 // C2 0.43 vs 0.39) and U = 4 / 8 CTAs, every warp slot of the SM filled (HBM-bound ones: C4 0.86 -> 0.98).
 // (Software-pipelined variants -- the next step's stream loads issued before this step's gathers -- measured no
 // better and were dropped.)
-template <typename T, bool PEERS, int U, int MINB>
-__global__ void __launch_bounds__(kThreads, MINB)
-sell_kernel(int slices, const long long *__restrict__ slice_ptr, const int *__restrict__ full,
-            const int *__restrict__ perm, const int *__restrict__ scol, const T *__restrict__ sval,
-            const T *__restrict__ x, T *__restrict__ y, const PeerList<T> peers)
+template <typename T, int U, typename Store>
+__device__ __forceinline__ void sell_body(unsigned tid, int slices, const long long *__restrict__ slice_ptr,
+                                          const int *__restrict__ full, const int *__restrict__ perm,
+                                          const int *__restrict__ scol, const T *__restrict__ sval,
+                                          const T *__restrict__ x, const Store &store)
 {
     const uint64_t pl = policy_evict_last(), pf = policy_evict_first();
-    const int s = (int)(((long long)blockIdx.x * kThreads + threadIdx.x) >> 5);
-    const int lane = threadIdx.x & 31;
+    const int s = (int)(((long long)blockIdx.x * kThreads + tid) >> 5);
+    const int lane = tid & 31;
     if (s >= slices) return;
     const long long base = slice_ptr[s];
     const int w = (int)((slice_ptr[s + 1] - base) >> 5);
     const int f = full[s];
     const int out_row = perm[(long long)s * kSellC + lane];
+    const auto early = store.early(true, out_row);
     const int *c = scol + base + lane;
     const T *v = sval + base + lane;
     // blocked summation (U columns -> 512 columns -> row) keeps the rounding error of a long row at
@@ -195,7 +196,26 @@ sell_kernel(int slices, const long long *__restrict__ slice_ptr, const int *__re
         if (++groups >= kGroups) { sum += mid; mid = 0; groups = 0; }
     }
     sum += mid;
-    store_y<PEERS>(y, peers, out_row, sum);
+    store.put(out_row, sum, early);
+}
+
+template <typename T, bool PEERS, int U, int MINB>
+__global__ void __launch_bounds__(kThreads, MINB)
+sell_kernel(int slices, const long long *__restrict__ slice_ptr, const int *__restrict__ full,
+            const int *__restrict__ perm, const int *__restrict__ scol, const T *__restrict__ sval,
+            const T *__restrict__ x, T *__restrict__ y, const PeerList<T> peers)
+{
+    sell_body<T, U>(threadIdx.x, slices, slice_ptr, full, perm, scol, sval, x, PeerStore<PEERS, T>{y, peers});
+}
+
+// spmv_b200_spmv_axpby on an unbanded SELL handle without long-row list (the CSR tail: csr_tail_axpby_kernel)
+template <typename T, int U, int MINB>
+__global__ void __launch_bounds__(kThreads, MINB)
+sell_axpby_kernel(int slices, const long long *__restrict__ slice_ptr, const int *__restrict__ full,
+                  const int *__restrict__ perm, const int *__restrict__ scol, const T *__restrict__ sval,
+                  const T *__restrict__ x, const ScaledStore<T> store)
+{
+    sell_body<T, U>(threadIdx.x, slices, slice_ptr, full, perm, scol, sval, x, store);
 }
 
 }  // namespace sb

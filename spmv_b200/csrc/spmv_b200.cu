@@ -62,7 +62,7 @@ struct Options {
                                        {"force_merge", 0}, {"sell_cap", 1024},
                                        {"long_thr", 0},    {"pipeline", 1},   {"sell_variant", -1},
                                        {"seg_bands", 0},    {"seg_prefetch", 1}, {"seg_ctas", 2},  {"auto", 0},     {"reorder", 0},    {"row_bins", 1},
-                                       {"pin_host", 1},     {"refresh", 0}};
+                                       {"pin_host", 1},     {"refresh", 0},    {"axpby_fused", 1}};
     std::map<std::string, bool> user_set;
 };
 static Options &options()
@@ -112,6 +112,7 @@ static CreateOptions read_create_options()
     o.reorder = opt("reorder") != 0;
     o.pin_host = opt("pin_host") != 0;
     o.refresh = opt("refresh") != 0;
+    o.axpby_fused = opt("axpby_fused") != 0;
     return o;
 }
 
@@ -990,35 +991,65 @@ static void launch_vector(DeviceState *st, int row0, int row1, const T *x, T *y,
     count_launch();
 }
 
-// y_out = the band partials of the virtual y (v.y) added in band order, copied to the peers too
+// y_out = the band partials of the virtual y (v.y) added in band order, copied to the peers too; scaled: y_out <- alpha
+// (that sum) + beta y_out instead, and no peers
 template <typename T>
-static bool launch_band_fold(DeviceState *st, T *y_out)
+static bool launch_band_fold(DeviceState *st, T *y_out, const ScaledStore<T> *scaled = nullptr)
 {
-    const PeerList<T> peers = peers_of<T>(st);
-    const auto kernel = peers.n > 0 ? band_reduce_kernel<T, true> : band_reduce_kernel<T, false>;
-    kernel<<<blocks_for(st->m), kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), y_out, peers);
+    if (scaled) {
+        band_reduce_axpby_kernel<T><<<blocks_for(st->m), kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), *scaled);
+    } else {
+        const PeerList<T> peers = peers_of<T>(st);
+        const auto kernel = peers.n > 0 ? band_reduce_kernel<T, true> : band_reduce_kernel<T, false>;
+        kernel<<<blocks_for(st->m), kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), y_out, peers);
+    }
     count_launch();
     return SB_CUDA(cudaGetLastError());
 }
 
 // CSR-vector over rows [row0, m) only (the CSR tail of SELL)
-template <typename T>
-__global__ void __launch_bounds__(kThreads)
-csr_tail_kernel(int row0, int m, int long_thr, const int *__restrict__ rowptr, const int *__restrict__ col,
-                const T *__restrict__ val, const T *__restrict__ x, T *__restrict__ y)
+template <typename T, typename Store>
+__device__ __forceinline__ void csr_tail_body(unsigned tid, int row0, int m, int long_thr, const int *__restrict__ rowptr,
+                                              const int *__restrict__ col, const T *__restrict__ val,
+                                              const T *__restrict__ x, const Store &store)
 {
     const uint64_t pl = policy_evict_last();
-    const long long w = ((long long)blockIdx.x * kThreads + threadIdx.x) >> 5;
-    const int lane = threadIdx.x & 31;
+    const long long w = ((long long)blockIdx.x * kThreads + tid) >> 5;
+    const int lane = tid & 31;
     if (row0 + w >= m) return;
     const int row = (int)(row0 + w);
     const int start = rowptr[row];
     int end = rowptr[row + 1];
     if (end - start > long_thr) end = start;  // hub row: y = 0 here, the long-row path adds the whole row
+    const auto early = store.early(lane == 0, row);
     T sum = 0;
     for (int j = start + lane; j < end; j += 32) sum = fma_t(val[j], ldg_x(x + col[j], pl), sum);
     sum = group_sum_c<T, 32>(sum);
-    if (lane == 0) y[row] = sum;
+    if (lane == 0) store.put(row, sum, early);
+}
+
+// csr_tail_kernel's store: a plain one (the tail rows are few; spmv() writes them through L1 as it always has)
+template <typename T>
+struct TailStore {
+    T *y;
+    __device__ __forceinline__ NoEarly early(bool, long long) const { return {}; }
+    __device__ __forceinline__ void put(long long row, T v, NoEarly) const { y[row] = v; }
+};
+
+template <typename T>
+__global__ void __launch_bounds__(kThreads)
+csr_tail_kernel(int row0, int m, int long_thr, const int *__restrict__ rowptr, const int *__restrict__ col,
+                const T *__restrict__ val, const T *__restrict__ x, T *__restrict__ y)
+{
+    csr_tail_body<T>(threadIdx.x, row0, m, long_thr, rowptr, col, val, x, TailStore<T>{y});
+}
+
+template <typename T>
+__global__ void __launch_bounds__(kThreads)
+csr_tail_axpby_kernel(int row0, int m, int long_thr, const int *__restrict__ rowptr, const int *__restrict__ col,
+                      const T *__restrict__ val, const T *__restrict__ x, const ScaledStore<T> store)
+{
+    csr_tail_body<T>(threadIdx.x, row0, m, long_thr, rowptr, col, val, x, store);
 }
 
 static int opt_cached_seg_prefetch()
@@ -1058,25 +1089,33 @@ static bool launch_seg_bands(DeviceState *st, int b0, int count, const T *x)
     return SB_CUDA(cudaGetLastError());
 }
 
-// band segments: carries of segments that cross a tile boundary, then pass 2 (y written once, peers included)
+// band segments: carries of segments that cross a tile boundary, then pass 2 (y written once, peers included; scaled:
+// y_out <- alpha (the row sums) + beta y_out, and no peers)
 template <typename T>
-static bool launch_seg_finish(DeviceState *st, T *y_out)
+static bool launch_seg_finish(DeviceState *st, T *y_out, const ScaledStore<T> *scaled = nullptr)
 {
     cudaStream_t s = st->stream;
     if (st->seg.cross) launch_carry_fixup<T>(st, s, st->tile.count * kSegChunks, st->tile.carry_row, st->tile.carry_val.as<T>(), st->seg.sums.as<T>());
     const PeerList<T> pr = peers_of<T>(st);
     auto merge = [&](auto mask_word) {  // row masks of 32 or 64 bands
         using M = decltype(mask_word);
+        const int grid = blocks_for((long long)st->seg.groups * 32);
+        if (scaled) {
+            bseg_merge_axpby_kernel<T, M><<<grid, kThreads, 0, s>>>(0, st->m, st->seg.bands, st->seg.mask.as<M>(), st->seg.gbase, st->seg.sums.as<T>(), *scaled);
+            return;
+        }
         const auto kernel = pr.n > 0 ? bseg_merge_kernel<T, M, true> : bseg_merge_kernel<T, M, false>;
-        kernel<<<blocks_for((long long)st->seg.groups * 32), kThreads, 0, s>>>(0, st->m, st->seg.bands, st->seg.mask.as<M>(), st->seg.gbase, st->seg.sums.as<T>(), y_out, pr);
+        kernel<<<grid, kThreads, 0, s>>>(0, st->m, st->seg.bands, st->seg.mask.as<M>(), st->seg.gbase, st->seg.sums.as<T>(), y_out, pr);
     };
     if (st->seg.mask64) merge((unsigned long long)0); else merge(uint32_t(0));
     count_launch();
     return SB_CUDA(cudaGetLastError());
 }
 
+// y_out = A x.  fold_scaled (spmv_b200_spmv_axpby on a band-major or band-segment handle): the last pass, the fold of
+// the band partials, writes y_out <- alpha A x + beta y_out instead.
 template <typename T>
-static bool launch(DeviceState *st, const T *x, T *y_out)
+static bool launch(DeviceState *st, const T *x, T *y_out, const ScaledStore<T> *fold_scaled = nullptr)
 {
     cudaStream_t s = st->stream;
     if (st->m == 0) return true;
@@ -1086,7 +1125,7 @@ static bool launch(DeviceState *st, const T *x, T *y_out)
     if (st->kernel == SPMV_B200_KERNEL_BAND_SEG) {
         // pass 1: segment sums of every tile (one launch, tiles in band order); carries of segments that cross a
         // tile boundary; pass 2: every row adds its segment sums in band order and writes y once
-        return launch_seg_bands<T>(st, 0, st->seg.bands, x) && launch_seg_finish<T>(st, y_out);
+        return launch_seg_bands<T>(st, 0, st->seg.bands, x) && launch_seg_finish<T>(st, y_out, fold_scaled);
     }
     // the active view: the CSR itself, or its band-major copy writing the virtual y
     const int m = st->a_m;
@@ -1191,9 +1230,107 @@ static bool launch(DeviceState *st, const T *x, T *y_out)
         final_kernel<<<blocks_for((long long)st->lr.rows * 32), kThreads, 0, s>>>(st->lr.rows, st->lr.accumulate, single, st->lr.row, st->lr.seg_ptr, st->lr.partial.as<T>(), y, fused);
         count_launch(2);
     }
-    if (banded) return launch_band_fold<T>(st, y_out);  // y and the peers
+    if (banded) return launch_band_fold<T>(st, y_out, fold_scaled);  // y and the peers
     if (fused.n > 0 && !wrote_fused) {  // kernels without a fused epilogue: one stream-ordered copy to the peers
         peer_copy_kernel<T><<<blocks_for(st->m), kThreads, 0, s>>>(st->m, y_out, fused);
+        count_launch();
+    }
+    return SB_CUDA(cudaGetLastError());
+}
+
+// ------------------------------------------------------------------------------------------------
+// y <- alpha A x + beta y (spmv_b200_spmv_axpby).  A x is summed by spmv()'s own kernels, bit for bit, and scaled where
+// its final value is stored: in the fold of the band partials (band-major copy, band segments), in the main kernel
+// (CSR-vector, row blocks, SELL and its CSR tail), or -- where the final value comes out of a carry fix-up (merge-path,
+// nnz-split, CSR5), of the long-row pass, of the row bins' several launches, or of the reference-order kernel -- in a
+// pass of its own over A x written to a scratch array.
+// ------------------------------------------------------------------------------------------------
+enum { kAxpbyScratch = 0, kAxpbyMain = 1, kAxpbyFold = 2 };  // spmv_b200_info "axpby_path"
+
+// Whether spmv() runs SELL's 8-column flavour (variant 0, or any variant with peers and no CSR tail).  The step width
+// orders the sums, so a scaled SELL kernel must step as spmv() does.  The 4-column flavour (variant 2) fits 32
+// registers, which is why it exists (every warp slot of the SM filled); its scaled twin does not (fp64: 100 bytes of
+// spills at 32 registers, against sell_kernel's own 76), so variant-2 handles take the scratch pass.
+static bool sell_eight_columns(const DeviceState *st)
+{
+    return st->sell.variant != 2 || (st->n_peers > 0 && st->sell.banner == st->m);
+}
+
+static int axpby_path(const DeviceState *st)
+{
+    if (!st->opts.axpby_fused) return kAxpbyScratch;  // option "axpby_fused" = 0
+    if (st->kernel == SPMV_B200_KERNEL_BAND_SEG) return kAxpbyFold;
+    if (st->x_bands > 1) return kAxpbyFold;  // (never Method_Serial: it is not banded)
+    if (st->lr.rows > 0) return kAxpbyScratch;
+    // one lane per row only: at 2..32 lanes the scaled CSR-vector kernel needs 48 registers against spmv()'s 40 and
+    // lost to the scratch pass on C4 (tpr 4: 1.121 against 1.086 ms), as a scaled row-block kernel did (46 registers
+    // against 40, 1.387 against 1.249 ms; profiles/r04a_axpby_all_fused.json, the run before both were dropped)
+    if (st->kernel == SPMV_B200_KERNEL_CSR_VECTOR) return st->lr.binned || st->tpr != 1 ? kAxpbyScratch : kAxpbyMain;
+    if (st->kernel == SPMV_B200_KERNEL_SELL) return sell_eight_columns(st) ? kAxpbyMain : kAxpbyScratch;
+    return kAxpbyScratch;  // also nnz == 0: s = +0
+}
+
+// the main-kernel path: the scaled twins of the kernels launch() runs on an unbanded view without long-row list
+template <typename T>
+static void launch_main_axpby(DeviceState *st, const T *x, const ScaledStore<T> &sc)
+{
+    cudaStream_t s = st->stream;
+    const int m = st->m;
+    const T *val = (const T *)st->a_val;
+    switch (st->kernel) {
+    case SPMV_B200_KERNEL_CSR_VECTOR: {
+        csr_vector_axpby_kernel<T, 1><<<blocks_for((long long)m * st->tpr), kThreads, 0, s>>>(0, m, st->lr.thr, st->a_rowptr, st->a_col, val, x, sc);
+        count_launch();
+        break;
+    }
+    case SPMV_B200_KERNEL_SELL:
+        if (st->sell.slices > 0) {  // (the 8-column flavour: sell_eight_columns)
+            sell_axpby_kernel<T, 8, 6><<<blocks_for((long long)st->sell.slices * 32), kThreads, 0, s>>>(
+                st->sell.slices, st->sell.slice_ptr, st->sell.full, st->sell.perm, st->sell.col, st->sell.val.as<T>(), x, sc);
+            count_launch();
+        }
+        if (st->sell.banner < m) {
+            csr_tail_axpby_kernel<T><<<blocks_for((long long)(m - st->sell.banner) * 32), kThreads, 0, s>>>(st->sell.banner, m, st->lr.thr, st->a_rowptr, st->a_col, val, x, sc);
+            count_launch();
+        }
+        break;
+    }
+}
+
+template <typename T>
+static bool launch_axpby(DeviceState *st, T alpha, const T *x, T beta, T *y)
+{
+    cudaStream_t s = st->stream;
+    const int m = st->m;
+    if (m == 0) return true;
+    const ScaledStore<T> sc{y, alpha, beta};
+    if (alpha == (T)0) {  // A and x are not read
+        if (beta == (T)0) {
+            if (!SB_CUDA(cudaMemsetAsync(y, 0, (size_t)m * sizeof(T), s))) return false;  // all-zero bits = +0.0
+        } else {
+            axpby_kernel<T><<<blocks_for(m), kThreads, 0, s>>>(m, nullptr, sc);
+            count_launch();
+        }
+    } else {
+        switch (axpby_path(st)) {
+        case kAxpbyFold:
+            if (!launch<T>(st, x, y, &sc)) return false;
+            break;
+        case kAxpbyMain:
+            launch_main_axpby<T>(st, x, sc);
+            break;
+        default: {
+            if (!st->stage.s.get() && !st->stage.s.alloc((size_t)m, st->vsize)) return false;
+            // exactly spmv()'s launches, peers included (with peers SELL runs another flavour, whose sums differ): the
+            // peers then hold A x until the copy below overwrites it with the scaled values
+            if (!launch<T>(st, x, st->stage.s.as<T>())) return false;
+            axpby_kernel<T><<<blocks_for(m), kThreads, 0, s>>>(m, st->stage.s.as<T>(), sc);
+            count_launch();
+        }
+        }
+    }
+    if (st->n_peers > 0) {  // the scaled kernels have no peer variants: one stream-ordered copy
+        peer_copy_kernel<T><<<blocks_for(m), kThreads, 0, s>>>(m, y, peers_of<T>(st));
         count_launch();
     }
     return SB_CUDA(cudaGetLastError());
@@ -1424,6 +1561,51 @@ void spmv(const spmv_Handle_t handle, BASIC_INT_TYPE m, const BASIC_INT_TYPE *Ro
         if (yb && !SB_CUDA(cudaMemcpyAsync(Vector_Val_Y, yd, yb, cudaMemcpyDeviceToHost, st->stream))) return;
         SB_CUDA(cudaStreamSynchronize(st->stream));  // host y is complete on return, as in the reference
     }
+}
+
+// y <- alpha A x + beta y (include/spmv_b200.h): spmv()'s pointer rules without the pipelined host path
+int spmv_b200_spmv_axpby(spmv_Handle_t handle, double alpha, const void *x, double beta, void *y)
+{
+    DeviceState *st = state_of(handle);
+    if (!st) { set_error("spmv_b200_spmv_axpby: NULL handle"); return -1; }
+    if (!st->ok) { set_error("spmv_b200_spmv_axpby: the handle's create failed"); return -1; }
+    if (!y) { set_error("spmv_b200_spmv_axpby: y is NULL"); return -1; }
+    if (!x && st->n > 0) { set_error("spmv_b200_spmv_axpby: x is NULL"); return -1; }
+    if (x == y) { set_error("spmv_b200_spmv_axpby: x and y are the same array"); return -1; }
+    std::lock_guard<std::mutex> lock(st->mu);
+    DeviceGuard guard(st->device);
+    if (st->m == 0) return 0;
+    const bool ok = with_precision(st, [&](auto t) {
+        using T = decltype(t);
+        const T a = (T)alpha, b = (T)beta;  // fp32 handles: alpha and beta rounded to float first
+        const bool read_x = a != (T)0 && st->n > 0, read_y = b != (T)0;
+        const bool x_dev = read_x && is_device_ptr(x), y_dev = is_device_ptr(y);
+        const size_t xb = (size_t)st->n * sizeof(T), yb = (size_t)st->m * sizeof(T);
+        if (st->opts.pin_host) {
+            if (read_x && !x_dev) note_host_buffer(st, 0, x, xb);
+            if (!y_dev) note_host_buffer(st, 1, y, yb);
+        }
+        const T *xd = (const T *)x;
+        T *yd = (T *)y;
+        if (read_x && !x_dev) {
+            if (!st->stage.x.get() && !st->stage.x.alloc(st->n, sizeof(T))) return false;
+            if (!SB_CUDA(cudaMemcpyAsync(st->stage.x.get(), x, xb, cudaMemcpyHostToDevice, st->stream))) return false;
+            xd = st->stage.x.as<T>();
+            if (y_dev) {  // as in spmv(): the caller may reuse x at once, so wait for its copy alone
+                if (!st->ev_x && !SB_CUDA(cudaEventCreateWithFlags(&st->ev_x, cudaEventDisableTiming))) return false;
+                if (!SB_CUDA(cudaEventRecord(st->ev_x, st->stream)) || !SB_CUDA(cudaEventSynchronize(st->ev_x))) return false;
+            }
+        }
+        if (!y_dev) {
+            if (!st->stage.y.get() && !st->stage.y.alloc(st->m, sizeof(T))) return false;
+            yd = st->stage.y.as<T>();
+            if (read_y && !SB_CUDA(cudaMemcpyAsync(yd, y, yb, cudaMemcpyHostToDevice, st->stream))) return false;
+        }
+        if (!launch_axpby<T>(st, a, xd, b, yd)) return false;
+        if (y_dev) return true;
+        return SB_CUDA(cudaMemcpyAsync(y, yd, yb, cudaMemcpyDeviceToHost, st->stream)) && SB_CUDA(cudaStreamSynchronize(st->stream));
+    });
+    return ok ? 0 : -1;
 }
 
 void spmv_clear_handle(spmv_Handle_t this_handle)  // reference gemv_Handle_clear, common.c:31-52,69-71
@@ -1752,6 +1934,7 @@ long long spmv_b200_info(spmv_Handle_t handle, const char *key)
     if (k == "owns_csr") return st->upload.rowptr.get() != nullptr;
     if (k == "released_csr") return st->released_csr;
     if (k == "dev_l2_bytes") return st->dev_l2;
+    if (k == "axpby_path") return axpby_path(st);
     return -1;
 }
 
