@@ -80,6 +80,36 @@ SPMV_B200_API int spmv_b200_set_values(spmv_Handle_t handle, const void *Matrix_
  * handle keeps working). */
 SPMV_B200_API int spmv_b200_spmv_axpby(spmv_Handle_t handle, double alpha, const void *x, double beta, void *y);
 
+/* y <- alpha * A x + beta * y as spmv_b200_spmv_axpby writes it, bit for bit and under all of its rules (rounding,
+ * beta == 0 and alpha == 0, fp32 rounding alpha and beta to float first, host and device pointers, "pin_host", y peers
+ * receiving the scaled values, x == y rejected), and *dot = sum over i of p_i = w[i] * y[i] over the y this call wrote:
+ * the dot product a CG step (p . Ap), a Lanczos step (v . w) or a normalised power method (|y|^2, x . y) needs next,
+ * taken by the kernel that stores each final y value instead of a second pass over y.
+ * p_i is fl(w[i] y[i]) on fp64 handles (one rounding, no FMA) and the exact product of the two floats in double on fp32
+ * handles; the sum is taken in double, and *dot is a double for both precisions.
+ * w: m values of the handle's precision, on the host or the device.  w == y is the new y (so |y|^2 is
+ * spmv_b200_spmv_axpby_dot(h, 1, x, 0, y, y, &d)); w == x is allowed on a square handle (CG's p . Ap; a host x is then
+ * read from its staged copy); any other w must not overlap y.  A host w goes through a staging array of m values,
+ * owned by the handle and allocated at its first use.
+ * dot: a host or a device pointer to one double.  A device dot is written in stream order on the handle's stream,
+ * without a host synchronisation (with device x, y and w the call is only enqueued, so a whole CG step can stay on the
+ * device and be captured in a CUDA graph after one call outside the capture); with a host dot the call is synchronous.
+ * Reproducible: identical inputs on one handle give the same bits in every call, on any stream and in graph replay (no
+ * float atomics; one fixed summation tree: per CTA of 256 rows an xor butterfly over each warp and a fixed tree over the
+ * 8 warp sums, then one CTA of 1024 threads that adds partials t, t + 1024, ... in order and halves in a fixed tree).
+ * Accuracy: no product passes through more than L = 18 + ceil(P / 1024) additions, P <= m + 2 the number of CTA
+ * partials, so |*dot - sum p_i| <= L 2^-53 sum |p_i|.
+ * alpha == beta == 0: y = +0 without reading the old y, and *dot is taken over those zeros (NaN if w holds +-Inf or
+ * NaN); nnz == 0 follows the rule; m == 0 writes *dot = +0 and nothing else.
+ * spmv_b200_info(h, "dot_path") says where the dot is taken, with the encoding of "axpby_path": the same kernel as
+ * spmv_b200_spmv_axpby, except band-segment handles, which take the scratch pass ("axpby_fused" = 0: always the scratch
+ * pass).  The partials (one double per CTA) are owned by the handle, allocated at the first call.
+ * Returns 0, or -1 (spmv_b200_last_error()): NULL handle, failed create, NULL y, NULL dot, NULL w, NULL x with n > 0,
+ * x == y, w == x on a handle that is not square, w overlapping y without being y (all with y and *dot untouched), or a
+ * failed allocation or launch. */
+SPMV_B200_API int spmv_b200_spmv_axpby_dot(spmv_Handle_t handle, double alpha, const void *x, double beta, void *y,
+                                           const void *w, double *dot);
+
 /* ---- streams -----------------------------------------------------------------------------------
  * spmv() with HOST x/y is synchronous (reference semantics).  With DEVICE x/y it is enqueued on the
  * handle's stream (default: the legacy default stream 0) and returns immediately. */
@@ -132,9 +162,9 @@ SPMV_B200_API void spmv_b200_sync(spmv_Handle_t handle);
  *   "refresh"         1 = create also keeps a source map of every value array the handle stores, so that
  *                     spmv_b200_set_values can refresh the values in place (4 bytes per stored slot); 0 (default) = no
  *                     maps, create is unchanged
- *   "axpby_fused"     1 (default) = spmv_b200_spmv_axpby scales in the kernel that stores each final y value where the
- *                     layout has such a kernel; 0 = always A x into the scratch array, then one scaling pass (the same
- *                     bits; for timing one against the other)
+ *   "axpby_fused"     1 (default) = spmv_b200_spmv_axpby (and _dot) scales in the kernel that stores each final y value
+ *                     where the layout has such a kernel; 0 = always A x into the scratch array, then one scaling pass
+ *                     (the same y bits; for timing one against the other)
  * Returns 0, or -1 for an unknown key. */
 SPMV_B200_API int spmv_b200_set_option(const char *key, long long value);
 SPMV_B200_API long long spmv_b200_get_option(const char *key);
@@ -147,7 +177,8 @@ SPMV_B200_API long long spmv_b200_get_option(const char *key);
  * "seg_ctas" (persistent CTAs per SM of the band-segment pass 1; 0 until the handle's first launch), "band_cols",
  * "active_rows", "owns_csr", "released_csr",
  * "layout_fallbacks", "auto_method", "values_snapshotted", "refreshable", "pipeline", "dev_l2_bytes", "axpby_path" (where
- * spmv_b200_spmv_axpby scales: 0 = scratch pass, 1 = main kernel, 2 = fold).  Returns -1 for an unknown key /
+ * spmv_b200_spmv_axpby scales: 0 = scratch pass, 1 = main kernel, 2 = fold), "dot_path" (the same for
+ * spmv_b200_spmv_axpby_dot).  Returns -1 for an unknown key /
  * NULL handle.
  *
  * spmv_b200_structure: copy a device layout array to HOST memory.  Returns its size in bytes (call

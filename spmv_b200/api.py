@@ -40,7 +40,7 @@ EXPORTED_FUNCTIONS = [
     "spmv_b200_recommend_method", "spmv_b200_bands", "spmv_b200_band_columns", "spmv_b200_spmv_bands",
     "spmv_b200_spmv_finish", "spmv_b200_memcpy_async", "spmv_b200_stream_write32", "spmv_b200_stream_wait32_geq",
     "spmv_b200_reorder", "spmv_b200_permute_csr", "spmv_b200_update_values", "spmv_b200_live_allocations",
-    "spmv_b200_set_values", "spmv_b200_spmv_axpby"]
+    "spmv_b200_set_values", "spmv_b200_spmv_axpby", "spmv_b200_spmv_axpby_dot"]
 EXPORTED_DATA = ["Methods_names", "Vectorized_names", "funcNames"]
 
 
@@ -117,6 +117,7 @@ def lib() -> C.CDLL:
     L.spmv_b200_update_values.argtypes = [spmv_Handle_t, vp]
     L.spmv_b200_set_values.argtypes = [spmv_Handle_t, vp]
     L.spmv_b200_spmv_axpby.argtypes = [spmv_Handle_t, C.c_double, vp, C.c_double, vp]
+    L.spmv_b200_spmv_axpby_dot.argtypes = [spmv_Handle_t, C.c_double, vp, C.c_double, vp, vp, vp]
     L.spmv_b200_reorder.argtypes = [i, vp, vp, vp]
     L.spmv_b200_permute_csr.argtypes = [i, vp, vp, vp, ul, vp, vp, vp, vp]
     L.spmv_b200_memcpy_async.argtypes = [vp, vp, C.c_size_t, vp]
@@ -213,6 +214,18 @@ class Handle:
         if lib().spmv_b200_spmv_axpby(self.h, float(alpha), _addr(x), float(beta), _addr(y)) != 0:
             raise RuntimeError("spmv_b200_spmv_axpby: " + last_error())
         return y
+
+    def spmv_axpby_dot(self, alpha, x, beta, y, w=None, dot=None):
+        """y <- alpha A x + beta y in place and w . y (spmv_b200_spmv_axpby_dot); w=None is w = y.  dot=None: returns the
+        dot as a float (synchronous); dot = a 1-element float64 CUDA tensor: written in stream order, returns None."""
+        out = C.c_double()
+        if dot is not None and not (getattr(dot, "is_cuda", False) and dot.numel() == 1 and dot.element_size() == 8):
+            raise ValueError("dot must be None or a 1-element float64 CUDA tensor")
+        where = C.addressof(out) if dot is None else _addr(dot)
+        if lib().spmv_b200_spmv_axpby_dot(self.h, float(alpha), _addr(x), float(beta), _addr(y),
+                                          _addr(y if w is None else w), where) != 0:
+            raise RuntimeError("spmv_b200_spmv_axpby_dot: " + last_error())
+        return out.value if dot is None else None
 
     def info(self, key: str) -> int:
         return int(lib().spmv_b200_info(self.h, key.encode()))

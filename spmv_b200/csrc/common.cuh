@@ -160,8 +160,12 @@ struct DeviceState {
     // staging for host-side x / y; the pipelined host path (CSR-vector kernel) copies x in pieces on s_in,
     // computes row chunks as soon as their prefix of x has arrived, and returns finished chunks of y on s_out
     // val: host values of spmv_b200_set_values, when no upload takes them; s: A x of spmv_b200_spmv_axpby on the handles
-    // whose last store has no scaled kernel (its scratch pass), allocated at the first such call
-    struct Staging { DeviceBytes x, y, val, s; } stage;
+    // whose last store has no scaled kernel (its scratch pass), allocated at the first such call; w: a host w of
+    // spmv_b200_spmv_axpby_dot
+    struct Staging { DeviceBytes x, y, val, s, w; } stage;
+    // spmv_b200_spmv_axpby_dot: the CTA partials of its sum (allocated at the first call, sized by dot_partials_bound)
+    // and, for a host dot, the device double the sum is copied back from
+    struct Dot { DeviceArray<double> partials, result; } dot;
     bool pipeline = false;
     cudaStream_t s_in = nullptr, s_out = nullptr;
     cudaEvent_t ev_in[kMaxPieces] = {}, ev_out[kPipeChunks] = {}, ev_start = nullptr, ev_x = nullptr;
@@ -398,10 +402,51 @@ struct ScaledStore {
     T *y;
     T alpha, beta;
     __device__ __forceinline__ T early(bool pred, long long row) const { return pred && beta != (T)0 ? __ldcs(y + row) : (T)0; }
-    __device__ __forceinline__ void put(long long row, T v, T y_old) const
+    __device__ __forceinline__ T value(T v, T y_old) const
     {
         const T av = mul_rn(alpha, v);
-        stg_y(y + row, beta != (T)0 ? add_rn(av, mul_rn(beta, y_old)) : av);
+        return beta != (T)0 ? add_rn(av, mul_rn(beta, y_old)) : av;
+    }
+    __device__ __forceinline__ void put(long long row, T v, T y_old) const { stg_y(y + row, value(v, y_old)); }
+};
+
+// ---- spmv_b200_spmv_axpby_dot: y <- alpha A x + beta y as ScaledStore writes it, and dot = sum_i fl(w_i y_i) over
+// the rows written, in double for both precisions (an fp32 product taken in double is exact).  w == NULL is w = y.
+// The sum has one fixed order, so identical inputs give identical bits:
+//   1. each thread adds the products of the rows it stores to its own double (one row per thread in every body);
+//   2. an xor butterfly over the warp (5 levels);
+//   3. the 8 warp sums of the CTA in a fixed tree of 3 levels (dot_partial), one partial per CTA, written to
+//      partials[the CTAs of earlier dot launches of the call + blockIdx.x];
+//   4. dot_finish_kernel, one CTA of 1024 threads: thread t adds partials t, t + 1024, ... in that order, then a fixed
+//      halving tree of 10 levels.
+// So no product passes through more than L = 18 + ceil(P / 1024) additions, P the number of partials (at most m + 2),
+// and |dot - sum_i p_i| <= L 2^-53 sum_i |p_i|.
+template <typename T>
+struct DotArgs {
+    ScaledStore<T> sc;
+    const T *w;         // NULL: w is the new y
+    double *partials;   // this launch's first partial
+};
+
+template <typename T>
+struct DotEarly {
+    T y_old, w;
+};
+
+template <typename T>
+struct DotStore {
+    const DotArgs<T> &d;
+    double &acc;
+    __device__ __forceinline__ DotEarly<T> early(bool pred, long long row) const
+    {
+        return {d.sc.early(pred, row), pred && d.w ? ldg_stream(d.w + row) : (T)0};
+    }
+    __device__ __forceinline__ void put(long long row, T v, DotEarly<T> e) const { keep(row, d.sc.value(v, e.y_old), e); }
+    // store the final y of the row and add its product
+    __device__ __forceinline__ void keep(long long row, T y, DotEarly<T> e) const
+    {
+        stg_y(d.sc.y + row, y);
+        acc += __dmul_rn((double)(d.w ? e.w : y), (double)y);
     }
 };
 
@@ -421,6 +466,21 @@ __device__ __forceinline__ T group_sum_c(T v)
 #pragma unroll
     for (int o = WIDTH >> 1; o > 0; o >>= 1) v += __shfl_xor_sync(kFull, v, o);
     return v;
+}
+
+// steps 2 and 3 of the dot's order (DotStore); every thread of the CTA must call it, so the kernel bodies before it
+// return, never exit, early, and hold no __syncthreads
+__device__ __forceinline__ void dot_partial(double acc, double *partials)
+{
+    __shared__ double warp_sum[kWarpsPerCta];
+    static_assert(kWarpsPerCta == 8, "the fixed tree below adds 8 warp sums");
+    acc = group_sum_c<double, 32>(acc);
+    if ((threadIdx.x & 31) == 0) warp_sum[threadIdx.x >> 5] = acc;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        const double *s = warp_sum;
+        partials[blockIdx.x] = ((s[0] + s[1]) + (s[2] + s[3])) + ((s[4] + s[5]) + (s[6] + s[7]));
+    }
 }
 
 // number of entries of a[0..size) that are <= key: the reference's

@@ -172,6 +172,18 @@ csr_vector_axpby_kernel(int row0, int m, int long_thr, const int *__restrict__ r
                                    (const T *)nullptr);
 }
 
+// spmv_b200_spmv_axpby_dot on the same handles: the scaled store, and the CTA's partial of w . y (DotStore)
+template <typename T, int TPR>
+__global__ void __launch_bounds__(kThreads)
+csr_vector_axpby_dot_kernel(int row0, int m, int long_thr, const int *__restrict__ rowptr, const int *__restrict__ col,
+                            const T *__restrict__ val, const T *__restrict__ x, const DotArgs<T> d)
+{
+    double acc = 0;
+    csr_vector_body<T, TPR, false>(threadIdx.x, row0, m, long_thr, rowptr, col, val, x, DotStore<T>{d, acc}, 0, 0,
+                                   (const T *)nullptr);
+    dot_partial(acc, d.partials);
+}
+
 // The same row walk over a LIST of rows: Method_Parallel on matrices whose rows are short but not uniformly so
 // (power-law graphs).  Rows are binned by length class at create and every bin gets the lanes per row that fit it,
 // so a warp only ever holds rows of similar length (no lane group waiting for a 100-entry neighbour).
@@ -395,6 +407,16 @@ __global__ void band_reduce_axpby_kernel(int row0, int row1, int m, int bands, c
     band_reduce_body<T>(row0, row1, m, bands, yv, store);
 }
 
+// spmv_b200_spmv_axpby_dot on a band-major handle: the scaled fold, and the CTA's partial of w . y
+template <typename T>
+__global__ void __launch_bounds__(kThreads)
+band_reduce_axpby_dot_kernel(int row0, int row1, int m, int bands, const T *__restrict__ yv, const DotArgs<T> d)
+{
+    double acc = 0;
+    band_reduce_body<T>(row0, row1, m, bands, yv, DotStore<T>{d, acc});
+    dot_partial(acc, d.partials);
+}
+
 // Largest column index used by each of `chunks` equal row chunks (+1): the prefix of x a chunk needs.  Lets the
 // host-pointer path start a chunk as soon as that prefix has arrived over PCIe.
 __global__ void chunk_xmax_kernel(int m, int chunks, const int *__restrict__ rowptr, const int *__restrict__ col,
@@ -439,6 +461,41 @@ __global__ void axpby_kernel(long long m, const T *__restrict__ s, const ScaledS
     const T y_old = store.early(true, r);
     if (s) store.put(r, ldg_stream(s + r), y_old);
     else stg_y(store.y + r, mul_rn(store.beta, y_old));
+}
+
+// spmv_b200_spmv_axpby_dot's scratch pass: axpby_kernel's values (s = NULL with beta == 0: +0, the old y not read), and
+// the CTA's partial of w . y
+template <typename T>
+__global__ void __launch_bounds__(kThreads) axpby_dot_kernel(long long m, const T *__restrict__ s, const DotArgs<T> d)
+{
+    const long long r = (long long)blockIdx.x * kThreads + threadIdx.x;
+    double acc = 0;
+    if (r < m) {
+        const DotStore<T> store{d, acc};
+        const DotEarly<T> e = store.early(true, r);
+        if (s) store.put(r, ldg_stream(s + r), e);
+        else store.keep(r, d.sc.beta != (T)0 ? mul_rn(d.sc.beta, e.y_old) : (T)0, e);
+    }
+    dot_partial(acc, d.partials);
+}
+
+// step 4 of the dot's order (DotStore): *dot = the sum of partials[0 .. parts)
+constexpr int kDotFinishThreads = 1024;
+__global__ void __launch_bounds__(kDotFinishThreads) dot_finish_kernel(int parts, const double *__restrict__ partials,
+                                                                       double *__restrict__ dot)
+{
+    __shared__ double sum[kDotFinishThreads];
+    const int t = threadIdx.x;
+    double acc = 0;
+    for (int i = t; i < parts; i += kDotFinishThreads) acc += partials[i];
+    sum[t] = acc;
+    __syncthreads();
+#pragma unroll
+    for (int h = kDotFinishThreads / 2; h > 0; h >>= 1) {
+        if (t < h) sum[t] += sum[t + h];
+        __syncthreads();
+    }
+    if (t == 0) *dot = sum[0];
 }
 
 }  // namespace sb

@@ -218,4 +218,16 @@ sell_axpby_kernel(int slices, const long long *__restrict__ slice_ptr, const int
     sell_body<T, U>(threadIdx.x, slices, slice_ptr, full, perm, scol, sval, x, store);
 }
 
+// spmv_b200_spmv_axpby_dot on the same handles (the CSR tail: csr_tail_axpby_dot_kernel)
+template <typename T, int U, int MINB>
+__global__ void __launch_bounds__(kThreads, MINB)
+sell_axpby_dot_kernel(int slices, const long long *__restrict__ slice_ptr, const int *__restrict__ full,
+                      const int *__restrict__ perm, const int *__restrict__ scol, const T *__restrict__ sval,
+                      const T *__restrict__ x, const DotArgs<T> d)
+{
+    double acc = 0;
+    sell_body<T, U>(threadIdx.x, slices, slice_ptr, full, perm, scol, sval, x, DotStore<T>{d, acc});
+    dot_partial(acc, d.partials);
+}
+
 }  // namespace sb

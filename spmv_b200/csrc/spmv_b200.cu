@@ -991,17 +991,37 @@ static void launch_vector(DeviceState *st, int row0, int row1, const T *x, T *y,
     count_launch();
 }
 
-// y_out = the band partials of the virtual y (v.y) added in band order, copied to the peers too; scaled: y_out <- alpha
-// (that sum) + beta y_out instead, and no peers
+// The final store of spmv_b200_spmv_axpby and spmv_b200_spmv_axpby_dot on the host side: the scaling, and for the dot
+// w and the partials array, filled launch after launch (DotStore)
 template <typename T>
-static bool launch_band_fold(DeviceState *st, T *y_out, const ScaledStore<T> *scaled = nullptr)
+struct Scaled {
+    ScaledStore<T> sc;
+    const T *w;              // dot: NULL = w is the new y
+    double *partials;        // NULL: no dot (spmv_b200_spmv_axpby)
+    int parts;               // partials written so far
+    // the arguments of the next dot launch, of `grid` CTAs
+    DotArgs<T> next(int grid)
+    {
+        const DotArgs<T> d{sc, w, partials + parts};
+        parts += grid;
+        return d;
+    }
+};
+
+// y_out = the band partials of the virtual y (v.y) added in band order, copied to the peers too; scaled: y_out <- alpha
+// (that sum) + beta y_out instead (and the dot), and no peers
+template <typename T>
+static bool launch_band_fold(DeviceState *st, T *y_out, Scaled<T> *scaled = nullptr)
 {
-    if (scaled) {
-        band_reduce_axpby_kernel<T><<<blocks_for(st->m), kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), *scaled);
+    const int grid = blocks_for(st->m);
+    if (scaled && scaled->partials) {
+        band_reduce_axpby_dot_kernel<T><<<grid, kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), scaled->next(grid));
+    } else if (scaled) {
+        band_reduce_axpby_kernel<T><<<grid, kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), scaled->sc);
     } else {
         const PeerList<T> peers = peers_of<T>(st);
         const auto kernel = peers.n > 0 ? band_reduce_kernel<T, true> : band_reduce_kernel<T, false>;
-        kernel<<<blocks_for(st->m), kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), y_out, peers);
+        kernel<<<grid, kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), y_out, peers);
     }
     count_launch();
     return SB_CUDA(cudaGetLastError());
@@ -1052,6 +1072,16 @@ csr_tail_axpby_kernel(int row0, int m, int long_thr, const int *__restrict__ row
     csr_tail_body<T>(threadIdx.x, row0, m, long_thr, rowptr, col, val, x, store);
 }
 
+template <typename T>
+__global__ void __launch_bounds__(kThreads)
+csr_tail_axpby_dot_kernel(int row0, int m, int long_thr, const int *__restrict__ rowptr, const int *__restrict__ col,
+                          const T *__restrict__ val, const T *__restrict__ x, const DotArgs<T> d)
+{
+    double acc = 0;
+    csr_tail_body<T>(threadIdx.x, row0, m, long_thr, rowptr, col, val, x, DotStore<T>{d, acc});
+    dot_partial(acc, d.partials);
+}
+
 static int opt_cached_seg_prefetch()
 {
     static const int v = (int)opt("seg_prefetch");  // read once: spmv() is the hot path
@@ -1092,7 +1122,7 @@ static bool launch_seg_bands(DeviceState *st, int b0, int count, const T *x)
 // band segments: carries of segments that cross a tile boundary, then pass 2 (y written once, peers included; scaled:
 // y_out <- alpha (the row sums) + beta y_out, and no peers)
 template <typename T>
-static bool launch_seg_finish(DeviceState *st, T *y_out, const ScaledStore<T> *scaled = nullptr)
+static bool launch_seg_finish(DeviceState *st, T *y_out, Scaled<T> *scaled = nullptr)
 {
     cudaStream_t s = st->stream;
     if (st->seg.cross) launch_carry_fixup<T>(st, s, st->tile.count * kSegChunks, st->tile.carry_row, st->tile.carry_val.as<T>(), st->seg.sums.as<T>());
@@ -1100,8 +1130,8 @@ static bool launch_seg_finish(DeviceState *st, T *y_out, const ScaledStore<T> *s
     auto merge = [&](auto mask_word) {  // row masks of 32 or 64 bands
         using M = decltype(mask_word);
         const int grid = blocks_for((long long)st->seg.groups * 32);
-        if (scaled) {
-            bseg_merge_axpby_kernel<T, M><<<grid, kThreads, 0, s>>>(0, st->m, st->seg.bands, st->seg.mask.as<M>(), st->seg.gbase, st->seg.sums.as<T>(), *scaled);
+        if (scaled) {  // (never with the dot: dot_path)
+            bseg_merge_axpby_kernel<T, M><<<grid, kThreads, 0, s>>>(0, st->m, st->seg.bands, st->seg.mask.as<M>(), st->seg.gbase, st->seg.sums.as<T>(), scaled->sc);
             return;
         }
         const auto kernel = pr.n > 0 ? bseg_merge_kernel<T, M, true> : bseg_merge_kernel<T, M, false>;
@@ -1112,10 +1142,10 @@ static bool launch_seg_finish(DeviceState *st, T *y_out, const ScaledStore<T> *s
     return SB_CUDA(cudaGetLastError());
 }
 
-// y_out = A x.  fold_scaled (spmv_b200_spmv_axpby on a band-major or band-segment handle): the last pass, the fold of
-// the band partials, writes y_out <- alpha A x + beta y_out instead.
+// y_out = A x.  fold_scaled (spmv_b200_spmv_axpby on a band-major or band-segment handle, _dot on a band-major one): the
+// last pass, the fold of the band partials, writes y_out <- alpha A x + beta y_out instead (and the dot's partials).
 template <typename T>
-static bool launch(DeviceState *st, const T *x, T *y_out, const ScaledStore<T> *fold_scaled = nullptr)
+static bool launch(DeviceState *st, const T *x, T *y_out, Scaled<T> *fold_scaled = nullptr)
 {
     cudaStream_t s = st->stream;
     if (st->m == 0) return true;
@@ -1270,49 +1300,89 @@ static int axpby_path(const DeviceState *st)
     return kAxpbyScratch;  // also nnz == 0: s = +0
 }
 
-// the main-kernel path: the scaled twins of the kernels launch() runs on an unbanded view without long-row list
+// spmv_b200_info "dot_path": where spmv_b200_spmv_axpby_dot scales and takes its products.  spmv_b200_spmv_axpby's
+// kernel, except on band segments: their pass-2 dot twin needed 40 registers against the scaled kernel's 32 and lost to
+// the scratch pass on the C5 shard (5.568 against 5.063 ms per call on one B200 at 1000 W, in the run before it was
+// dropped).  The other twins beat their scratch pass (profiles/r05_axpby_dot.json: C1 0.0291 against 0.0333 ms, C2
+// 2.645 against 2.696 ms).
+static int dot_path(const DeviceState *st)
+{
+    return st->kernel == SPMV_B200_KERNEL_BAND_SEG ? kAxpbyScratch : axpby_path(st);
+}
+
+// Partials of one dot: one per CTA of its dot launches, at most -- one CTA per 256 rows (the scratch pass, alpha == 0,
+// the CSR-vector kernel, the band-major fold), plus the slices and the CSR tail of an unbanded SELL handle
+static long long dot_partials_bound(const DeviceState *st)
+{
+    long long p = blocks_for(st->m);
+    if (st->kernel == SPMV_B200_KERNEL_SELL && st->x_bands == 1)
+        p += blocks_for((long long)st->sell.slices * 32) + blocks_for((long long)(st->m - st->sell.banner) * 32);
+    return p;
+}
+
+// the main-kernel path: the scaled (or dot) twins of the kernels launch() runs on an unbanded view without long-row list
 template <typename T>
-static void launch_main_axpby(DeviceState *st, const T *x, const ScaledStore<T> &sc)
+static void launch_main_axpby(DeviceState *st, const T *x, Scaled<T> &sc)
 {
     cudaStream_t s = st->stream;
     const int m = st->m;
     const T *val = (const T *)st->a_val;
     switch (st->kernel) {
     case SPMV_B200_KERNEL_CSR_VECTOR: {
-        csr_vector_axpby_kernel<T, 1><<<blocks_for((long long)m * st->tpr), kThreads, 0, s>>>(0, m, st->lr.thr, st->a_rowptr, st->a_col, val, x, sc);
+        const int grid = blocks_for((long long)m * st->tpr);
+        if (sc.partials) csr_vector_axpby_dot_kernel<T, 1><<<grid, kThreads, 0, s>>>(0, m, st->lr.thr, st->a_rowptr, st->a_col, val, x, sc.next(grid));
+        else csr_vector_axpby_kernel<T, 1><<<grid, kThreads, 0, s>>>(0, m, st->lr.thr, st->a_rowptr, st->a_col, val, x, sc.sc);
         count_launch();
         break;
     }
     case SPMV_B200_KERNEL_SELL:
         if (st->sell.slices > 0) {  // (the 8-column flavour: sell_eight_columns)
-            sell_axpby_kernel<T, 8, 6><<<blocks_for((long long)st->sell.slices * 32), kThreads, 0, s>>>(
-                st->sell.slices, st->sell.slice_ptr, st->sell.full, st->sell.perm, st->sell.col, st->sell.val.as<T>(), x, sc);
+            const int grid = blocks_for((long long)st->sell.slices * 32);
+            if (sc.partials) {
+                sell_axpby_dot_kernel<T, 8, 6><<<grid, kThreads, 0, s>>>(
+                    st->sell.slices, st->sell.slice_ptr, st->sell.full, st->sell.perm, st->sell.col, st->sell.val.as<T>(), x, sc.next(grid));
+            } else {
+                sell_axpby_kernel<T, 8, 6><<<grid, kThreads, 0, s>>>(
+                    st->sell.slices, st->sell.slice_ptr, st->sell.full, st->sell.perm, st->sell.col, st->sell.val.as<T>(), x, sc.sc);
+            }
             count_launch();
         }
         if (st->sell.banner < m) {
-            csr_tail_axpby_kernel<T><<<blocks_for((long long)(m - st->sell.banner) * 32), kThreads, 0, s>>>(st->sell.banner, m, st->lr.thr, st->a_rowptr, st->a_col, val, x, sc);
+            const int grid = blocks_for((long long)(m - st->sell.banner) * 32);
+            if (sc.partials) csr_tail_axpby_dot_kernel<T><<<grid, kThreads, 0, s>>>(st->sell.banner, m, st->lr.thr, st->a_rowptr, st->a_col, val, x, sc.next(grid));
+            else csr_tail_axpby_kernel<T><<<grid, kThreads, 0, s>>>(st->sell.banner, m, st->lr.thr, st->a_rowptr, st->a_col, val, x, sc.sc);
             count_launch();
         }
         break;
     }
 }
 
+// y <- alpha s + beta y over s = A x in the scratch array; s = NULL: alpha == 0
 template <typename T>
-static bool launch_axpby(DeviceState *st, T alpha, const T *x, T beta, T *y)
+static void launch_scratch_pass(DeviceState *st, const T *s, Scaled<T> &sc)
+{
+    const int grid = blocks_for(st->m);
+    if (sc.partials) axpby_dot_kernel<T><<<grid, kThreads, 0, st->stream>>>(st->m, s, sc.next(grid));
+    else axpby_kernel<T><<<grid, kThreads, 0, st->stream>>>(st->m, s, sc.sc);
+    count_launch();
+}
+
+// y <- alpha A x + beta y into sc.sc.y, and the dot's partials when sc.partials is set
+template <typename T>
+static bool launch_axpby(DeviceState *st, const T *x, Scaled<T> &sc)
 {
     cudaStream_t s = st->stream;
     const int m = st->m;
+    T *y = sc.sc.y;
     if (m == 0) return true;
-    const ScaledStore<T> sc{y, alpha, beta};
-    if (alpha == (T)0) {  // A and x are not read
-        if (beta == (T)0) {
+    if (sc.sc.alpha == (T)0) {  // A and x are not read
+        if (sc.sc.beta == (T)0 && !sc.partials) {
             if (!SB_CUDA(cudaMemsetAsync(y, 0, (size_t)m * sizeof(T), s))) return false;  // all-zero bits = +0.0
         } else {
-            axpby_kernel<T><<<blocks_for(m), kThreads, 0, s>>>(m, nullptr, sc);
-            count_launch();
+            launch_scratch_pass<T>(st, (const T *)nullptr, sc);
         }
     } else {
-        switch (axpby_path(st)) {
+        switch (sc.partials ? dot_path(st) : axpby_path(st)) {
         case kAxpbyFold:
             if (!launch<T>(st, x, y, &sc)) return false;
             break;
@@ -1324,8 +1394,7 @@ static bool launch_axpby(DeviceState *st, T alpha, const T *x, T beta, T *y)
             // exactly spmv()'s launches, peers included (with peers SELL runs another flavour, whose sums differ): the
             // peers then hold A x until the copy below overwrites it with the scaled values
             if (!launch<T>(st, x, st->stage.s.as<T>())) return false;
-            axpby_kernel<T><<<blocks_for(m), kThreads, 0, s>>>(m, st->stage.s.as<T>(), sc);
-            count_launch();
+            launch_scratch_pass<T>(st, st->stage.s.as<T>(), sc);
         }
         }
     }
@@ -1333,6 +1402,16 @@ static bool launch_axpby(DeviceState *st, T alpha, const T *x, T beta, T *y)
         peer_copy_kernel<T><<<blocks_for(m), kThreads, 0, s>>>(m, y, peers_of<T>(st));
         count_launch();
     }
+    return SB_CUDA(cudaGetLastError());
+}
+
+// launch_axpby with the dot, then *dot (a device double) = the sum of its partials
+template <typename T>
+static bool launch_axpby_dot(DeviceState *st, const T *x, Scaled<T> &sc, double *dot)
+{
+    if (!launch_axpby<T>(st, x, sc)) return false;
+    dot_finish_kernel<<<1, kDotFinishThreads, 0, st->stream>>>(sc.parts, sc.partials, dot);
+    count_launch();
     return SB_CUDA(cudaGetLastError());
 }
 
@@ -1563,24 +1642,41 @@ void spmv(const spmv_Handle_t handle, BASIC_INT_TYPE m, const BASIC_INT_TYPE *Ro
     }
 }
 
-// y <- alpha A x + beta y (include/spmv_b200.h): spmv()'s pointer rules without the pipelined host path
-int spmv_b200_spmv_axpby(spmv_Handle_t handle, double alpha, const void *x, double beta, void *y)
+// y <- alpha A x + beta y, and with_dot: *dot = w . y (include/spmv_b200.h).  spmv()'s pointer rules without the
+// pipelined host path; fn names the entry point in the errors.
+static int scaled_product(const char *fn, spmv_Handle_t handle, double alpha, const void *x, double beta, void *y,
+                          bool with_dot, const void *w, double *dot)
 {
     DeviceState *st = state_of(handle);
-    if (!st) { set_error("spmv_b200_spmv_axpby: NULL handle"); return -1; }
-    if (!st->ok) { set_error("spmv_b200_spmv_axpby: the handle's create failed"); return -1; }
-    if (!y) { set_error("spmv_b200_spmv_axpby: y is NULL"); return -1; }
-    if (!x && st->n > 0) { set_error("spmv_b200_spmv_axpby: x is NULL"); return -1; }
-    if (x == y) { set_error("spmv_b200_spmv_axpby: x and y are the same array"); return -1; }
+    if (!st) { set_error("%s: NULL handle", fn); return -1; }
+    if (!st->ok) { set_error("%s: the handle's create failed", fn); return -1; }
+    if (!y) { set_error("%s: y is NULL", fn); return -1; }
+    if (with_dot && !dot) { set_error("%s: dot is NULL", fn); return -1; }
+    if (with_dot && !w) { set_error("%s: w is NULL", fn); return -1; }
+    if (!x && st->n > 0) { set_error("%s: x is NULL", fn); return -1; }
+    if (x == y) { set_error("%s: x and y are the same array", fn); return -1; }
+    const bool w_is_x = with_dot && w == x, w_is_y = with_dot && w == y;
+    if (w_is_x && st->m != st->n) { set_error("%s: w is x on a handle that is not square", fn); return -1; }
+    const size_t yb = (size_t)st->m * st->vsize;
+    if (with_dot && !w_is_y && (const char *)w < (const char *)y + yb && (const char *)y < (const char *)w + yb) {
+        set_error("%s: w overlaps y without being y", fn);
+        return -1;
+    }
     std::lock_guard<std::mutex> lock(st->mu);
     DeviceGuard guard(st->device);
-    if (st->m == 0) return 0;
+    const bool dot_dev = with_dot && is_device_ptr(dot);
+    if (st->m == 0) {
+        if (!with_dot) return 0;
+        if (!dot_dev) { *dot = 0.0; return 0; }
+        return SB_CUDA(cudaMemsetAsync(dot, 0, sizeof(double), st->stream)) ? 0 : -1;  // all-zero bits = +0.0
+    }
     const bool ok = with_precision(st, [&](auto t) {
         using T = decltype(t);
         const T a = (T)alpha, b = (T)beta;  // fp32 handles: alpha and beta rounded to float first
-        const bool read_x = a != (T)0 && st->n > 0, read_y = b != (T)0;
+        const bool read_x = (a != (T)0 && st->n > 0) || w_is_x, read_y = b != (T)0;
         const bool x_dev = read_x && is_device_ptr(x), y_dev = is_device_ptr(y);
-        const size_t xb = (size_t)st->n * sizeof(T), yb = (size_t)st->m * sizeof(T);
+        const bool stage_w = with_dot && !w_is_x && !w_is_y && !is_device_ptr(w);
+        const size_t xb = (size_t)st->n * sizeof(T);
         if (st->opts.pin_host) {
             if (read_x && !x_dev) note_host_buffer(st, 0, x, xb);
             if (!y_dev) note_host_buffer(st, 1, y, yb);
@@ -1591,21 +1687,49 @@ int spmv_b200_spmv_axpby(spmv_Handle_t handle, double alpha, const void *x, doub
             if (!st->stage.x.get() && !st->stage.x.alloc(st->n, sizeof(T))) return false;
             if (!SB_CUDA(cudaMemcpyAsync(st->stage.x.get(), x, xb, cudaMemcpyHostToDevice, st->stream))) return false;
             xd = st->stage.x.as<T>();
-            if (y_dev) {  // as in spmv(): the caller may reuse x at once, so wait for its copy alone
-                if (!st->ev_x && !SB_CUDA(cudaEventCreateWithFlags(&st->ev_x, cudaEventDisableTiming))) return false;
-                if (!SB_CUDA(cudaEventRecord(st->ev_x, st->stream)) || !SB_CUDA(cudaEventSynchronize(st->ev_x))) return false;
-            }
+        }
+        const T *wd = w_is_y ? nullptr : w_is_x ? xd : (const T *)w;  // w_is_x: a host x's staged copy
+        if (stage_w) {
+            if (!st->stage.w.get() && !st->stage.w.alloc(st->m, sizeof(T))) return false;
+            if (!SB_CUDA(cudaMemcpyAsync(st->stage.w.get(), w, yb, cudaMemcpyHostToDevice, st->stream))) return false;
+            wd = st->stage.w.as<T>();
+        }
+        // as in spmv(): a call that returns before its kernels end waits for the copies of host inputs alone, so that
+        // the caller may reuse them at once
+        if (((read_x && !x_dev) || stage_w) && y_dev && (!with_dot || dot_dev)) {
+            if (!st->ev_x && !SB_CUDA(cudaEventCreateWithFlags(&st->ev_x, cudaEventDisableTiming))) return false;
+            if (!SB_CUDA(cudaEventRecord(st->ev_x, st->stream)) || !SB_CUDA(cudaEventSynchronize(st->ev_x))) return false;
         }
         if (!y_dev) {
             if (!st->stage.y.get() && !st->stage.y.alloc(st->m, sizeof(T))) return false;
             yd = st->stage.y.as<T>();
             if (read_y && !SB_CUDA(cudaMemcpyAsync(yd, y, yb, cudaMemcpyHostToDevice, st->stream))) return false;
         }
-        if (!launch_axpby<T>(st, a, xd, b, yd)) return false;
-        if (y_dev) return true;
-        return SB_CUDA(cudaMemcpyAsync(y, yd, yb, cudaMemcpyDeviceToHost, st->stream)) && SB_CUDA(cudaStreamSynchronize(st->stream));
+        Scaled<T> sc{{yd, a, b}, wd, nullptr, 0};
+        if (!with_dot) {
+            if (!launch_axpby<T>(st, xd, sc)) return false;
+        } else {
+            if (!st->dot.partials && !st->dot.partials.alloc((size_t)dot_partials_bound(st))) return false;
+            if (!dot_dev && !st->dot.result && !st->dot.result.alloc(1)) return false;
+            sc.partials = st->dot.partials;
+            if (!launch_axpby_dot<T>(st, xd, sc, dot_dev ? dot : st->dot.result.get())) return false;
+        }
+        if (!y_dev && !SB_CUDA(cudaMemcpyAsync(y, yd, yb, cudaMemcpyDeviceToHost, st->stream))) return false;
+        if (with_dot && !dot_dev && !SB_CUDA(cudaMemcpyAsync(dot, st->dot.result.get(), sizeof(double), cudaMemcpyDeviceToHost, st->stream))) return false;
+        return (y_dev && (!with_dot || dot_dev)) || SB_CUDA(cudaStreamSynchronize(st->stream));
     });
     return ok ? 0 : -1;
+}
+
+int spmv_b200_spmv_axpby(spmv_Handle_t handle, double alpha, const void *x, double beta, void *y)
+{
+    return scaled_product("spmv_b200_spmv_axpby", handle, alpha, x, beta, y, false, nullptr, nullptr);
+}
+
+int spmv_b200_spmv_axpby_dot(spmv_Handle_t handle, double alpha, const void *x, double beta, void *y, const void *w,
+                             double *dot)
+{
+    return scaled_product("spmv_b200_spmv_axpby_dot", handle, alpha, x, beta, y, true, w, dot);
 }
 
 void spmv_clear_handle(spmv_Handle_t this_handle)  // reference gemv_Handle_clear, common.c:31-52,69-71
@@ -1935,6 +2059,7 @@ long long spmv_b200_info(spmv_Handle_t handle, const char *key)
     if (k == "released_csr") return st->released_csr;
     if (k == "dev_l2_bytes") return st->dev_l2;
     if (k == "axpby_path") return axpby_path(st);
+    if (k == "dot_path") return dot_path(st);
     return -1;
 }
 
