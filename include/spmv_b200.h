@@ -110,6 +110,34 @@ SPMV_B200_API int spmv_b200_spmv_axpby(spmv_Handle_t handle, double alpha, const
 SPMV_B200_API int spmv_b200_spmv_axpby_dot(spmv_Handle_t handle, double alpha, const void *x, double beta, void *y,
                                            const void *w, double *dot);
 
+/* y <- alpha * (A - sigma I) x + beta * y on a square handle (m == n), and optionally x . y and y . y over the y this
+ * call wrote: one step of a Chebyshev iteration or smoother, a Chebyshev filter or the kernel polynomial method
+ * (t_{k+1} = 2 ((A - c I) / e) t_k - t_{k-1}: alpha = 2 / e, sigma = c, beta = -1, x = t_k, y = t_{k-1} overwritten),
+ * or of a normalised power method on A - sigma I (the Rayleigh quotient x . y and |y|^2), in the kernel that stores
+ * each final y value instead of an axpy and two dot passes over x and y.
+ * With s = the y that spmv() on this handle writes for this x, bit for bit, every row gets
+ * y[i] = fl(fl(alpha fl(s[i] - fl(sigma x[i]))) + fl(beta y_old[i])): five roundings, no FMA, so the result is
+ * reproducible on a CPU.  sigma == 0 skips the shift term entirely (s - fl(0 x) would turn a -0 into +0): the call then
+ * writes spmv_b200_spmv_axpby's y, bit for bit.  Every rule of spmv_b200_spmv_axpby applies unchanged: beta == 0 never
+ * reads the old y (y[i] = fl(alpha fl(s[i] - fl(sigma x[i])))); alpha == 0 reads neither A nor x for y and writes
+ * fl(beta y_old[i]), or +0 when beta == 0; fp32 handles round alpha, beta and sigma to float first; nnz == 0 follows
+ * the rule with s = +0; host and device x and y, "pin_host"; y peers receive the final values; x == y is rejected.
+ * dots: NULL = no dots.  Otherwise a host or a device pointer to 2 doubles: dots[0] = sum over i of fl(x[i] y[i]) and
+ * dots[1] = sum over i of fl(y[i] y[i]), over the y this call wrote, each with spmv_b200_spmv_axpby_dot's products
+ * (one rounding in double on fp64 handles, exact on fp32), its one fixed summation order, its reproducibility and its
+ * bound |dots[k] - sum p_i| <= L 2^-53 sum |p_i|, L = 18 + ceil(P / 1024), P <= m + 2.  So with sigma == 0, dots[0] and
+ * dots[1] are, bit for bit, the *dot of spmv_b200_spmv_axpby_dot(h, alpha, x, beta, y, w, &d) with w = x and with
+ * w = y.  With alpha == 0 and dots, x is read only for dots[0].  A device dots is written in stream order on the
+ * handle's stream without a host synchronisation (with device x and y the call is only enqueued and can be captured
+ * in a CUDA graph after one call outside the capture); with host dots the call is synchronous.  m == 0 writes dots +0,
+ * +0 (when given) and nothing else.
+ * The call takes the paths spmv_b200_info(h, "dot_path") reports, with or without dots.  The partials (two doubles per
+ * CTA) and, for host dots, 2 device doubles are owned by the handle, allocated at their first use.
+ * Returns 0, or -1 (spmv_b200_last_error()): NULL handle, failed create, a handle that is not square, NULL y, NULL x
+ * with n > 0, x == y (all with y and dots untouched), or a failed allocation or launch. */
+SPMV_B200_API int spmv_b200_spmv_shifted(spmv_Handle_t handle, double alpha, double sigma, const void *x, double beta,
+                                         void *y, double *dots);
+
 /* ---- streams -----------------------------------------------------------------------------------
  * spmv() with HOST x/y is synchronous (reference semantics).  With DEVICE x/y it is enqueued on the
  * handle's stream (default: the legacy default stream 0) and returns immediately. */
@@ -162,9 +190,9 @@ SPMV_B200_API void spmv_b200_sync(spmv_Handle_t handle);
  *   "refresh"         1 = create also keeps a source map of every value array the handle stores, so that
  *                     spmv_b200_set_values can refresh the values in place (4 bytes per stored slot); 0 (default) = no
  *                     maps, create is unchanged
- *   "axpby_fused"     1 (default) = spmv_b200_spmv_axpby (and _dot) scales in the kernel that stores each final y value
- *                     where the layout has such a kernel; 0 = always A x into the scratch array, then one scaling pass
- *                     (the same y bits; for timing one against the other)
+ *   "axpby_fused"     1 (default) = spmv_b200_spmv_axpby (_dot, _shifted) scales in the kernel that stores each final y
+ *                     value where the layout has such a kernel; 0 = always A x into the scratch array, then one
+ *                     scaling pass (the same y bits; for timing one against the other)
  * Returns 0, or -1 for an unknown key. */
 SPMV_B200_API int spmv_b200_set_option(const char *key, long long value);
 SPMV_B200_API long long spmv_b200_get_option(const char *key);

@@ -40,7 +40,8 @@ EXPORTED_FUNCTIONS = [
     "spmv_b200_recommend_method", "spmv_b200_bands", "spmv_b200_band_columns", "spmv_b200_spmv_bands",
     "spmv_b200_spmv_finish", "spmv_b200_memcpy_async", "spmv_b200_stream_write32", "spmv_b200_stream_wait32_geq",
     "spmv_b200_reorder", "spmv_b200_permute_csr", "spmv_b200_update_values", "spmv_b200_live_allocations",
-    "spmv_b200_set_values", "spmv_b200_spmv_axpby", "spmv_b200_spmv_axpby_dot"]
+    "spmv_b200_set_values", "spmv_b200_spmv_axpby", "spmv_b200_spmv_axpby_dot",
+    "spmv_b200_spmv_shifted"]
 EXPORTED_DATA = ["Methods_names", "Vectorized_names", "funcNames"]
 
 
@@ -118,6 +119,7 @@ def lib() -> C.CDLL:
     L.spmv_b200_set_values.argtypes = [spmv_Handle_t, vp]
     L.spmv_b200_spmv_axpby.argtypes = [spmv_Handle_t, C.c_double, vp, C.c_double, vp]
     L.spmv_b200_spmv_axpby_dot.argtypes = [spmv_Handle_t, C.c_double, vp, C.c_double, vp, vp, vp]
+    L.spmv_b200_spmv_shifted.argtypes = [spmv_Handle_t, C.c_double, C.c_double, vp, C.c_double, vp, vp]
     L.spmv_b200_reorder.argtypes = [i, vp, vp, vp]
     L.spmv_b200_permute_csr.argtypes = [i, vp, vp, vp, ul, vp, vp, vp, vp]
     L.spmv_b200_memcpy_async.argtypes = [vp, vp, C.c_size_t, vp]
@@ -226,6 +228,19 @@ class Handle:
                                           _addr(y if w is None else w), where) != 0:
             raise RuntimeError("spmv_b200_spmv_axpby_dot: " + last_error())
         return out.value if dot is None else None
+
+    def spmv_shifted(self, alpha, sigma, x, beta, y, dots=None):
+        """y <- alpha (A - sigma I) x + beta y in place, with x . y and y . y (spmv_b200_spmv_shifted).  dots=None:
+        returns (x . y, y . y) as floats (synchronous); dots = a 2-element float64 CUDA tensor: written in stream order,
+        returns None."""
+        out = (C.c_double * 2)()
+        if dots is not None and not (getattr(dots, "is_cuda", False) and dots.numel() == 2 and dots.element_size() == 8
+                                     and dots.is_contiguous()):
+            raise ValueError("dots must be None or a contiguous 2-element float64 CUDA tensor")
+        where = C.addressof(out) if dots is None else _addr(dots)
+        if lib().spmv_b200_spmv_shifted(self.h, float(alpha), float(sigma), _addr(x), float(beta), _addr(y), where) != 0:
+            raise RuntimeError("spmv_b200_spmv_shifted: " + last_error())
+        return (out[0], out[1]) if dots is None else None
 
     def info(self, key: str) -> int:
         return int(lib().spmv_b200_info(self.h, key.encode()))

@@ -164,8 +164,9 @@ struct DeviceState {
     // spmv_b200_spmv_axpby_dot
     struct Staging { DeviceBytes x, y, val, s, w; } stage;
     // spmv_b200_spmv_axpby_dot: the CTA partials of its sum (allocated at the first call, sized by dot_partials_bound)
-    // and, for a host dot, the device double the sum is copied back from
-    struct Dot { DeviceArray<double> partials, result; } dot;
+    // and, for a host dot, the device double the sum is copied back from.  spmv_b200_spmv_shifted with dots: partials
+    // (x . y), yy (y . y, the same size) and, for host dots, pair (2 doubles); each allocated at its first use
+    struct Dot { DeviceArray<double> partials, result, yy, pair; } dot;
     bool pipeline = false;
     cudaStream_t s_in = nullptr, s_out = nullptr;
     cudaEvent_t ev_in[kMaxPieces] = {}, ev_out[kPipeChunks] = {}, ev_start = nullptr, ev_x = nullptr;
@@ -393,6 +394,8 @@ __device__ __forceinline__ double mul_rn(double a, double b) { return __dmul_rn(
 __device__ __forceinline__ float mul_rn(float a, float b) { return __fmul_rn(a, b); }
 __device__ __forceinline__ double add_rn(double a, double b) { return __dadd_rn(a, b); }
 __device__ __forceinline__ float add_rn(float a, float b) { return __fadd_rn(a, b); }
+__device__ __forceinline__ double sub_rn(double a, double b) { return __dsub_rn(a, b); }
+__device__ __forceinline__ float sub_rn(float a, float b) { return __fsub_rn(a, b); }
 
 // y[row] = fl(fl(alpha v) + fl(beta y_old)), three roundings and no FMA (what numpy computes from spmv()'s bits); beta ==
 // 0: fl(alpha v), and the old y is never read, so whatever it holds does not propagate.  (alpha == 0 never reaches a
@@ -450,6 +453,40 @@ struct DotStore {
     }
 };
 
+// ---- spmv_b200_spmv_shifted (square handles): y <- alpha (A - sigma I) x + beta y, the step of a Chebyshev or KPM
+// recurrence, with y[row] = fl(fl(alpha fl(v - fl(sigma x[row]))) + fl(beta y_old)); sigma == 0 skips the shift, so the
+// value is ScaledStore's, bit for bit (v - fl(0 x) would turn a -0 into +0).  With partials, also x . y and y . y over
+// the rows written, each as DotStore takes w . y (w = x and w = y): the same products, the same per-thread sums and the
+// same fixed tree (shift_partials), so that with sigma == 0 both equal spmv_b200_spmv_axpby_dot's bit for bit.
+template <typename T>
+struct ShiftArgs {
+    ScaledStore<T> sc;
+    T sigma;
+    const T *x;         // the x of the product, read again at the stored row
+    double *xy, *yy;    // this launch's first partial of x . y and of y . y; NULL: no dots
+};
+
+template <typename T>
+struct ShiftStore {
+    const ShiftArgs<T> &d;
+    double &xy, &yy;
+    __device__ __forceinline__ T early(bool pred, long long row) const { return d.sc.early(pred, row); }
+    // x[row] is a coalesced streaming read (the row walk gathers x through the evict-last path), issued here rather
+    // than in early(): held through the row walk it takes two more registers, and the fp64 SELL twin spills at its 40
+    __device__ __forceinline__ void put(long long row, T v, T y_old) const
+    {
+        const T xr = ldg_stream(d.x + row);
+        keep(row, d.sc.value(d.sigma != (T)0 ? sub_rn(v, mul_rn(d.sigma, xr)) : v, y_old), xr);
+    }
+    // store the final y of the row and add its two products
+    __device__ __forceinline__ void keep(long long row, T y, T xr) const
+    {
+        stg_y(d.sc.y + row, y);
+        xy += __dmul_rn((double)xr, (double)y);
+        yy += __dmul_rn((double)y, (double)y);
+    }
+};
+
 __device__ __forceinline__ double fma_t(double a, double b, double c) { return fma(a, b, c); }
 __device__ __forceinline__ float fma_t(float a, float b, float c) { return fmaf(a, b, c); }
 
@@ -468,18 +505,39 @@ __device__ __forceinline__ T group_sum_c(T v)
     return v;
 }
 
+// step 3 of the dot's order: the fixed tree over the 8 warp sums of a CTA
+__device__ __forceinline__ double warp_sums_tree(const double *s)
+{
+    static_assert(kWarpsPerCta == 8, "the fixed tree below adds 8 warp sums");
+    return ((s[0] + s[1]) + (s[2] + s[3])) + ((s[4] + s[5]) + (s[6] + s[7]));
+}
+
 // steps 2 and 3 of the dot's order (DotStore); every thread of the CTA must call it, so the kernel bodies before it
 // return, never exit, early, and hold no __syncthreads
 __device__ __forceinline__ void dot_partial(double acc, double *partials)
 {
     __shared__ double warp_sum[kWarpsPerCta];
-    static_assert(kWarpsPerCta == 8, "the fixed tree below adds 8 warp sums");
     acc = group_sum_c<double, 32>(acc);
     if ((threadIdx.x & 31) == 0) warp_sum[threadIdx.x >> 5] = acc;
     __syncthreads();
+    if (threadIdx.x == 0) partials[blockIdx.x] = warp_sums_tree(warp_sum);
+}
+
+// dot_partial for ShiftStore's two sums, each in that order; xy == NULL (no dots) skips it (uniform over the CTA)
+__device__ __forceinline__ void shift_partials(double xy, double yy, double *pxy, double *pyy)
+{
+    __shared__ double warp_sum[2][kWarpsPerCta];
+    if (!pxy) return;
+    xy = group_sum_c<double, 32>(xy);
+    yy = group_sum_c<double, 32>(yy);
+    if ((threadIdx.x & 31) == 0) {
+        warp_sum[0][threadIdx.x >> 5] = xy;
+        warp_sum[1][threadIdx.x >> 5] = yy;
+    }
+    __syncthreads();
     if (threadIdx.x == 0) {
-        const double *s = warp_sum;
-        partials[blockIdx.x] = ((s[0] + s[1]) + (s[2] + s[3])) + ((s[4] + s[5]) + (s[6] + s[7]));
+        pxy[blockIdx.x] = warp_sums_tree(warp_sum[0]);
+        pyy[blockIdx.x] = warp_sums_tree(warp_sum[1]);
     }
 }
 

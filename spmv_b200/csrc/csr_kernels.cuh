@@ -184,6 +184,18 @@ csr_vector_axpby_dot_kernel(int row0, int m, int long_thr, const int *__restrict
     dot_partial(acc, d.partials);
 }
 
+// spmv_b200_spmv_shifted on the same handles: the shifted store, and the CTA's partials of x . y and y . y (ShiftStore)
+template <typename T, int TPR>
+__global__ void __launch_bounds__(kThreads)
+csr_vector_shift_kernel(int row0, int m, int long_thr, const int *__restrict__ rowptr, const int *__restrict__ col,
+                        const T *__restrict__ val, const T *__restrict__ x, const ShiftArgs<T> d)
+{
+    double xy = 0, yy = 0;
+    csr_vector_body<T, TPR, false>(threadIdx.x, row0, m, long_thr, rowptr, col, val, x, ShiftStore<T>{d, xy, yy}, 0,
+                                   0, (const T *)nullptr);
+    shift_partials(xy, yy, d.xy, d.yy);
+}
+
 // The same row walk over a LIST of rows: Method_Parallel on matrices whose rows are short but not uniformly so
 // (power-law graphs).  Rows are binned by length class at create and every bin gets the lanes per row that fit it,
 // so a warp only ever holds rows of similar length (no lane group waiting for a 100-entry neighbour).
@@ -417,6 +429,16 @@ band_reduce_axpby_dot_kernel(int row0, int row1, int m, int bands, const T *__re
     dot_partial(acc, d.partials);
 }
 
+// spmv_b200_spmv_shifted on a band-major handle: the shifted fold (x read at the folded row), and the CTA's partials
+template <typename T>
+__global__ void __launch_bounds__(kThreads)
+band_reduce_shift_kernel(int row0, int row1, int m, int bands, const T *__restrict__ yv, const ShiftArgs<T> d)
+{
+    double xy = 0, yy = 0;
+    band_reduce_body<T>(row0, row1, m, bands, yv, ShiftStore<T>{d, xy, yy});
+    shift_partials(xy, yy, d.xy, d.yy);
+}
+
 // Largest column index used by each of `chunks` equal row chunks (+1): the prefix of x a chunk needs.  Lets the
 // host-pointer path start a chunk as soon as that prefix has arrived over PCIe.
 __global__ void chunk_xmax_kernel(int m, int chunks, const int *__restrict__ rowptr, const int *__restrict__ col,
@@ -477,6 +499,22 @@ __global__ void __launch_bounds__(kThreads) axpby_dot_kernel(long long m, const 
         else store.keep(r, d.sc.beta != (T)0 ? mul_rn(d.sc.beta, e.y_old) : (T)0, e);
     }
     dot_partial(acc, d.partials);
+}
+
+// spmv_b200_spmv_shifted's scratch pass over s = A x (s = NULL: alpha == 0, y = fl(beta y_old), or +0 with beta == 0
+// and the old y not read), and the CTA's partials
+template <typename T>
+__global__ void __launch_bounds__(kThreads) shift_kernel(long long m, const T *__restrict__ s, const ShiftArgs<T> d)
+{
+    const long long r = (long long)blockIdx.x * kThreads + threadIdx.x;
+    double xy = 0, yy = 0;
+    if (r < m) {
+        const ShiftStore<T> store{d, xy, yy};
+        const T y_old = store.early(true, r);
+        if (s) store.put(r, ldg_stream(s + r), y_old);
+        else store.keep(r, d.sc.beta != (T)0 ? mul_rn(d.sc.beta, y_old) : (T)0, ldg_stream(d.x + r));
+    }
+    shift_partials(xy, yy, d.xy, d.yy);
 }
 
 // step 4 of the dot's order (DotStore): *dot = the sum of partials[0 .. parts)

@@ -230,4 +230,16 @@ sell_axpby_dot_kernel(int slices, const long long *__restrict__ slice_ptr, const
     dot_partial(acc, d.partials);
 }
 
+// spmv_b200_spmv_shifted on the same handles (the CSR tail: csr_tail_shift_kernel)
+template <typename T, int U, int MINB>
+__global__ void __launch_bounds__(kThreads, MINB)
+sell_shift_kernel(int slices, const long long *__restrict__ slice_ptr, const int *__restrict__ full,
+                  const int *__restrict__ perm, const int *__restrict__ scol, const T *__restrict__ sval,
+                  const T *__restrict__ x, const ShiftArgs<T> d)
+{
+    double xy = 0, yy = 0;
+    sell_body<T, U>(threadIdx.x, slices, slice_ptr, full, perm, scol, sval, x, ShiftStore<T>{d, xy, yy});
+    shift_partials(xy, yy, d.xy, d.yy);
+}
+
 }  // namespace sb

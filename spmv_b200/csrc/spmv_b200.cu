@@ -991,14 +991,19 @@ static void launch_vector(DeviceState *st, int row0, int row1, const T *x, T *y,
     count_launch();
 }
 
-// The final store of spmv_b200_spmv_axpby and spmv_b200_spmv_axpby_dot on the host side: the scaling, and for the dot
-// w and the partials array, filled launch after launch (DotStore)
+// The final store of spmv_b200_spmv_axpby, spmv_b200_spmv_axpby_dot and spmv_b200_spmv_shifted on the host side: the
+// scaling, for the dot w and the partials array, filled launch after launch (DotStore), and for the shifted store its
+// shift and x (ShiftStore: x . y partials in `partials`, y . y partials in `yy`, both NULL without dots)
 template <typename T>
 struct Scaled {
     ScaledStore<T> sc;
     const T *w;              // dot: NULL = w is the new y
     double *partials;        // NULL: no dot (spmv_b200_spmv_axpby)
     int parts;               // partials written so far
+    bool shifted = false;
+    T sigma = 0;
+    const T *x = nullptr;
+    double *yy = nullptr;
     // the arguments of the next dot launch, of `grid` CTAs
     DotArgs<T> next(int grid)
     {
@@ -1006,15 +1011,24 @@ struct Scaled {
         parts += grid;
         return d;
     }
+    // the arguments of the next shifted launch, of `grid` CTAs
+    ShiftArgs<T> next_shift(int grid)
+    {
+        const ShiftArgs<T> d{sc, sigma, x, partials ? partials + parts : nullptr, partials ? yy + parts : nullptr};
+        if (partials) parts += grid;
+        return d;
+    }
 };
 
 // y_out = the band partials of the virtual y (v.y) added in band order, copied to the peers too; scaled: y_out <- alpha
-// (that sum) + beta y_out instead (and the dot), and no peers
+// (that sum) + beta y_out instead (and the dot, or the shift), and no peers
 template <typename T>
 static bool launch_band_fold(DeviceState *st, T *y_out, Scaled<T> *scaled = nullptr)
 {
     const int grid = blocks_for(st->m);
-    if (scaled && scaled->partials) {
+    if (scaled && scaled->shifted) {
+        band_reduce_shift_kernel<T><<<grid, kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), scaled->next_shift(grid));
+    } else if (scaled && scaled->partials) {
         band_reduce_axpby_dot_kernel<T><<<grid, kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), scaled->next(grid));
     } else if (scaled) {
         band_reduce_axpby_kernel<T><<<grid, kThreads, 0, st->stream>>>(0, st->m, st->m, st->x_bands, st->v.y.as<T>(), scaled->sc);
@@ -1082,6 +1096,16 @@ csr_tail_axpby_dot_kernel(int row0, int m, int long_thr, const int *__restrict__
     dot_partial(acc, d.partials);
 }
 
+template <typename T>
+__global__ void __launch_bounds__(kThreads)
+csr_tail_shift_kernel(int row0, int m, int long_thr, const int *__restrict__ rowptr, const int *__restrict__ col,
+                      const T *__restrict__ val, const T *__restrict__ x, const ShiftArgs<T> d)
+{
+    double xy = 0, yy = 0;
+    csr_tail_body<T>(threadIdx.x, row0, m, long_thr, rowptr, col, val, x, ShiftStore<T>{d, xy, yy});
+    shift_partials(xy, yy, d.xy, d.yy);
+}
+
 static int opt_cached_seg_prefetch()
 {
     static const int v = (int)opt("seg_prefetch");  // read once: spmv() is the hot path
@@ -1130,7 +1154,7 @@ static bool launch_seg_finish(DeviceState *st, T *y_out, Scaled<T> *scaled = nul
     auto merge = [&](auto mask_word) {  // row masks of 32 or 64 bands
         using M = decltype(mask_word);
         const int grid = blocks_for((long long)st->seg.groups * 32);
-        if (scaled) {  // (never with the dot: dot_path)
+        if (scaled) {  // (never with the dot or the shift: dot_path)
             bseg_merge_axpby_kernel<T, M><<<grid, kThreads, 0, s>>>(0, st->m, st->seg.bands, st->seg.mask.as<M>(), st->seg.gbase, st->seg.sums.as<T>(), scaled->sc);
             return;
         }
@@ -1320,7 +1344,8 @@ static long long dot_partials_bound(const DeviceState *st)
     return p;
 }
 
-// the main-kernel path: the scaled (or dot) twins of the kernels launch() runs on an unbanded view without long-row list
+// the main-kernel path: the scaled (dot, shifted) twins of the kernels launch() runs on an unbanded view without long-row
+// list
 template <typename T>
 static void launch_main_axpby(DeviceState *st, const T *x, Scaled<T> &sc)
 {
@@ -1330,7 +1355,8 @@ static void launch_main_axpby(DeviceState *st, const T *x, Scaled<T> &sc)
     switch (st->kernel) {
     case SPMV_B200_KERNEL_CSR_VECTOR: {
         const int grid = blocks_for((long long)m * st->tpr);
-        if (sc.partials) csr_vector_axpby_dot_kernel<T, 1><<<grid, kThreads, 0, s>>>(0, m, st->lr.thr, st->a_rowptr, st->a_col, val, x, sc.next(grid));
+        if (sc.shifted) csr_vector_shift_kernel<T, 1><<<grid, kThreads, 0, s>>>(0, m, st->lr.thr, st->a_rowptr, st->a_col, val, x, sc.next_shift(grid));
+        else if (sc.partials) csr_vector_axpby_dot_kernel<T, 1><<<grid, kThreads, 0, s>>>(0, m, st->lr.thr, st->a_rowptr, st->a_col, val, x, sc.next(grid));
         else csr_vector_axpby_kernel<T, 1><<<grid, kThreads, 0, s>>>(0, m, st->lr.thr, st->a_rowptr, st->a_col, val, x, sc.sc);
         count_launch();
         break;
@@ -1338,7 +1364,10 @@ static void launch_main_axpby(DeviceState *st, const T *x, Scaled<T> &sc)
     case SPMV_B200_KERNEL_SELL:
         if (st->sell.slices > 0) {  // (the 8-column flavour: sell_eight_columns)
             const int grid = blocks_for((long long)st->sell.slices * 32);
-            if (sc.partials) {
+            if (sc.shifted) {
+                sell_shift_kernel<T, 8, 6><<<grid, kThreads, 0, s>>>(
+                    st->sell.slices, st->sell.slice_ptr, st->sell.full, st->sell.perm, st->sell.col, st->sell.val.as<T>(), x, sc.next_shift(grid));
+            } else if (sc.partials) {
                 sell_axpby_dot_kernel<T, 8, 6><<<grid, kThreads, 0, s>>>(
                     st->sell.slices, st->sell.slice_ptr, st->sell.full, st->sell.perm, st->sell.col, st->sell.val.as<T>(), x, sc.next(grid));
             } else {
@@ -1349,7 +1378,8 @@ static void launch_main_axpby(DeviceState *st, const T *x, Scaled<T> &sc)
         }
         if (st->sell.banner < m) {
             const int grid = blocks_for((long long)(m - st->sell.banner) * 32);
-            if (sc.partials) csr_tail_axpby_dot_kernel<T><<<grid, kThreads, 0, s>>>(st->sell.banner, m, st->lr.thr, st->a_rowptr, st->a_col, val, x, sc.next(grid));
+            if (sc.shifted) csr_tail_shift_kernel<T><<<grid, kThreads, 0, s>>>(st->sell.banner, m, st->lr.thr, st->a_rowptr, st->a_col, val, x, sc.next_shift(grid));
+            else if (sc.partials) csr_tail_axpby_dot_kernel<T><<<grid, kThreads, 0, s>>>(st->sell.banner, m, st->lr.thr, st->a_rowptr, st->a_col, val, x, sc.next(grid));
             else csr_tail_axpby_kernel<T><<<grid, kThreads, 0, s>>>(st->sell.banner, m, st->lr.thr, st->a_rowptr, st->a_col, val, x, sc.sc);
             count_launch();
         }
@@ -1362,7 +1392,8 @@ template <typename T>
 static void launch_scratch_pass(DeviceState *st, const T *s, Scaled<T> &sc)
 {
     const int grid = blocks_for(st->m);
-    if (sc.partials) axpby_dot_kernel<T><<<grid, kThreads, 0, st->stream>>>(st->m, s, sc.next(grid));
+    if (sc.shifted) shift_kernel<T><<<grid, kThreads, 0, st->stream>>>(st->m, s, sc.next_shift(grid));
+    else if (sc.partials) axpby_dot_kernel<T><<<grid, kThreads, 0, st->stream>>>(st->m, s, sc.next(grid));
     else axpby_kernel<T><<<grid, kThreads, 0, st->stream>>>(st->m, s, sc.sc);
     count_launch();
 }
@@ -1382,7 +1413,7 @@ static bool launch_axpby(DeviceState *st, const T *x, Scaled<T> &sc)
             launch_scratch_pass<T>(st, (const T *)nullptr, sc);
         }
     } else {
-        switch (sc.partials ? dot_path(st) : axpby_path(st)) {
+        switch (sc.partials || sc.shifted ? dot_path(st) : axpby_path(st)) {
         case kAxpbyFold:
             if (!launch<T>(st, x, y, &sc)) return false;
             break;
@@ -1405,13 +1436,15 @@ static bool launch_axpby(DeviceState *st, const T *x, Scaled<T> &sc)
     return SB_CUDA(cudaGetLastError());
 }
 
-// launch_axpby with the dot, then *dot (a device double) = the sum of its partials
+// launch_axpby with the dot, then *dot (a device double) = the sum of its partials; shifted: dot[0] and dot[1] = the
+// sums of the x . y and the y . y partials, each in the finish kernel's one order
 template <typename T>
 static bool launch_axpby_dot(DeviceState *st, const T *x, Scaled<T> &sc, double *dot)
 {
     if (!launch_axpby<T>(st, x, sc)) return false;
     dot_finish_kernel<<<1, kDotFinishThreads, 0, st->stream>>>(sc.parts, sc.partials, dot);
-    count_launch();
+    if (sc.shifted) dot_finish_kernel<<<1, kDotFinishThreads, 0, st->stream>>>(sc.parts, sc.yy, dot + 1);
+    count_launch(sc.shifted ? 2 : 1);
     return SB_CUDA(cudaGetLastError());
 }
 
@@ -1642,40 +1675,48 @@ void spmv(const spmv_Handle_t handle, BASIC_INT_TYPE m, const BASIC_INT_TYPE *Ro
     }
 }
 
-// y <- alpha A x + beta y, and with_dot: *dot = w . y (include/spmv_b200.h).  spmv()'s pointer rules without the
-// pipelined host path; fn names the entry point in the errors.
+// y <- alpha A x + beta y, and with_dot: *dot = w . y; sigma (spmv_b200_spmv_shifted): y <- alpha (A - sigma I) x +
+// beta y instead, and with_dot: dot[0] = x . y, dot[1] = y . y (w unused) (include/spmv_b200.h).  spmv()'s pointer
+// rules without the pipelined host path; fn names the entry point in the errors.
 static int scaled_product(const char *fn, spmv_Handle_t handle, double alpha, const void *x, double beta, void *y,
-                          bool with_dot, const void *w, double *dot)
+                          bool with_dot, const void *w, double *dot, const double *sigma = nullptr)
 {
     DeviceState *st = state_of(handle);
     if (!st) { set_error("%s: NULL handle", fn); return -1; }
     if (!st->ok) { set_error("%s: the handle's create failed", fn); return -1; }
+    if (sigma && st->m != st->n) { set_error("%s: the handle is not square", fn); return -1; }
     if (!y) { set_error("%s: y is NULL", fn); return -1; }
-    if (with_dot && !dot) { set_error("%s: dot is NULL", fn); return -1; }
-    if (with_dot && !w) { set_error("%s: w is NULL", fn); return -1; }
+    const bool with_w = with_dot && !sigma;
+    if (with_w && !dot) { set_error("%s: dot is NULL", fn); return -1; }
+    if (with_w && !w) { set_error("%s: w is NULL", fn); return -1; }
     if (!x && st->n > 0) { set_error("%s: x is NULL", fn); return -1; }
     if (x == y) { set_error("%s: x and y are the same array", fn); return -1; }
-    const bool w_is_x = with_dot && w == x, w_is_y = with_dot && w == y;
+    const bool w_is_x = with_w && w == x, w_is_y = with_w && w == y;
     if (w_is_x && st->m != st->n) { set_error("%s: w is x on a handle that is not square", fn); return -1; }
     const size_t yb = (size_t)st->m * st->vsize;
-    if (with_dot && !w_is_y && (const char *)w < (const char *)y + yb && (const char *)y < (const char *)w + yb) {
+    if (with_w && !w_is_y && (const char *)w < (const char *)y + yb && (const char *)y < (const char *)w + yb) {
         set_error("%s: w overlaps y without being y", fn);
         return -1;
     }
     std::lock_guard<std::mutex> lock(st->mu);
     DeviceGuard guard(st->device);
     const bool dot_dev = with_dot && is_device_ptr(dot);
+    const int ndots = sigma ? 2 : 1;
     if (st->m == 0) {
         if (!with_dot) return 0;
-        if (!dot_dev) { *dot = 0.0; return 0; }
-        return SB_CUDA(cudaMemsetAsync(dot, 0, sizeof(double), st->stream)) ? 0 : -1;  // all-zero bits = +0.0
+        if (!dot_dev) { std::fill(dot, dot + ndots, 0.0); return 0; }
+        return SB_CUDA(cudaMemsetAsync(dot, 0, ndots * sizeof(double), st->stream)) ? 0 : -1;  // all-zero bits = +0.0
     }
     const bool ok = with_precision(st, [&](auto t) {
         using T = decltype(t);
         const T a = (T)alpha, b = (T)beta;  // fp32 handles: alpha and beta rounded to float first
-        const bool read_x = (a != (T)0 && st->n > 0) || w_is_x, read_y = b != (T)0;
+        const T sg = sigma ? (T)*sigma : (T)0;  // and sigma
+        // the shifted kernels run when there is a shift to apply or dots to take; otherwise the call is
+        // spmv_b200_spmv_axpby's, bit for bit and launch for launch
+        const bool shifted = sigma && (with_dot || (a != (T)0 && sg != (T)0));
+        const bool read_x = (a != (T)0 && st->n > 0) || w_is_x || (sigma && with_dot), read_y = b != (T)0;
         const bool x_dev = read_x && is_device_ptr(x), y_dev = is_device_ptr(y);
-        const bool stage_w = with_dot && !w_is_x && !w_is_y && !is_device_ptr(w);
+        const bool stage_w = with_w && !w_is_x && !w_is_y && !is_device_ptr(w);
         const size_t xb = (size_t)st->n * sizeof(T);
         if (st->opts.pin_host) {
             if (read_x && !x_dev) note_host_buffer(st, 0, x, xb);
@@ -1706,16 +1747,25 @@ static int scaled_product(const char *fn, spmv_Handle_t handle, double alpha, co
             if (read_y && !SB_CUDA(cudaMemcpyAsync(yd, y, yb, cudaMemcpyHostToDevice, st->stream))) return false;
         }
         Scaled<T> sc{{yd, a, b}, wd, nullptr, 0};
+        if (shifted) {
+            sc.shifted = true;
+            sc.sigma = sg;
+            sc.x = xd;  // a host x: its staged copy
+        }
+        DeviceArray<double> &result = sigma ? st->dot.pair : st->dot.result;
         if (!with_dot) {
             if (!launch_axpby<T>(st, xd, sc)) return false;
         } else {
-            if (!st->dot.partials && !st->dot.partials.alloc((size_t)dot_partials_bound(st))) return false;
-            if (!dot_dev && !st->dot.result && !st->dot.result.alloc(1)) return false;
+            const size_t bound = (size_t)dot_partials_bound(st);
+            if (!st->dot.partials && !st->dot.partials.alloc(bound)) return false;
+            if (sigma && !st->dot.yy && !st->dot.yy.alloc(bound)) return false;
+            if (!dot_dev && !result && !result.alloc(ndots)) return false;
             sc.partials = st->dot.partials;
-            if (!launch_axpby_dot<T>(st, xd, sc, dot_dev ? dot : st->dot.result.get())) return false;
+            sc.yy = st->dot.yy;
+            if (!launch_axpby_dot<T>(st, xd, sc, dot_dev ? dot : result.get())) return false;
         }
         if (!y_dev && !SB_CUDA(cudaMemcpyAsync(y, yd, yb, cudaMemcpyDeviceToHost, st->stream))) return false;
-        if (with_dot && !dot_dev && !SB_CUDA(cudaMemcpyAsync(dot, st->dot.result.get(), sizeof(double), cudaMemcpyDeviceToHost, st->stream))) return false;
+        if (with_dot && !dot_dev && !SB_CUDA(cudaMemcpyAsync(dot, result.get(), ndots * sizeof(double), cudaMemcpyDeviceToHost, st->stream))) return false;
         return (y_dev && (!with_dot || dot_dev)) || SB_CUDA(cudaStreamSynchronize(st->stream));
     });
     return ok ? 0 : -1;
@@ -1730,6 +1780,12 @@ int spmv_b200_spmv_axpby_dot(spmv_Handle_t handle, double alpha, const void *x, 
                              double *dot)
 {
     return scaled_product("spmv_b200_spmv_axpby_dot", handle, alpha, x, beta, y, true, w, dot);
+}
+
+int spmv_b200_spmv_shifted(spmv_Handle_t handle, double alpha, double sigma, const void *x, double beta, void *y,
+                           double *dots)
+{
+    return scaled_product("spmv_b200_spmv_shifted", handle, alpha, x, beta, y, dots != nullptr, nullptr, dots, &sigma);
 }
 
 void spmv_clear_handle(spmv_Handle_t this_handle)  // reference gemv_Handle_clear, common.c:31-52,69-71
